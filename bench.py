@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's algorithm on the host cores (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write obs / reward / done of the last timed step as DIR/*.npy
 
 A "step" is one control step of every env of the batch (one launch of step_fused_kernel):
 reset-if-flagged + 5 physics sub-steps + CaptureXY obs + reward + penalties + done, full per-env
@@ -29,6 +30,8 @@ import torch  # noqa: E402
 
 BYTES_PER_ENV_STEP = 268          # "A, full DR, stats off" (SURVEY 8(d)): 156 B read + 112 B written
 METRIC, UNIT = "ASV env-steps/sec", "env-steps/s"
+DUMP_LIMIT_BYTES = 64_000_000     # --dump-outputs: all files together (2^20 envs x (13 + 1 + 1) float32 = 62.9 MB fits whole)
+NPY_HEADER_BYTES = 128
 
 
 def log(*a):
@@ -155,12 +158,14 @@ def run_reference(args, emit):
     if rank != 0:
         return
     budget = 150.0
-    cb, s_per_step = cpu_port(budget, steps=args.steps if args.steps <= 64 else None, warmup=min(args.warmup, 3))
+    # exactly --warmup + --steps control steps; only the env count is sized to the budget
+    cb, s_per_step = cpu_port(budget, steps=args.steps, warmup=args.warmup)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": s_per_step * 1e3, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": workload_config(args.envs, note="reference arm: the oracle port of the reference's torch path on host cores "
-                                      "(the Python reference needs Isaac Sim and cannot travel to the GPU box); each step is a bounded sample"),
+                                      "(the Python reference needs Isaac Sim); the env count is sized so that warm-up + timed steps "
+                                      f"fit a {budget:.0f} s budget"),
             "cpu_baseline": cb, "e2e": {"value": cb["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     emit(line)
@@ -174,6 +179,29 @@ def workload_config(envs, note=None):
     if note:
         c["note"] = note
     return c
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes per-env arrays (first dim = env) as <out_dir>/<name>.npy in float32, so that two builds can be compared output for output.
+    Above DUMP_LIMIT_BYTES in all, every array keeps the same fixed, seeded sample of env rows; env_index.npy (float64) lists them."""
+    import numpy as np
+
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(4 * a[0].numel() for a in arrays.values())
+    keep = None
+    if n * row_bytes + NPY_HEADER_BYTES * len(arrays) > DUMP_LIMIT_BYTES:
+        m = (DUMP_LIMIT_BYTES - NPY_HEADER_BYTES * (len(arrays) + 1)) // (row_bytes + 8)
+        keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:m].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach()
+        if keep is not None:
+            a = a[keep.to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.to(torch.float32).cpu().numpy())
+    if keep is not None:
+        np.save(os.path.join(out_dir, "env_index.npy"), keep.to(torch.float64).numpy())
+    log(f"  outputs of the last timed step -> {out_dir}: {', '.join(arrays)}"
+        + (f" ({len(keep)} of {n} envs, env_index.npy)" if keep is not None else f" ({n} envs)"))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -614,7 +642,13 @@ def main():
     ap.add_argument("--no-loopz", action="store_true", help="skip the loopz-learner leg")
     ap.add_argument("--ppo-envs", type=int, default=16384, help="envs per GPU of the PPO leg (BASELINE config[2])")
     ap.add_argument("--ppo-epochs", type=int, default=10)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write obs / reward / done of the last one (rank 0's envs) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the timed CUDA path: use it with --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -648,6 +682,9 @@ def main():
     clocks = sampler.stop()
     launches = _lib.launch_count() - launches0 - args.warmup
     env.check_finite()
+    if args.dump_outputs and rank == 0:
+        # env.step returns the env's own buffers: until the next step they hold what the last timed step returned
+        dump_outputs(args.dump_outputs, {"obs": env.obs, "reward": env.rew, "done": env.reset_buf})
     value = world * n * args.steps / (ms * 1e-3)
     ms_per_step = ms / args.steps
     peak, peak_src = measured_peak()

@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY.  Generates tests/golden/*.npz by executing the UNMODIFIED reference
-modules (/root/reference, CPU torch, fp32) under oracle/ref_shim.py on seeded synthetic inputs.
+modules (a reference checkout, CPU torch, fp32) under oracle/ref_shim.py on seeded synthetic inputs.
 
-Run in the build container (the reference does not exist on the GPU box):
-    python -m oracle.make_golden
+Run where a checkout of the reference exists:
+    USV_REFERENCE_ROOT=<reference checkout> python -m oracle.make_golden
 The fixtures are small (N=32) and committed; tests/test_oracle_cpu.py checks the oracle restatement
 against them and tests/test_gpu_parity.py checks the CUDA kernels against them.
 

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """TEST INFRASTRUCTURE ONLY.  Runs the UNMODIFIED reference classes of the USV SysID distillation step (StateHistoryEncoder,
 USVSysIDAgent, USVSysIDTrainer, ObsStorage; OIGE/algo/ppo/{module,dagger,storage}.py) on seeded inputs and freezes
-tests/golden/dagger_sysid.npz.  Build container only (needs /root/reference):  python oracle/make_golden_dagger.py"""
+tests/golden/dagger_sysid.npz.  Needs a reference checkout:  USV_REFERENCE_ROOT=<reference checkout> python oracle/make_golden_dagger.py"""
 import os
 import sys
 

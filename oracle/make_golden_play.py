@@ -3,7 +3,8 @@
 (`_quantize_xy`, `_hash_obstacles_xy`, `_bootstrap_mean_ci`, `_infer_done_reason`, `_apply_mass_mode_to_obs`;
 OIGE/scripts/rlgames_play_loopz.py:135-171,493-533,560-621)
 into tests/golden/play_metrics.json.  The script itself imports hydra / Isaac Sim at module level, so the function definitions are
-taken out of its syntax tree and executed unmodified.  Run in the build container (needs /root/reference):  python oracle/make_golden_play.py"""
+taken out of its syntax tree and executed unmodified.  Needs a reference checkout:
+USV_REFERENCE_ROOT=<reference checkout> python oracle/make_golden_play.py"""
 import ast
 import hashlib
 import json
@@ -13,7 +14,7 @@ from typing import Any, Dict, Optional, Tuple
 
 import numpy as np
 
-REF = "/root/reference/omniisaacgymenvs/scripts/rlgames_play_loopz.py"
+REF = os.path.join(os.environ.get("USV_REFERENCE_ROOT", ""), "omniisaacgymenvs", "scripts", "rlgames_play_loopz.py")
 WANT = {"_quantize_xy", "_hash_obstacles_xy", "_bootstrap_mean_ci", "_infer_done_reason", "_apply_mass_mode_to_obs"}
 
 

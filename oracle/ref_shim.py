@@ -1,10 +1,11 @@
 """TEST INFRASTRUCTURE ONLY -- never imported by the product path.
 
-Import shim that lets the *unmodified* reference modules under /root/reference be
-executed on CPU in the build container (no Isaac Sim, no pytorch3d, no gym).
-It is used by ``oracle/make_golden.py`` to generate the committed fixtures in
-``tests/golden/`` and by ``tests/test_oracle_vs_reference.py`` (skipped when
-/root/reference is absent, e.g. on the GPU box).
+Import shim that lets the *unmodified* reference modules of a reference checkout
+(the directory named by the environment variable USV_REFERENCE_ROOT) be executed on
+CPU (no Isaac Sim, no pytorch3d, no gym).  The reference is not part of this
+repository.  The shim is used by ``oracle/make_golden*.py`` to generate the committed
+fixtures in ``tests/golden/`` and by the tests that compare with the reference
+directly, which skip when USV_REFERENCE_ROOT is unset.
 
 What is faked (SURVEY.md section 8(c)):
   * ``omni.*``, ``pxr.*``, ``carb``, ``gym``, ``matplotlib``, ``ray``, ``tensorboardX``,
@@ -30,7 +31,7 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("USV_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("USV_REFERENCE_ROOT", "")
 
 _FAKE_ROOTS = (
     "omni", "pxr", "carb", "gym", "matplotlib", "ray", "tensorboardX", "cv2",
@@ -39,7 +40,7 @@ _FAKE_ROOTS = (
 
 
 def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "omniisaacgymenvs"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "omniisaacgymenvs"))
 
 
 def snapshot_dir() -> str:
@@ -139,7 +140,7 @@ def install() -> None:
     if _installed:
         return
     if not reference_available():
-        raise FileNotFoundError(f"reference not found at {REFERENCE_ROOT}")
+        raise FileNotFoundError(f"no reference checkout at USV_REFERENCE_ROOT={REFERENCE_ROOT!r}: set it to the reference project's root")
     sys.meta_path.insert(0, _FakeFinder())
 
     p3d = types.ModuleType("pytorch3d")

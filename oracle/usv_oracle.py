@@ -6,9 +6,8 @@ reference file:line it follows.  Only tests/, __graft_entry__.smoke() and bench.
 --impl reference legs may import this module.
 
 Pinning: this restatement is checked against outputs of the *reference modules themselves*
-(imported in the build container through oracle/ref_shim.py) frozen in tests/golden/*.npz by
-oracle/make_golden.py, and -- when /root/reference is present -- live against the reference
-classes in tests/test_oracle_vs_reference.py.  The reference's own tests hold no vectors for
+(imported from a reference checkout through oracle/ref_shim.py) frozen in tests/golden/*.npz by
+oracle/make_golden.py.  The reference's own tests hold no vectors for
 this path (SURVEY 4.2).  The PhysX step is NOT in the reference tree: its stand-in (planar
 semi-implicit Euler, DESIGN.md) is "parity unpinned" and is checked against the float64 host
 integration in oracle/integrator64.py instead.

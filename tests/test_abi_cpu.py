@@ -10,6 +10,10 @@ import pytest
 from omniisaacgymenvs_loop_b200 import _lib
 from omniisaacgymenvs_loop_b200.config import UsvEnvConfig, parse_penalty_lambda, load_task_yaml, PenaltyTerm
 from omniisaacgymenvs_loop_b200 import config as C
+from oracle import ref_shim
+
+# the reference project's YAML files are not part of this repository: point USV_REFERENCE_ROOT at a checkout of it to run these
+needs_reference = pytest.mark.skipif(not ref_shim.reference_available(), reason="needs a checkout of the reference project (USV_REFERENCE_ROOT)")
 
 
 def test_library_loads_and_exports_every_declared_symbol():
@@ -84,12 +88,12 @@ def test_penalty_lambda_closed_set():
         f("lambda x,step: torch.tanh(x)")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference YAMLs only exist in the build container")
+@needs_reference
 def test_reference_yamls_parse():
-    snap = glob.glob("/root/reference/811*/USV_Virtual_CaptureXY_SysID-TEST.yaml")[0]
+    snap = os.path.join(ref_shim.snapshot_dir(), "USV_Virtual_CaptureXY_SysID-TEST.yaml")
     cfg = UsvEnvConfig.from_task_cfg(load_task_yaml(snap))
     assert dataclasses.asdict(cfg) == dataclasses.asdict(UsvEnvConfig())   # defaults ARE the classic snapshot
-    for y in glob.glob("/root/reference/omniisaacgymenvs/cfg/task/USV/IROS2024/USV_Virtual_CaptureXY_*DR50.yaml"):
+    for y in glob.glob(os.path.join(ref_shim.REFERENCE_ROOT, "omniisaacgymenvs/cfg/task/USV/IROS2024/USV_Virtual_CaptureXY_*DR50.yaml")):
         c = UsvEnvConfig.from_task_cfg(load_task_yaml(y, num_envs=64))
         assert c.num_envs == 64 and c.use_sin_force and c.drag_rand and c.thr_rand and c.n_substeps == 5
 
@@ -115,9 +119,10 @@ def test_live_task_cfg_round_trip():
         UsvLiveConfig.from_task_cfg(tb)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference YAMLs only exist in the build container")
+@needs_reference
 def test_reference_live_yaml_parses_to_the_shipped_defaults():
     from omniisaacgymenvs_loop_b200.config import UsvLiveConfig, live_default_config, live_env_config
-    y = load_task_yaml("/root/reference/omniisaacgymenvs/cfg/task/USV/IROS2024/USV_Virtual_CaptureXY_SysID-TEST.yaml", num_envs=128)
+    y = load_task_yaml(os.path.join(ref_shim.REFERENCE_ROOT, "omniisaacgymenvs/cfg/task/USV/IROS2024/USV_Virtual_CaptureXY_SysID-TEST.yaml"),
+                       num_envs=128)
     assert dataclasses.asdict(live_env_config(y)) == dataclasses.asdict(live_default_config(num_envs=128))
     assert UsvLiveConfig.from_task_cfg(y) == UsvLiveConfig()
