@@ -11,7 +11,6 @@ schedule only moves when `update_scheduler()` is called (the live script never c
 from __future__ import annotations
 
 import ctypes
-import os
 
 import numpy as np
 import torch
@@ -85,7 +84,7 @@ class PPO:
         # tcgen05 path of the minibatch gradient (TF32 operands; in-order minibatches only); the fp32 SIMT kernels are the numerics reference
         self.tensor_cores = bool(tensor_cores) and mini_batch_sampling == "in_order"
         self._tc_ws = None
-        self.use_cuda_graph = bool(use_cuda_graph) and mini_batch_sampling == "in_order" and os.environ.get("USV_NO_GRAPH") != "1"
+        self.use_cuda_graph = bool(use_cuda_graph) and mini_batch_sampling == "in_order"
         self._graph = None
         self._gen = torch.Generator(device=self.device)
         self._gen.manual_seed(store.seed)

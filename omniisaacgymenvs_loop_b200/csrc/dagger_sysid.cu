@@ -497,23 +497,14 @@ __global__ void __launch_bounds__(256) mlp_forward_kernel(const float* __restric
   }
 }
 
-static int num_sms() {
-  static int n = 0;
-  if (!n) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
-  }
-  return n;
-}
-
 template <int T>
 static int launch_forward(const float* prm, const float* hist, int64_t ld, int In, int Out, float* out, int64_t M, cudaStream_t st) {
   const size_t smem = fwd_smem_bytes<T>(In, Out);
   if (smem > 227 * 1024) return USV_E_SIZE;
-  cudaFuncSetAttribute(encoder_forward_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  usv::ensure_dynamic_smem(encoder_forward_kernel<T>, smem);
   const int64_t want = (M + kWarps - 1) / kWarps;
-  const int grid = (int)(want < num_sms() ? want : num_sms());
+  const int sms = usv::num_sms();
+  const int grid = (int)(want < sms ? want : sms);
   encoder_forward_kernel<T><<<grid, kThreads, smem, st>>>(prm, hist, ld, In, Out, out, M);
   return usv::finish_launch();
 }
@@ -523,9 +514,10 @@ static int launch_train(const float* prm, const float* hist, int64_t ld, const f
                         cudaStream_t st) {
   const size_t smem = fwd_smem_bytes<T>(In, Out);
   if (smem > 227 * 1024) return USV_E_SIZE;
-  cudaFuncSetAttribute(train_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  usv::ensure_dynamic_smem(train_kernel<T>, smem);
   const int64_t want = (M + kWarps - 1) / kWarps;
-  const int grid = (int)(want < num_sms() ? want : num_sms());
+  const int sms = usv::num_sms();
+  const int grid = (int)(want < sms ? want : sms);
   *nparts = grid;
   train_kernel<T><<<grid, kThreads, smem, st>>>(prm, hist, ld, zstar, In, Out, partial, M);
   return usv::finish_launch();
@@ -606,9 +598,10 @@ int dagger_mlp_forward_f32(const float* params, int32_t n_layers, const int32_t*
   for (int l = 0; l < n_layers; ++l) { d.w[l] = w_offsets[l]; d.b[l] = b_offsets[l]; fl += (size_t)dims[l] * dims[l + 1] + dims[l + 1]; }
   const size_t smem = (((fl + 3) & ~(size_t)3) + 8 * 256) * sizeof(float);
   if (smem > 227 * 1024) return USV_E_SIZE;
-  cudaFuncSetAttribute(mlp_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  usv::ensure_dynamic_smem(mlp_forward_kernel, smem);
   const int64_t want = (M + 7) / 8;
-  const int grid = (int)(want < num_sms() ? want : num_sms());
+  const int sms = usv::num_sms();
+  const int grid = (int)(want < sms ? want : sms);
   mlp_forward_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(params, d, x, x_ld, y, M);
   return usv::finish_launch();
 }

@@ -849,17 +849,6 @@ __global__ void __launch_bounds__(256) adv_norm_kernel(float* __restrict__ adv, 
     adv[q] = sanitize0((adv[q] - mean) / den);
 }
 
-static int g_num_sms = 0;
-static int num_sms() {
-  if (!g_num_sms) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-    if (g_num_sms <= 0) g_num_sms = 148;
-  }
-  return g_num_sms;
-}
-
 static int check_net(const PpoLoopzNet* net) {
   if (!net) return USV_E_NULL;
   if (net->mass_dim < 1 || net->mass_dim > PPO_LOOPZ_MAX_MASS || net->obs_dim <= net->mass_dim || net->obs_dim > PPO_MAX_OBS) return USV_E_SIZE;
@@ -893,10 +882,11 @@ int ppo_loopz_act_f32(const float* params, const PpoLoopzNet* net, const float* 
   if ((do_actor && !actor_obs) || (do_critic && !critic_obs) || (log_prob && !actions && !eval_actions) || (eval_actions && (actions || !log_prob)))
     return USV_E_NULL;
   const size_t smem = smem_floats(net->obs_dim, net->mass_dim, false) * sizeof(float);
-  cudaFuncSetAttribute(act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  usv::ensure_dynamic_smem(act_kernel, smem);
   const int64_t ntiles = (M + TM - 1) / TM;
   const int nn = (do_actor ? 1 : 0) + (do_critic ? 1 : 0);
-  const int cap = num_sms() / nn > 0 ? num_sms() / nn : 1;
+  const int sms = usv::num_sms();
+  const int cap = sms / nn > 0 ? sms / nn : 1;
   const int gx = (int)(ntiles < cap ? ntiles : cap);
   act_kernel<<<dim3(gx, nn), NT, smem, (cudaStream_t)stream>>>(params, *net, do_actor ? 0 : 1, actor_obs, critic_obs, seed, counter,
                                                                counter_offset, row_offset, eval_actions, actions, log_prob, means, values, M);
@@ -929,9 +919,9 @@ int ppo_loopz_minibatch_grad_f32(const float* params, const PpoLoopzNet* net, co
   if (!params || !actor_obs || !critic_obs || !actions || !old_log_prob || !advantages || !target_values || !returns || !lp || !grads || !scratch)
     return USV_E_NULL;
   const size_t smem = smem_floats(net->obs_dim, net->mass_dim, true) * sizeof(float);
-  cudaFuncSetAttribute(train_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  usv::ensure_dynamic_smem(train_kernel, smem);
   const int64_t ntiles = (M + TM - 1) / TM;
-  int gx = num_sms() / 2;
+  int gx = usv::num_sms() / 2;
   if (gx > kMaxParts) gx = kMaxParts;
   if (gx < 1) gx = 1;
   if (ntiles < gx) gx = (int)ntiles;

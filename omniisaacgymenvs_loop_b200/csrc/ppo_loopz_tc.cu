@@ -341,32 +341,25 @@ int ppo_loopz_minibatch_grad_tc(const float* params, const PpoLoopzNet* net, con
   if (sp.IN >= DP) return USV_E_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
   const int md = net->mass_dim, encn = enc_floats(md);
-  const int64_t ld = (M + 127) / 128 * 128;
-  // workspace carve-up (every piece a multiple of 4 floats)
-  float* p = workspace;
-  TrainWs ws;
-  ws.ld = ld;
-  ws.h1t = p; p += H * ld; ws.h2t = p; p += H * ld; ws.dz2t = p; p += H * ld; ws.dz1t = p; p += H * ld;
-  ws.xt = p; p += DP * ld; ws.dz3t = p; p += 16 * ld;
+  // workspace carve-up (every piece a multiple of 4 floats): the T1 / T2 slabs first, whole 128-sample T1 tiles
+  const TrainSetup t = train_setup(workspace, M, TM);
+  const TrainWs& ws = t.ws;
+  const int64_t ld = ws.ld;
+  float* p = ws.dz3t + 16 * ld;
   float* zin = p; p += (2 * M * sp.IN + 7) / 8 * 8;
   float* pk[2]; pk[0] = p; p += PK_TOTAL; pk[1] = p; p += PK_TOTAL;
   float* t1s[2]; float* t2s[2]; float* encs[2];
   for (int k = 0; k < 2; ++k) { t1s[k] = p; p += 160 * 16; }
   for (int k = 0; k < 2; ++k) { t2s[k] = p; p += (size_t)kWgradCtas * slot_stride(Layout(packed_dims(sp.IN, md, 2))); }
   for (int k = 0; k < 2; ++k) { encs[k] = p; p += (size_t)kEncSlots * encn; }
-  const int sms = num_sms();
-  const int64_t ntiles = ld / TM, nchunks = ld / WK, etiles = (M + ETM - 1) / ETM;
-  const int g1 = (int)(ntiles < sms ? ntiles : sms);
-  int g2 = (int)(nchunks < sms ? nchunks : sms);
-  if (g2 > kWgradCtas) g2 = kWgradCtas;
+  const int sms = usv::num_sms();
+  const int64_t etiles = (M + ETM - 1) / ETM;
   int g3 = (int)(etiles < 2 * sms ? etiles : 2 * sms);       // 55 KB of shared memory: two or more CTAs per SM
   if (g3 > kEncSlots) g3 = kEncSlots;
   const size_t smem_ef = (size_t)enc_smem_floats(md) * sizeof(float);
   const size_t smem_eb = (size_t)(enc_smem_floats(md) + 4 * ETM * MS + E3 * H + ETM * MS + encn) * sizeof(float);
-  cudaFuncSetAttribute(enc_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ef);
-  cudaFuncSetAttribute(enc_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_eb);
-  cudaFuncSetAttribute(train_fwd_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)train_smem_bytes());
-  cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wgrad_smem_bytes());
+  usv::ensure_dynamic_smem(enc_fwd_kernel, smem_ef);
+  usv::ensure_dynamic_smem(enc_bwd_kernel, smem_eb);
   cudaMemsetAsync(ws.dz3t, 0, sizeof(float) * 16 * ld, st);               // rows >= 2 of dz3^T are structurally zero
   const int gef = (int)(etiles < 2 * sms ? etiles : 2 * sms);   // x 2 networks: four CTAs per SM (33 KB of shared memory each)
   enc_fwd_kernel<<<dim3(gef, 2), ENT, smem_ef, st>>>(params, *net, actor_obs, critic_obs, zin, M);
@@ -375,13 +368,13 @@ int ppo_loopz_minibatch_grad_tc(const float* params, const PpoLoopzNet* net, con
     const float* prm_net = params + (k == 0 ? 0 : sp.critic);
     const int dims = packed_dims(sp.IN, md, k == 0 ? 2 : 1);
     pack_weights_kernel<<<(PK_TOTAL + 255) / 256, 256, 0, st>>>(prm_net, dims, pk[k]);
-    train_fwd_bwd_tc_kernel<<<g1, NT, train_smem_bytes(), st>>>(prm_net, pk[k], zin + (size_t)k * M * sp.IN, dims, params + sp.std, k, *net, in,
+    train_fwd_bwd_tc_kernel<<<t.g1, NT, train_smem_bytes(), st>>>(prm_net, pk[k], zin + (size_t)k * M * sp.IN, dims, params + sp.std, k, *net, in,
                                                                 *lp, ws, t1s[k], M);
-    wgrad_tc_kernel<<<g2, NT, wgrad_smem_bytes(), st>>>(ws, dims, t2s[k], 0, nchunks);
+    wgrad_tc_kernel<<<t.g2, NT, wgrad_smem_bytes(), st>>>(ws, dims, t2s[k], 0, t.nchunks);
     enc_bwd_kernel<<<g3, ENT, smem_eb, st>>>(prm_net, *net, k == 0 ? actor_obs : critic_obs, ws.dz1t, ld, encs[k], M);
   }
   RedIn ri;
-  for (int k = 0; k < 2; ++k) { ri.t1[k] = t1s[k]; ri.t2[k] = t2s[k]; ri.enc[k] = encs[k]; ri.g1[k] = g1; ri.g2[k] = g2; ri.g3[k] = g3; }
+  for (int k = 0; k < 2; ++k) { ri.t1[k] = t1s[k]; ri.t2[k] = t2s[k]; ri.enc[k] = encs[k]; ri.g1[k] = t.g1; ri.g2[k] = t.g2; ri.g3[k] = g3; }
   const int n = sp.P + PPO_LOOPZ_STAT_COUNT;
   reduce_kernel<<<(n + 63) / 64, 256, 0, st>>>(ri, *net, grads);
   return usv::finish_launch(10);

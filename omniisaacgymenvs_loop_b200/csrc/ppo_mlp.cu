@@ -593,16 +593,6 @@ __global__ void __launch_bounds__(256) rms_update_kernel(const float* __restrict
 __global__ void rms_count_kernel(double* count, double add) { *count += add; }
 __global__ void adam_roll_kernel(float* lr, int* step) { lr[0] = lr[1]; step[0] = step[1]; }
 
-static int g_num_sms = 0;
-static int num_sms() {
-  if (!g_num_sms) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-    if (g_num_sms <= 0) g_num_sms = 148;
-  }
-  return g_num_sms;
-}
 constexpr int kMaxParts = 160;
 
 void launch_reduce(const float* scratch, int nparts, int n, float* grads, const PpoLossParams& lp, int P, cudaStream_t s) {
@@ -628,9 +618,10 @@ int ppo_policy_forward_f32(const float* params, const float* obs, int32_t obs_di
   if (!params || !obs || !obs_mean || !obs_var) return USV_E_NULL;
   if ((value_mean == nullptr) != (value_var == nullptr)) return USV_E_NULL;
   const size_t smem = smem_floats(obs_dim, false) * sizeof(float);
-  cudaFuncSetAttribute(forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  usv::ensure_dynamic_smem(forward_kernel, smem);
   const int64_t ntiles = (M + TM - 1) / TM;
-  const int grid = (int)(ntiles < num_sms() ? ntiles : num_sms());
+  const int sms = usv::num_sms();
+  const int grid = (int)(ntiles < sms ? ntiles : sms);
   forward_kernel<<<grid, NT, smem, (cudaStream_t)stream>>>(params, obs, obs_dim, obs_mean, obs_var, value_mean, value_var, seed,
                                                            counter, counter_offset, row_offset, actions, neglogp, values, mus, sigmas, M);
   return usv::finish_launch();
@@ -647,9 +638,10 @@ int ppo_minibatch_grad_f32(const float* params, const float* obs, int32_t obs_di
   const Layout L(obs_dim);
   const size_t smem = smem_floats(obs_dim, true) * sizeof(float);
   if (smem > 227 * 1024) return USV_E_UNSUPPORTED;
-  cudaFuncSetAttribute(train_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  usv::ensure_dynamic_smem(train_kernel, smem);
   const int64_t ntiles = (M + TM - 1) / TM;
-  int grid = (int)(ntiles < num_sms() ? ntiles : num_sms());
+  const int sms = usv::num_sms();
+  int grid = (int)(ntiles < sms ? ntiles : sms);
   if (grid > kMaxParts) grid = kMaxParts;
   LossIn in{actions, old_neglogp, advantages, old_values, returns, old_mu, old_sigma};
   train_kernel<<<grid, NT, smem, (cudaStream_t)stream>>>(params, obs, obs_dim, obs_mean, obs_var, in, *lp, scratch, M);

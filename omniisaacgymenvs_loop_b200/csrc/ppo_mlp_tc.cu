@@ -18,7 +18,6 @@
 // which remain the numerics reference (DESIGN.md section 6).
 #include <cooperative_groups.h>
 #include <math_constants.h>
-#include <stdlib.h>
 #include <string.h>
 #include "philox.cuh"
 #include "usv_common.cuh"

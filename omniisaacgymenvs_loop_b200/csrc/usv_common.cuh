@@ -3,6 +3,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <atomic>
+#include <map>
+#include <mutex>
+#include <utility>
 #include "../../include/usv_b200.h"
 
 namespace usv {
@@ -16,6 +19,38 @@ inline int finish_launch(int n_launches = 1) {
 }
 
 inline int grid_for(int64_t n, int block) { return (int)((n + block - 1) / block); }
+
+// SM count of the current device, queried once per device; 148 (a B200) when the query fails.  Concurrent first calls on one
+// device store the same value.
+inline int num_sms() {
+  constexpr int kMaxDevices = 64;
+  static std::atomic<int> cached[kMaxDevices];
+  int dev = 0;
+  cudaGetDevice(&dev);
+  const bool keyed = dev >= 0 && dev < kMaxDevices;
+  int n = keyed ? cached[dev].load(std::memory_order_relaxed) : 0;
+  if (n == 0) {
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
+    if (keyed) cached[dev].store(n, std::memory_order_relaxed);
+  }
+  return n;
+}
+
+// Lets `kernel` launch with `bytes` of dynamic shared memory on the current device.  The largest size set per (kernel, device) is
+// remembered and the attribute is set again only when a request exceeds it: some kernels' sizes depend on their arguments.
+inline void ensure_dynamic_smem(const void* kernel, size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> set_bytes;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& have = set_bytes[{kernel, dev}];
+  if (bytes > have && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) == cudaSuccess) have = bytes;
+}
+template <typename... Args>
+inline void ensure_dynamic_smem(void (*kernel)(Args...), size_t bytes) {
+  ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), bytes);
+}
 
 // rotation-matrix rows needed for R^T v with R = quaternion_to_matrix(q), q = (r,i,j,k) real-first,
 // two_s = 2/|q|^2  (public PyTorch3D formula; see oracle/ref_shim.py for the restatement we pin)

@@ -319,8 +319,7 @@ int usv_thruster_target_f32(const float* cmd2, const float* lutL, const float* l
   if (!cmd2 || !lutL || !lutR || !before2) return USV_E_NULL;
   if (((uintptr_t)cmd2 & 7) || ((uintptr_t)before2 & 7) || ((uintptr_t)after2 & 7)) return USV_E_ALIGN;
   const size_t smem = 2 * (size_t)n_lut * sizeof(float);
-  if (smem > 48 * 1024)
-    cudaFuncSetAttribute(thruster_target_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  ensure_dynamic_smem(thruster_target_kernel, smem);
   thruster_target_kernel<<<grid_for(n, 256), 256, smem, (cudaStream_t)stream>>>(
       (const float2*)cmd2, lutL, lutR, n_lut, mL, mR, (float2*)before2, (float2*)after2, n);
   return finish_launch();

@@ -167,10 +167,7 @@ __device__ __forceinline__ void place_obstacles(const UsvStepParams& p, uint64_t
 // (the env's own field slot) -- never seen with the task's obstacle placement, covered by a dense-batch test.
 constexpr int kCostThreads = 512, kCostWarps = kCostThreads / 32;
 constexpr int kAsyncSweepCap = 4 * kMaxSweeps;
-#ifndef USV_SCENE_INNER
-#define USV_SCENE_INNER 16
-#endif
-constexpr int kInner = USV_SCENE_INNER;            // passes of a warp over its tile per outer sweep (a value crosses a tile in <= 8; 12..32 time alike)
+constexpr int kInner = 16;            // passes of a warp over its tile per outer sweep (a value crosses a tile in <= 8; 12..32 time alike)
 constexpr float kJacobiSafeCost = 224.0f;
 
 __device__ __forceinline__ float block_reduce_max_cost(float v, float* s_red) {
@@ -504,10 +501,7 @@ __device__ __forceinline__ float global_vis_inf(const uint32_t* counters, int ha
 
 // field[env] = (G - min G) / (max G - min G + 1e-6) + 0.5 (J - min J) / (max J - min J + 1e-6)  (d_multi_gemini.py:205-271), one cell per
 // thread-iteration; a scene is cut into kFieldChunks row blocks so that ~150 scenes spread over every SM instead of one CTA each
-#ifndef USV_FIELD_CHUNKS
-#define USV_FIELD_CHUNKS 10
-#endif
-constexpr int kFieldThreads = 256, kFieldChunks = USV_FIELD_CHUNKS, kFieldRows = kG / kFieldChunks;   // 15 rows = 2250 cells per item
+constexpr int kFieldThreads = 256, kFieldChunks = 10, kFieldRows = kG / kFieldChunks;   // 15 rows = 2250 cells per item
 static_assert(kFieldRows * kFieldChunks == kG, "row blocks must tile the grid");
 
 __global__ void __launch_bounds__(kFieldThreads) scene_field_kernel(SceneIO io, const uint32_t* __restrict__ counters) {
@@ -582,24 +576,10 @@ __global__ void compact_resets_kernel(const int64_t* __restrict__ reset_buf, int
 
 static size_t cost_smem_bytes() { return (size_t)(kGPR * kGS + 64 + 32 + 2 * kActStride + 160 + 160) * sizeof(float) + (size_t)kTiles * 32 + (size_t)kNearCap * 2; }
 
-static int scene_grid() {
-  static int sms = 0;
-  if (!sms) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0) sms = 148;
-  }
-  return sms;
-}
-
 static int launch_scene(const SceneIO& io, uint32_t* counters, int place, const UsvStepParams* p, const uint64_t* step_offset,
                         cudaStream_t s) {
-  static bool attr = false;
-  if (!attr) {
-    cudaFuncSetAttribute(scene_cost_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cost_smem_bytes());
-    attr = true;
-  }
-  const int grid = scene_grid();
+  ensure_dynamic_smem(scene_cost_kernel, cost_smem_bytes());
+  const int grid = num_sms();
   scene_cost_kernel<<<2 * grid, kCostThreads, cost_smem_bytes(), s>>>(io, counters, place, *p, step_offset);   // two scenes per SM
   scene_field_kernel<<<8 * grid, kFieldThreads, 0, s>>>(io, counters);
   return finish_launch(2);

@@ -14,15 +14,11 @@
 // issue-bound and ends in a partial wave: with 256 x 3 (24 warps per SM, 78 registers) 2^20 envs are 9.23 waves and the last 0.23 runs one
 // CTA per SM for a whole thread's latency; 28 warps per SM make it 7.9 waves.  Same-box A/B at 2^20 envs, 2000 steps (r02): 256 x 3 1.940e10
 // env-steps/s, 160 x 5 1.977, 224 x 4 2.014, 64 x 14 2.016, 128 x 7 2.02-2.05, 32 x 28 2.03; 64 registers (128 x 8, 96 x 10) 1.96-1.97.
-#ifndef USV_BLOCK
-#define USV_BLOCK 128
-#endif
-#ifndef USV_MINB
-#define USV_MINB 7
-#endif
 #include "usv_step_core.cuh"
 
 namespace usv {
+
+constexpr int kBlock = 128, kMinB = 7;   // threads per CTA, CTAs per SM (see above)
 
 // Variant A (classic CaptureXY) task part of a control step: observation (13), reward + penalties, kills / done
 // `what` (USV_TASK_* bits) selects which of the reference's four calls advance their cross-step state: compute_reward owns the goal
@@ -144,10 +140,9 @@ __device__ __forceinline__ void control_step(EnvState& e, EnvConst& k, const Usv
   post_classic(e, k, p, do_reset, first_call, s, o);
 }
 
-__device__ __forceinline__ void accumulate_stats(float* __restrict__ st0, int64_t /*cap*/, int64_t i0, bool was_reset,
+__device__ __forceinline__ void accumulate_stats(float* __restrict__ st0, int64_t i0, bool was_reset,
                                                  const StepOut& o, const UsvStepParams& p) {
   float* __restrict__ st = st0 + tile_base(i0, USV_ST_COUNT);
-  constexpr int i = 0;
   // episode_sums[k][i] += term  [ref SNAP/USV_capture_xy.py:278-306 ; SNAP/USV_task_rewards.py:526-540 ;
   // SNAP/USV_Virtual.py:819-830]; sums are cleared by the reset that precedes this step.
   const float v[USV_ST_COUNT] = {o.dist_rew, o.align_rew, o.speed_rew, o.d, o.speed, o.bpen, o.bdist,
@@ -155,8 +150,8 @@ __device__ __forceinline__ void accumulate_stats(float* __restrict__ st0, int64_
                                  o.speed, o.absw, o.asum};
 #pragma unroll
   for (int f = 0; f < USV_ST_COUNT; ++f) {
-    const float prev = was_reset ? 0.0f : st[f * kTile + i];
-    st[f * kTile + i] = prev + v[f];
+    const float prev = was_reset ? 0.0f : st[f * kTile];
+    st[f * kTile] = prev + v[f];
   }
 }
 
@@ -189,7 +184,7 @@ __device__ __forceinline__ void write_obs_tile(float* s_obs, const StepOut& o, b
 }
 
 template <int kDisturb, bool kStats>
-__global__ void __launch_bounds__(kBlock, USV_MINB) step_fused_kernel(UsvEnvBuffers b, const float2* __restrict__ actions,
+__global__ void __launch_bounds__(kBlock, kMinB) step_fused_kernel(UsvEnvBuffers b, const float2* __restrict__ actions,
                                                             float* __restrict__ obs, float* __restrict__ rew,
                                                             int64_t n, const __grid_constant__ UsvStepParams p) {
   extern __shared__ __align__(16) float smem[];
@@ -207,8 +202,8 @@ __global__ void __launch_bounds__(kBlock, USV_MINB) step_fused_kernel(UsvEnvBuff
   bool do_reset = false;
   float2 act = make_float2(0.f, 0.f);
   if (active) {
-    load_state(b.state, b.state_stride, i, e);
-    load_consts<kDisturb>(b.consts, b.consts_stride, i, k);
+    load_state(b.state, i, e);
+    load_consts<kDisturb>(b.consts, i, k);
     do_reset = b.reset_buf[i] != 0;
     act = actions[i];
   }
@@ -216,9 +211,9 @@ __global__ void __launch_bounds__(kBlock, USV_MINB) step_fused_kernel(UsvEnvBuff
   if (active) {
     control_step<kDisturb, true>(e, k, p, do_reset, act, (uint64_t)(p.env_id_offset + i), i, p.step_counter + (b.step_offset ? *b.step_offset : 0ull),
                                  p.first_call != 0, s_lutL, s_lutR, o);
-    store_state(b.state, b.state_stride, i, e);
-    if (do_reset) store_consts<kDisturb>(b.consts, b.consts_stride, i, k);
-    if (kStats) accumulate_stats(b.stats, b.stats_stride, i, do_reset, o, p);
+    store_state(b.state, i, e);
+    if (do_reset) store_consts<kDisturb>(b.consts, i, k);
+    if (kStats) accumulate_stats(b.stats, i, do_reset, o, p);
     rew[i] = o.rew;
     b.reset_buf[i] = (int64_t)o.done;
     if (b.nonfinite_flag) {
@@ -253,8 +248,8 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(UsvEnvBuffers b, 
   bool do_reset = false;
   bool consts_dirty = false;
   if (active) {
-    load_state(b.state, b.state_stride, i, e);
-    load_consts<kDisturb>(b.consts, b.consts_stride, i, k);
+    load_state(b.state, i, e);
+    load_consts<kDisturb>(b.consts, i, k);
     do_reset = b.reset_buf[i] != 0;
   }
   __syncthreads();
@@ -268,7 +263,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(UsvEnvBuffers b, 
       control_step<kDisturb, false>(e, k, p, do_reset, act, (uint64_t)(p.env_id_offset + i), i, step0 + (uint64_t)t,
                              first_call, s_lutL, s_lutR, o);
       consts_dirty |= do_reset;
-      if (kStats) accumulate_stats(b.stats, b.stats_stride, i, do_reset, o, p);
+      if (kStats) accumulate_stats(b.stats, i, do_reset, o, p);
       if (rew) rew[(int64_t)t * n + i] = o.rew;
       if (done) done[(int64_t)t * n + i] = (int64_t)o.done;
       bad |= !o.finite || !isfinite(act.x) || !isfinite(act.y);
@@ -280,8 +275,8 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(UsvEnvBuffers b, 
     }
   }
   if (active) {
-    store_state(b.state, b.state_stride, i, e);
-    if (consts_dirty) store_consts<kDisturb>(b.consts, b.consts_stride, i, k);
+    store_state(b.state, i, e);
+    if (consts_dirty) store_consts<kDisturb>(b.consts, i, k);
     b.reset_buf[i] = do_reset ? 1 : 0;
     if (b.nonfinite_flag && bad) atomicOr(b.nonfinite_flag, 1u);
   }
@@ -294,8 +289,8 @@ __global__ void __launch_bounds__(kBlock) planar_forces_kernel(UsvEnvBuffers b, 
   if (i >= n) return;
   EnvState e;
   EnvConst k;
-  load_state(b.state, b.state_stride, i, e);
-  load_consts<kDisturb>(b.consts, b.consts_stride, i, k);
+  load_state(b.state, i, e);
+  load_consts<kDisturb>(b.consts, i, k);
   float ox = 0.0f, oy = 0.0f;
   if (kDisturb && p.envs_per_row > 0) {
     ox = p.grid_row_offset - (float)(int)(i / p.envs_per_row) * p.env_spacing;
@@ -308,31 +303,8 @@ __global__ void __launch_bounds__(kBlock) planar_forces_kernel(UsvEnvBuffers b, 
   o[0] = du; o[1] = dv; o[2] = dr; o[3] = Fx; o[4] = Fy; o[5] = Tz; o[6] = ax; o[7] = ay;
 }
 
-static int check_common(const UsvEnvBuffers* b, int64_t n, const UsvStepParams* p) {
-  if (!b || !p) return USV_E_NULL;
-  if (n < 0) return USV_E_SIZE;
-  if (!b->state || !b->consts || !b->reset_buf || !b->lut_left || !b->lut_right) return USV_E_NULL;
-  if (b->state_stride < n || b->consts_stride < n || (b->state_stride & 31) || (b->consts_stride & 31)) return USV_E_SIZE;
-  if (b->stats && (b->stats_stride < n || (b->stats_stride & 31))) return USV_E_SIZE;
-  if (p->n_lut < 2 || p->n_lut > 8192) return USV_E_PARAM;
-  if (p->n_substeps < 0 || p->n_substeps > 1024) return USV_E_PARAM;
-  if (!(p->izz > 0.0f)) return USV_E_PARAM;
-  if (p->reward_mode < USV_REWARD_LINEAR || p->reward_mode > USV_REWARD_EXPONENTIAL) return USV_E_PARAM;
-  return USV_OK;
-}
-
-static bool wants_disturb(const UsvStepParams* p) {
-  return p->use_force_disturbance || p->use_torque_disturbance || p->use_const_force || p->use_sin_force ||
-         p->use_const_torque || p->use_sin_torque || p->use_water_current;   // a water current rides in the generic variant
-}
-
 static size_t step_smem(const UsvStepParams* p) { return (size_t)(kBlock * kObs + 2 * p->n_lut) * sizeof(float); }
 static size_t step_smem_nolut() { return (size_t)(kBlock * kObs) * sizeof(float); }
-
-template <typename K>
-static void ensure_smem(K kernel, size_t smem) {
-  if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-}
 
 // CaptureXYTask.get_state_observations / compute_reward / update_kills and Penalties.compute_penalty on the caller's own state tensors:
 // the SAME device code as the task part of the fused step (post_classic), one env per thread, plain row-major inputs.
@@ -430,7 +402,7 @@ int usv_step_fused_f32(const UsvEnvBuffers* b, const float* actions, float* obs,
   cudaStream_t s = (cudaStream_t)stream;
 #define USV_LAUNCH_STEP(D, S)                                                                              \
   do {                                                                                                     \
-    ensure_smem(step_fused_kernel<D, S>, smem);                                                            \
+    ensure_dynamic_smem(step_fused_kernel<D, S>, smem);                                                    \
     step_fused_kernel<D, S><<<grid, kBlock, smem, s>>>(*b, (const float2*)actions, obs, rew, n, *p);       \
   } while (0)
   const bool all4 = p->use_const_force && p->use_sin_force && p->use_const_torque && p->use_sin_torque && !p->use_water_current;
@@ -457,7 +429,7 @@ int usv_rollout_fused_f32(const UsvEnvBuffers* b, const float* actions, float* o
   cudaStream_t s = (cudaStream_t)stream;
 #define USV_LAUNCH_ROLL(D, S)                                                                              \
   do {                                                                                                     \
-    ensure_smem(rollout_fused_kernel<D, S>, smem);                                                         \
+    ensure_dynamic_smem(rollout_fused_kernel<D, S>, smem);                                                 \
     rollout_fused_kernel<D, S><<<grid, kBlock, smem, s>>>(*b, (const float2*)actions, obs, rew, done, T, n, *p); \
   } while (0)
   if (dis && st) USV_LAUNCH_ROLL(true, true);

@@ -7,11 +7,11 @@
 //
 // HBM traffic per env-step (stats off, no disturbances): state 13+3 fields r/w (128 B), consts 13+35 fields (192 B), 4 field
 // taps (<= 4 x 32 B sectors), obs 132 B, action 8 B, reward 4 B, reset_buf 16 B  ->  ~610 B.
-#include <stdlib.h>
 #include "usv_step_core.cuh"
 
 namespace usv {
 
+constexpr int kBlock = 256;   // threads per CTA; CTAs per SM are the kernels' kMinB / __launch_bounds__ arguments
 constexpr int kObsB = USV_B_OBS;
 constexpr int kGridB = USV_B_GRID;
 
@@ -367,8 +367,8 @@ __global__ void __launch_bounds__(kB, kMinB) step_live_kernel(UsvEnvBuffers b, U
   float* __restrict__ bs = lb.bstate + tile_base(active ? i : 0, USV_BS_COUNT);
   float* __restrict__ bc = lb.bconsts + tile_base(active ? i : 0, USV_BC_COUNT);
   if (active) {
-    load_state(b.state, b.state_stride, i, e);
-    load_consts<kDisturb>(b.consts, b.consts_stride, i, k);
+    load_state(b.state, i, e);
+    load_consts<kDisturb>(b.consts, i, k);
     ls.prev_h = bs[USV_BS_PREV_H * kTile];
     ls.prev_pot = bs[USV_BS_PREV_POT * kTile];
     ls.outcome = __float_as_int(bs[USV_BS_OUTCOME * kTile]);
@@ -394,8 +394,8 @@ __global__ void __launch_bounds__(kB, kMinB) step_live_kernel(UsvEnvBuffers b, U
       for (int j = 0; j < 3; ++j) bcs[(USV_BC_COM_X + j) * kTile] = bc[(USV_BC_COM_X + j) * kTile];
     }
     post_live<kStats>(e, k, ls, bcs, lb.field + i * (int64_t)(kGridB * kGridB), p, lp, do_reset, any_reset, p.first_call != 0, s, o);
-    store_state(b.state, b.state_stride, i, e);
-    if (do_reset) store_consts<kDisturb>(b.consts, b.consts_stride, i, k);
+    store_state(b.state, i, e);
+    if (do_reset) store_consts<kDisturb>(b.consts, i, k);
     bs[USV_BS_PREV_H * kTile] = ls.prev_h;
     bs[USV_BS_PREV_POT * kTile] = ls.prev_pot;
     bs[USV_BS_OUTCOME * kTile] = __int_as_float(ls.outcome);
@@ -538,8 +538,8 @@ __global__ void __launch_bounds__(kBlock, 3) step_task_kernel(UsvEnvBuffers b, U
   if (active) {
     EnvState e;
     EnvConst k;
-    load_state(b.state, b.state_stride, i, e);
-    load_consts<kDisturb>(b.consts, b.consts_stride, i, k);
+    load_state(b.state, i, e);
+    load_consts<kDisturb>(b.consts, i, k);
     float* __restrict__ bc = lb.bconsts + tile_base(i, USV_BC_COUNT);
     const bool do_reset = b.reset_buf[i] != 0;
     const float2 act = actions[i];
@@ -560,8 +560,8 @@ __global__ void __launch_bounds__(kBlock, 3) step_task_kernel(UsvEnvBuffers b, U
     DynOut s;
     step_dynamics<kDisturb, true>(e, k, p, do_reset, act, gid, i, step, b.lut_left, b.lut_right, s);
     post_task<kTask>(e, k, bc, p, lp, do_reset, p.first_call != 0, s, o);
-    store_state(b.state, b.state_stride, i, e);
-    if (do_reset) store_consts<kDisturb>(b.consts, b.consts_stride, i, k);
+    store_state(b.state, i, e);
+    if (do_reset) store_consts<kDisturb>(b.consts, i, k);
     rew[i] = o.rew;
     b.reset_buf[i] = (int64_t)o.done;
     if (b.nonfinite_flag) {
@@ -578,66 +578,43 @@ using namespace usv;
 
 extern "C" int usv_step_live_f32(const UsvEnvBuffers* b, const UsvLiveBuffers* lb, const float* actions, float* obs, float* rew,
                                  int64_t n, const UsvStepParams* p, const UsvLiveParams* lp, void* stream) {
-  if (!b || !lb || !p || !lp) return USV_E_NULL;
-  if (n < 0) return USV_E_SIZE;
-  if (!b->state || !b->consts || !b->reset_buf || !b->lut_left || !b->lut_right) return USV_E_NULL;
+  if (!lb || !lp) return USV_E_NULL;
+  int rc = check_common(b, n, p);
+  if (rc) return rc;
   if (lp->task < USV_TASK_CAPTURE_OBSTACLES || lp->task > USV_TASK_TRACK_XY_VELOCITY) return USV_E_PARAM;
   const bool obst = lp->task == USV_TASK_CAPTURE_OBSTACLES;
   if (!lb->bconsts || (obst && (!lb->bstate || !lb->field || !lb->reset_epoch))) return USV_E_NULL;
-  if (b->state_stride < n || b->consts_stride < n || (b->state_stride & 31) || (b->consts_stride & 31)) return USV_E_SIZE;
   if (lb->bconsts_stride < n || (lb->bconsts_stride & 31)) return USV_E_SIZE;
   if (obst && (lb->bstate_stride < n || (lb->bstate_stride & 31))) return USV_E_SIZE;
   if (lb->bstats && (lb->bstats_stride < n || (lb->bstats_stride & 31))) return USV_E_SIZE;
-  if (p->n_lut < 2 || p->n_lut > 8192) return USV_E_PARAM;
-  if (p->n_substeps < 0 || p->n_substeps > 1024) return USV_E_PARAM;
-  if (!(p->izz > 0.0f) || !(lp->map_size > 0.0f)) return USV_E_PARAM;
+  if (!(lp->map_size > 0.0f)) return USV_E_PARAM;
   if (lp->priv_mode < USV_PRIV_RAW || lp->priv_mode > USV_PRIV_MINMAX) return USV_E_PARAM;
   if (lp->priv_dim != 0 && lp->priv_dim != 4 && lp->priv_dim != 8) return USV_E_PARAM;
   if (n == 0) return USV_OK;
   if (!actions || !obs || !rew) return USV_E_NULL;
   if ((uintptr_t)actions & 7) return USV_E_ALIGN;
-  const size_t smem = (size_t)kBlock * kObsB * sizeof(float);
-  const size_t smem_live = smem + (size_t)(kBlock / 32) * USV_BC_COUNT * kTile * sizeof(float);   // + the staged bconsts tiles
-  static bool attr = false;
-  if (!attr) {
-    cudaFuncSetAttribute(step_live_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_live);
-    cudaFuncSetAttribute(step_live_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_live);
-    cudaFuncSetAttribute(step_live_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_live);
-    cudaFuncSetAttribute(step_live_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_live);
-    cudaFuncSetAttribute(step_live_kernel<true, false, true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_live);
-    cudaFuncSetAttribute(step_live_kernel<false, false, true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_live);
-    attr = true;
-  }
   const int grid = grid_for(n, kBlock);
-  const bool dis = p->use_force_disturbance || p->use_torque_disturbance || p->use_const_force || p->use_sin_force ||
-                   p->use_const_torque || p->use_sin_torque || p->use_water_current;
-  const bool st = lb->bstats != nullptr;
-  cudaStream_t s = (cudaStream_t)stream;
+  const bool dis = wants_disturb(p), st = lb->bstats != nullptr;
   // staged bconsts (cp.async into shared memory) vs direct loads, A/B on one B200 (r02, profiles/r02_live_kernels.md): 13.9 vs 14.9 us at
   // 16 384 envs, 16.8 vs 18.4 at 65 536, 41.5 vs 44.7 at 131 072 -- but 83.5 vs 76.1 us at 262 144, where the 24 GB of per-env fields make
-  // every tap a DRAM access and the 36 KB of extra shared memory per CTA cost more L1 than the staging saves.  USV_LIVE_NO_STAGE / USV_LIVE_STAGE
-  // force one of them (profiling runs).
-  static const int force = getenv("USV_LIVE_NO_STAGE") ? 0 : (getenv("USV_LIVE_STAGE") ? 1 : -1);
-  const bool no_stage = force >= 0 ? force == 0 : n > 196608;
+  // every tap a DRAM access and the 36 KB of extra shared memory per CTA cost more L1 than the staging saves.
+  const bool no_stage = n > 196608;
   // one wave at two CTAs per SM (and no statistics: the rarely used stats build stays on one register budget)
-  static const int sms = [] { int d = 0, v = 0; cudaGetDevice(&d); return (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, d) == cudaSuccess && v > 0) ? v : 148; }();
-  static const bool force3 = getenv("USV_LIVE_MINB3") != nullptr;      // profiling runs: always the 80-register build
-  const bool one_wave = !no_stage && grid <= 2 * sms && !force3;
-#define USV_LAUNCH_LIVE(D, S)                                                                                                      \
-  do {                                                                                                                             \
-    if (no_stage) step_live_kernel<D, S, false><<<grid, kBlock, smem, s>>>(*b, *lb, (const float2*)actions, obs, rew, n, *p, *lp);  \
-    else if (one_wave && !S) step_live_kernel<D, false, true, 2><<<grid, kBlock, smem_live, s>>>(*b, *lb, (const float2*)actions, obs, rew, n, *p, *lp); \
-    else step_live_kernel<D, S, true><<<grid, kBlock, smem_live, s>>>(*b, *lb, (const float2*)actions, obs, rew, n, *p, *lp);       \
-  } while (0)
-#define USV_LAUNCH_TASK(T, D) step_task_kernel<T, D><<<grid, kBlock, smem, s>>>(*b, *lb, (const float2*)actions, obs, rew, n, *p, *lp)
-  if (lp->task == USV_TASK_GO_TO_POSE) { if (dis) USV_LAUNCH_TASK(USV_TASK_GO_TO_POSE, true); else USV_LAUNCH_TASK(USV_TASK_GO_TO_POSE, false); }
-  else if (lp->task == USV_TASK_KEEP_XY) { if (dis) USV_LAUNCH_TASK(USV_TASK_KEEP_XY, true); else USV_LAUNCH_TASK(USV_TASK_KEEP_XY, false); }
-  else if (lp->task == USV_TASK_TRACK_XY_VELOCITY) { if (dis) USV_LAUNCH_TASK(USV_TASK_TRACK_XY_VELOCITY, true); else USV_LAUNCH_TASK(USV_TASK_TRACK_XY_VELOCITY, false); }
-  else if (dis && st) USV_LAUNCH_LIVE(true, true);
-  else if (dis) USV_LAUNCH_LIVE(true, false);
-  else if (st) USV_LAUNCH_LIVE(false, true);
-  else USV_LAUNCH_LIVE(false, false);
-#undef USV_LAUNCH_LIVE
-#undef USV_LAUNCH_TASK
+  const bool one_wave = !no_stage && grid <= 2 * num_sms();
+  decltype(&step_live_kernel<false, false>) kernel;
+#define USV_LIVE_KERNEL(D, S) \
+  (no_stage ? step_live_kernel<D, S, false> : (one_wave && !S) ? step_live_kernel<D, false, true, 2> : step_live_kernel<D, S, true>)
+#define USV_TASK_KERNEL(T) (dis ? step_task_kernel<T, true> : step_task_kernel<T, false>)
+  if (lp->task == USV_TASK_GO_TO_POSE) kernel = USV_TASK_KERNEL(USV_TASK_GO_TO_POSE);
+  else if (lp->task == USV_TASK_KEEP_XY) kernel = USV_TASK_KERNEL(USV_TASK_KEEP_XY);
+  else if (lp->task == USV_TASK_TRACK_XY_VELOCITY) kernel = USV_TASK_KERNEL(USV_TASK_TRACK_XY_VELOCITY);
+  else if (dis) kernel = st ? USV_LIVE_KERNEL(true, true) : USV_LIVE_KERNEL(true, false);
+  else kernel = st ? USV_LIVE_KERNEL(false, true) : USV_LIVE_KERNEL(false, false);
+#undef USV_LIVE_KERNEL
+#undef USV_TASK_KERNEL
+  size_t smem = (size_t)kBlock * kObsB * sizeof(float);
+  if (obst && !no_stage) smem += (size_t)(kBlock / 32) * USV_BC_COUNT * kTile * sizeof(float);   // + the staged bconsts tiles
+  ensure_dynamic_smem(kernel, smem);
+  kernel<<<grid, kBlock, smem, (cudaStream_t)stream>>>(*b, *lb, (const float2*)actions, obs, rew, n, *p, *lp);
   return finish_launch();
 }

@@ -1,5 +1,6 @@
 // Shared device code of the fused ASV step kernels (Variant A classic / Variant B live): AoSoA state access, branch-free
-// trigonometry, per-episode reset randomisation, the planar force model and the action->physics part of a control step.
+// trigonometry, per-episode reset randomisation, the planar force model and the action->physics part of a control step; plus the
+// host-side argument checks both step entry points share.
 #pragma once
 #include <math_constants.h>
 #include "philox.cuh"
@@ -7,13 +8,6 @@
 
 namespace usv {
 
-#ifndef USV_BLOCK
-#define USV_BLOCK 256
-#endif
-#ifndef USV_MINB
-#define USV_MINB 3
-#endif
-constexpr int kBlock = USV_BLOCK;
 constexpr int kObs = 13;
 // python: math.pi / 2*math.pi are doubles that meet fp32 tensors -> rounded to fp32
 #define USV_PI_F 3.14159274101257324f
@@ -44,107 +38,102 @@ struct StepOut {
 // ~100 of the 1678 instructions per env-step in the r01 profile).
 constexpr int kTile = 32;
 __device__ __forceinline__ int64_t tile_base(int64_t i, int count) { return (i >> 5) * (int64_t)(count * kTile) + (i & 31); }
-#define stride kTile
 
-__device__ __forceinline__ void load_state(const float* __restrict__ s0, int64_t /*cap*/, int64_t i0, EnvState& e) {
+__device__ __forceinline__ void load_state(const float* __restrict__ s0, int64_t i0, EnvState& e) {
   const float* __restrict__ s = s0 + tile_base(i0, USV_S_COUNT);
-  constexpr int i = 0;
-  e.x = s[USV_S_X * stride + i];
-  e.y = s[USV_S_Y * stride + i];
-  e.psi = s[USV_S_PSI * stride + i];
-  e.vx = s[USV_S_VX * stride + i];
-  e.vy = s[USV_S_VY * stride + i];
-  e.r = s[USV_S_R * stride + i];
-  e.thrL = s[USV_S_THR_L * stride + i];
-  e.thrR = s[USV_S_THR_R * stride + i];
-  e.prev_d = s[USV_S_PREV_D * stride + i];
-  e.prev_w = s[USV_S_PREV_W * stride + i];
-  e.prev_asum = s[USV_S_PREV_ASUM * stride + i];
-  e.goal_cnt = __float_as_int(s[USV_S_GOAL_CNT * stride + i]);
-  e.progress = __float_as_int(s[USV_S_PROGRESS * stride + i]);
+  e.x = s[USV_S_X * kTile];
+  e.y = s[USV_S_Y * kTile];
+  e.psi = s[USV_S_PSI * kTile];
+  e.vx = s[USV_S_VX * kTile];
+  e.vy = s[USV_S_VY * kTile];
+  e.r = s[USV_S_R * kTile];
+  e.thrL = s[USV_S_THR_L * kTile];
+  e.thrR = s[USV_S_THR_R * kTile];
+  e.prev_d = s[USV_S_PREV_D * kTile];
+  e.prev_w = s[USV_S_PREV_W * kTile];
+  e.prev_asum = s[USV_S_PREV_ASUM * kTile];
+  e.goal_cnt = __float_as_int(s[USV_S_GOAL_CNT * kTile]);
+  e.progress = __float_as_int(s[USV_S_PROGRESS * kTile]);
 }
 
-__device__ __forceinline__ void store_state(float* __restrict__ s0, int64_t /*cap*/, int64_t i0, const EnvState& e) {
+__device__ __forceinline__ void store_state(float* __restrict__ s0, int64_t i0, const EnvState& e) {
   float* __restrict__ s = s0 + tile_base(i0, USV_S_COUNT);
-  constexpr int i = 0;
-  s[USV_S_X * stride + i] = e.x;
-  s[USV_S_Y * stride + i] = e.y;
-  s[USV_S_PSI * stride + i] = e.psi;
-  s[USV_S_VX * stride + i] = e.vx;
-  s[USV_S_VY * stride + i] = e.vy;
-  s[USV_S_R * stride + i] = e.r;
-  s[USV_S_THR_L * stride + i] = e.thrL;
-  s[USV_S_THR_R * stride + i] = e.thrR;
-  s[USV_S_PREV_D * stride + i] = e.prev_d;
-  s[USV_S_PREV_W * stride + i] = e.prev_w;
-  s[USV_S_PREV_ASUM * stride + i] = e.prev_asum;
-  s[USV_S_GOAL_CNT * stride + i] = __int_as_float(e.goal_cnt);
-  s[USV_S_PROGRESS * stride + i] = __int_as_float(e.progress);
+  s[USV_S_X * kTile] = e.x;
+  s[USV_S_Y * kTile] = e.y;
+  s[USV_S_PSI * kTile] = e.psi;
+  s[USV_S_VX * kTile] = e.vx;
+  s[USV_S_VY * kTile] = e.vy;
+  s[USV_S_R * kTile] = e.r;
+  s[USV_S_THR_L * kTile] = e.thrL;
+  s[USV_S_THR_R * kTile] = e.thrR;
+  s[USV_S_PREV_D * kTile] = e.prev_d;
+  s[USV_S_PREV_W * kTile] = e.prev_w;
+  s[USV_S_PREV_ASUM * kTile] = e.prev_asum;
+  s[USV_S_GOAL_CNT * kTile] = __int_as_float(e.goal_cnt);
+  s[USV_S_PROGRESS * kTile] = __int_as_float(e.progress);
 }
 
 template <int kDisturb>
-__device__ __forceinline__ void load_consts(const float* __restrict__ c0, int64_t /*cap*/, int64_t i0, EnvConst& k) {
+__device__ __forceinline__ void load_consts(const float* __restrict__ c0, int64_t i0, EnvConst& k) {
   const float* __restrict__ c = c0 + tile_base(i0, USV_C_COUNT);
-  constexpr int i = 0;
-  k.tx = c[USV_C_TX * stride + i];
-  k.ty = c[USV_C_TY * stride + i];
-  k.mass = c[USV_C_MASS * stride + i];
-  k.linu = c[USV_C_LIN_U * stride + i];
-  k.linv = c[USV_C_LIN_V * stride + i];
-  k.linr = c[USV_C_LIN_R * stride + i];
-  k.quadu = c[USV_C_QUAD_U * stride + i];
-  k.quadv = c[USV_C_QUAD_V * stride + i];
-  k.quadr = c[USV_C_QUAD_R * stride + i];
-  k.kdrag = c[USV_C_KDRAG * stride + i];
-  k.mL = c[USV_C_THR_ML * stride + i];
-  k.mR = c[USV_C_THR_MR * stride + i];
-  k.kiz = c[USV_C_KIZ * stride + i];
+  k.tx = c[USV_C_TX * kTile];
+  k.ty = c[USV_C_TY * kTile];
+  k.mass = c[USV_C_MASS * kTile];
+  k.linu = c[USV_C_LIN_U * kTile];
+  k.linv = c[USV_C_LIN_V * kTile];
+  k.linr = c[USV_C_LIN_R * kTile];
+  k.quadu = c[USV_C_QUAD_U * kTile];
+  k.quadv = c[USV_C_QUAD_V * kTile];
+  k.quadr = c[USV_C_QUAD_R * kTile];
+  k.kdrag = c[USV_C_KDRAG * kTile];
+  k.mL = c[USV_C_THR_ML * kTile];
+  k.mR = c[USV_C_THR_MR * kTile];
+  k.kiz = c[USV_C_KIZ * kTile];
   if (kDisturb) {
-    k.fcx = c[USV_C_FCX * stride + i];
-    k.fcy = c[USV_C_FCY * stride + i];
-    k.fxf = c[USV_C_FXF * stride + i];
-    k.fyf = c[USV_C_FYF * stride + i];
-    k.fxs = c[USV_C_FXS * stride + i];
-    k.fys = c[USV_C_FYS * stride + i];
-    k.famp = c[USV_C_FAMP * stride + i];
-    k.tc = c[USV_C_TC * stride + i];
-    k.tf = c[USV_C_TF * stride + i];
-    k.ts = c[USV_C_TS * stride + i];
-    k.tamp = c[USV_C_TAMP * stride + i];
+    k.fcx = c[USV_C_FCX * kTile];
+    k.fcy = c[USV_C_FCY * kTile];
+    k.fxf = c[USV_C_FXF * kTile];
+    k.fyf = c[USV_C_FYF * kTile];
+    k.fxs = c[USV_C_FXS * kTile];
+    k.fys = c[USV_C_FYS * kTile];
+    k.famp = c[USV_C_FAMP * kTile];
+    k.tc = c[USV_C_TC * kTile];
+    k.tf = c[USV_C_TF * kTile];
+    k.ts = c[USV_C_TS * kTile];
+    k.tamp = c[USV_C_TAMP * kTile];
   } else {
     k.fcx = k.fcy = k.fxf = k.fyf = k.fxs = k.fys = k.famp = k.tc = k.tf = k.ts = k.tamp = 0.0f;
   }
 }
 
 template <int kDisturb>
-__device__ __forceinline__ void store_consts(float* __restrict__ c0, int64_t /*cap*/, int64_t i0, const EnvConst& k) {
+__device__ __forceinline__ void store_consts(float* __restrict__ c0, int64_t i0, const EnvConst& k) {
   float* __restrict__ c = c0 + tile_base(i0, USV_C_COUNT);
-  constexpr int i = 0;
-  c[USV_C_TX * stride + i] = k.tx;
-  c[USV_C_TY * stride + i] = k.ty;
-  c[USV_C_MASS * stride + i] = k.mass;
-  c[USV_C_LIN_U * stride + i] = k.linu;
-  c[USV_C_LIN_V * stride + i] = k.linv;
-  c[USV_C_LIN_R * stride + i] = k.linr;
-  c[USV_C_QUAD_U * stride + i] = k.quadu;
-  c[USV_C_QUAD_V * stride + i] = k.quadv;
-  c[USV_C_QUAD_R * stride + i] = k.quadr;
-  c[USV_C_KDRAG * stride + i] = k.kdrag;
-  c[USV_C_THR_ML * stride + i] = k.mL;
-  c[USV_C_THR_MR * stride + i] = k.mR;
-  c[USV_C_KIZ * stride + i] = k.kiz;
+  c[USV_C_TX * kTile] = k.tx;
+  c[USV_C_TY * kTile] = k.ty;
+  c[USV_C_MASS * kTile] = k.mass;
+  c[USV_C_LIN_U * kTile] = k.linu;
+  c[USV_C_LIN_V * kTile] = k.linv;
+  c[USV_C_LIN_R * kTile] = k.linr;
+  c[USV_C_QUAD_U * kTile] = k.quadu;
+  c[USV_C_QUAD_V * kTile] = k.quadv;
+  c[USV_C_QUAD_R * kTile] = k.quadr;
+  c[USV_C_KDRAG * kTile] = k.kdrag;
+  c[USV_C_THR_ML * kTile] = k.mL;
+  c[USV_C_THR_MR * kTile] = k.mR;
+  c[USV_C_KIZ * kTile] = k.kiz;
   if (kDisturb) {
-    c[USV_C_FCX * stride + i] = k.fcx;
-    c[USV_C_FCY * stride + i] = k.fcy;
-    c[USV_C_FXF * stride + i] = k.fxf;
-    c[USV_C_FYF * stride + i] = k.fyf;
-    c[USV_C_FXS * stride + i] = k.fxs;
-    c[USV_C_FYS * stride + i] = k.fys;
-    c[USV_C_FAMP * stride + i] = k.famp;
-    c[USV_C_TC * stride + i] = k.tc;
-    c[USV_C_TF * stride + i] = k.tf;
-    c[USV_C_TS * stride + i] = k.ts;
-    c[USV_C_TAMP * stride + i] = k.tamp;
+    c[USV_C_FCX * kTile] = k.fcx;
+    c[USV_C_FCY * kTile] = k.fcy;
+    c[USV_C_FXF * kTile] = k.fxf;
+    c[USV_C_FYF * kTile] = k.fyf;
+    c[USV_C_FXS * kTile] = k.fxs;
+    c[USV_C_FYS * kTile] = k.fys;
+    c[USV_C_FAMP * kTile] = k.famp;
+    c[USV_C_TC * kTile] = k.tc;
+    c[USV_C_TF * kTile] = k.tf;
+    c[USV_C_TS * kTile] = k.ts;
+    c[USV_C_TAMP * kTile] = k.tamp;
   }
 }
 
@@ -562,6 +551,23 @@ __device__ __forceinline__ void step_dynamics(EnvState& e, EnvConst& k, const Us
   s.pxn = pxn; s.pyn = pyn; s.vxn = vxn; s.vyn = vyn; s.wn = wn; s.yawn = yawn; s.hs = hs; s.hc = hc;
 }
 
-#undef stride
+// argument checks shared by the step entry points (classic and live)
+inline int check_common(const UsvEnvBuffers* b, int64_t n, const UsvStepParams* p) {
+  if (!b || !p) return USV_E_NULL;
+  if (n < 0) return USV_E_SIZE;
+  if (!b->state || !b->consts || !b->reset_buf || !b->lut_left || !b->lut_right) return USV_E_NULL;
+  if (b->state_stride < n || b->consts_stride < n || (b->state_stride & 31) || (b->consts_stride & 31)) return USV_E_SIZE;
+  if (b->stats && (b->stats_stride < n || (b->stats_stride & 31))) return USV_E_SIZE;
+  if (p->n_lut < 2 || p->n_lut > 8192) return USV_E_PARAM;
+  if (p->n_substeps < 0 || p->n_substeps > 1024) return USV_E_PARAM;
+  if (!(p->izz > 0.0f)) return USV_E_PARAM;
+  if (p->reward_mode < USV_REWARD_LINEAR || p->reward_mode > USV_REWARD_EXPONENTIAL) return USV_E_PARAM;
+  return USV_OK;
+}
+
+inline bool wants_disturb(const UsvStepParams* p) {
+  return p->use_force_disturbance || p->use_torque_disturbance || p->use_const_force || p->use_sin_force ||
+         p->use_const_torque || p->use_sin_torque || p->use_water_current;   // a water current rides in the generic variant
+}
 
 }  // namespace usv

@@ -48,7 +48,7 @@ class LoopzRunner:
         dev = ppo.device
         self.task = env._task
         self.engine = getattr(self.task, "engine", None)
-        self.use_cuda_graph = bool(use_cuda_graph) and os.environ.get("USV_NO_GRAPH") != "1" and self.engine is not None
+        self.use_cuda_graph = bool(use_cuda_graph) and self.engine is not None
         self.ep_ret = torch.zeros(env.num_envs, device=dev)
         self.ep_len = torch.zeros(env.num_envs, device=dev)
         self.fin = torch.zeros(3, dtype=torch.float64, device=dev)        # finished episodes: sum of returns, sum of lengths, count

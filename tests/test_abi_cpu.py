@@ -119,6 +119,21 @@ def test_live_task_cfg_round_trip():
         UsvLiveConfig.from_task_cfg(tb)
 
 
+def test_live_step_rejects_an_unknown_reward_mode():
+    """usv_step_live_f32 checks the step parameters like the classic step does; argument errors return before any CUDA call."""
+    from omniisaacgymenvs_loop_b200.config import UsvLiveConfig, live_default_config
+    L, E = _lib.lib(), _lib.ENUMS
+    b, lb = _lib.UsvEnvBuffers(), _lib.UsvLiveBuffers()
+    b.state = b.consts = b.reset_buf = b.lut_left = b.lut_right = 256          # never dereferenced
+    lb.bstate = lb.bconsts = lb.field = lb.reset_epoch = 256
+    p, lp = live_default_config(num_envs=32).to_params(), UsvLiveConfig().to_params()
+    step = lambda: L.usv_step_live_f32(ctypes.byref(b), ctypes.byref(lb), None, None, None, ctypes.c_int64(0), ctypes.byref(p),
+                                       ctypes.byref(lp), None)
+    assert step() == E["USV_OK"]                                                   # valid arguments, no envs: nothing to do
+    p.reward_mode = E["USV_REWARD_EXPONENTIAL"] + 1
+    assert step() == E["USV_E_PARAM"]
+
+
 @needs_reference
 def test_reference_live_yaml_parses_to_the_shipped_defaults():
     from omniisaacgymenvs_loop_b200.config import UsvLiveConfig, live_default_config, live_env_config
