@@ -674,6 +674,24 @@ int ppo_loopz_adam_step_f32(float* params, float* grads, float* exp_avg, float* 
 /* SquashedGaussianDiagonalCovariance.enforce_minimum_std   [ref: module.py:649-659] */
 int ppo_loopz_enforce_min_std_f32(float* std, const float* min_std, int32_t dim, void* stream);
 
+/* The loopz learner on `world` ranks (one process per GPU): each rank holds n envs of a W x n batch, and two exchanges over the         */
+/* PpoPeerComm windows make a W-rank update equal to the one-rank update over all W x n envs (up to summation order), with bit-identical */
+/* results on every rank.  Every entry travels as an 8-byte {fp32 value, sequence} packet stored into each peer's window and the values  */
+/* are added in rank order.  comm: windows from ppo_peer_window_alloc/open with cap >= world * ppo_loopz_peer_entries(net) * 2 floats,  */
+/* shared by both exchanges; seq_dev: device uint32[2], zero at start, shared by both exchanges and the same on every rank; err_flag:     */
+/* device word OR-ed with 1 when a peer does not arrive within 10 s -- sticky: later exchanges stop waiting, the gradient exchange then   */
+/* makes Adam skip its step, and the advantages come out zero.  Every rank must issue the same sequence of exchanges.                   */
+int64_t ppo_loopz_peer_entries(const PpoLoopzNet* net);   /* packets per rank and parity; < 0: unsupported shape */
+/* ppo_loopz_returns_f32 with the advantage moments (fp64 sum a, sum a^2) summed over the ranks: advantages are standardised over the */
+/* whole W x T x n batch.                                                                                                             */
+int ppo_loopz_returns_peer_f32(const float* rewards, const float* values, const uint8_t* dones, const float* last_values, float gamma,
+                               float lam, float* returns, float* advantages, void* scratch /*ppo_loopz_returns_scratch_bytes()*/, int32_t T,
+                               int64_t n, const PpoPeerComm* comm, uint32_t* seq_dev, uint32_t* err_flag, void* stream);
+/* between ppo_loopz_minibatch_grad_f32 / _tc and ppo_loopz_adam_step_f32 (called with M = world x the local minibatch): grads[0, P) */
+/* becomes the mean of the ranks' gradients, the three statistic sums behind it their sum.                                          */
+int ppo_loopz_grad_exchange_f32(const PpoPeerComm* comm, const PpoLoopzNet* net, float* grads, uint32_t* seq_dev, uint32_t* err_flag,
+                                void* stream);
+
 /* ------------------------------------------------------------------------- */
 /* D  the USV SysID / DAgger student (SURVEY 8(f) row 4, second half): what OIGE/scripts/dagger_usv_sysid_loopz.py trains   */
 /*   StateHistoryEncoder: hist[M, tsteps*In] -> per-step Linear(In,32)+LeakyReLU -> RESHAPE (bs,32,T) (the reference's      */

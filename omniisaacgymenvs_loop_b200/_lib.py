@@ -130,6 +130,7 @@ def lib() -> ctypes.CDLL:
     L.usv_live_scene_workspace_bytes.restype = ctypes.c_int64
     L.ppo_peer_window_bytes.restype = ctypes.c_int64
     L.ppo_minibatch_step_peer_entries.restype = ctypes.c_int64
+    L.ppo_loopz_peer_entries.restype = ctypes.c_int64
     L.dagger_history_encoder_param_count.restype = ctypes.c_int64
     L.dagger_train_scratch_floats.restype = ctypes.c_int64
     L.usv_live_scene_workspace_bytes.argtypes = [ctypes.c_int64]

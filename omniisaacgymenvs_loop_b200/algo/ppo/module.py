@@ -328,6 +328,7 @@ class _Store:
         # (counter - _offset_host) + *counter_offset == counter at every launch (same scheme as FusedUsvEnv.step_offset)
         self.counter_offset = torch.zeros(1, dtype=torch.int64, device=device)
         self._offset_host = 0
+        self.row_offset = 0          # global id of the first env this process samples for (rank x num_envs on `world` ranks)
 
     def advance_counter_offset(self, calls: int) -> None:
         """Inside a CUDA-graph capture containing `calls` sampling launches: the next replay draws fresh Philox samples."""
@@ -362,7 +363,7 @@ def _act(store: _Store, actor_obs, critic_obs, eval_actions, actions, log_prob, 
         store.counter += 1
     rc = L.ppo_loopz_act_f32(_lib.ptr(store.flat), ctypes.byref(store.net), _lib.ptr(actor_obs), _lib.ptr(critic_obs),
                              ctypes.c_uint64(store.seed), ctypes.c_uint64(store.counter - store._offset_host), _lib.ptr(store.counter_offset),
-                             ctypes.c_int64(0),
+                             ctypes.c_int64(store.row_offset),
                              _lib.ptr(eval_actions), _lib.ptr(actions), _lib.ptr(log_prob), _lib.ptr(means), _lib.ptr(values),
                              ctypes.c_int64(M), _lib.stream())
     _lib.check(rc, "ppo_loopz_act_f32")

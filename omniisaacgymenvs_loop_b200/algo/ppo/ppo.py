@@ -7,7 +7,15 @@ the whole `_train_step` is replayed from one CUDA graph.  Kept behaviours: advan
 minibatches are contiguous time-major row blocks (`in_order`) or chunks of one permutation per epoch (`shuffle`), an
 optimiser step is skipped when its loss is not finite, the mean losses are taken over the valid updates, the learning-rate
 schedule only moves when `update_scheduler()` is called (the live script never calls it).
-`flat_expert` (the imitation term of a different project's teacher) is not supported: the USV pipeline passes None."""
+`flat_expert` (the imitation term of a different project's teacher) is not supported: the USV pipeline passes None.
+
+Data-parallel over `world_size` ranks (one process per GPU, `num_envs` envs each, rank r owning global envs [r*num_envs, (r+1)*num_envs)):
+the parameters are broadcast from rank 0 at construction, sampling draws the Philox streams of the global env ids, the advantage moments
+and every minibatch gradient are summed over the ranks inside the update (rl.peer.PeerLoopzExchange, no host in the loop, capturable),
+and Adam sees the mean over all ranks' samples.  With `in_order` sampling the union of the ranks' minibatch k is the one-rank minibatch k
+over all envs, so a W-rank update equals the one-rank update over W x num_envs envs up to summation order, with bit-identical
+parameters on every rank.  With `shuffle` each rank permutes its own rows (the same generator seed on every rank): parameters stay
+identical across ranks, but the minibatches are not those of any one-rank run."""
 from __future__ import annotations
 
 import ctypes
@@ -28,7 +36,10 @@ class PPO:
     def __init__(self, actor: Actor, critic: Critic, num_envs, num_transitions_per_env, num_learning_epochs, num_mini_batches,
                  clip_param=0.2, gamma=0.998, lam=0.95, value_loss_coef=0.5, entropy_coef=0.0, learning_rate=5e-4, max_grad_norm=0.5,
                  use_clipped_value_loss=True, log_dir="run", device="cuda:0", mini_batch_sampling="shuffle", log_intervals=10,
-                 flat_expert=None, use_cuda_graph=True, tensor_cores=False):
+                 flat_expert=None, use_cuda_graph=True, tensor_cores=False, rank=0, world_size=1, group=None, peer=None):
+        """`rank`, `world_size`, `group`: data-parallel training (torch.distributed must be initialised when world_size > 1; it is used
+        at construction only).  `peer`: the exchange windows to use instead of building a rl.peer.PeerLoopzExchange over `group`
+        (one rank of rl.peer.InProcessLoopzExchange); no parameter broadcast then."""
         if flat_expert is not None:
             raise NotImplementedError("flat_expert (imitation term) is not part of the USV pipeline (rlgames_train_loopz.py:93)")
         if mini_batch_sampling not in ("shuffle", "in_order"):
@@ -48,6 +59,20 @@ class PPO:
         critic._bind(store)
         self._store = store
         self.P = store.P
+        self.rank, self.world = int(rank), int(world_size)
+        if not 0 <= self.rank < self.world:
+            raise ValueError(f"rank {rank} outside world_size {world_size}")
+        store.row_offset = self.rank * int(num_envs)
+        self.peer = None
+        if self.world > 1:
+            if peer is None:
+                import torch.distributed as dist
+                from ...rl.peer import PeerLoopzExchange
+                dist.broadcast(store.flat, 0, group=group)                    # every rank starts from rank 0's parameters
+                peer = PeerLoopzExchange(net, self.device, self.rank, self.world, group)
+            if peer.world != self.world or peer.rank != self.rank:
+                raise ValueError(f"exchange windows of rank {peer.rank} / {peer.world} for rank {self.rank} / {self.world}")
+            self.peer = peer
         f32 = dict(dtype=torch.float32, device=self.device)
         self.params = store.flat
         self.exp_avg, self.exp_avg_sq = torch.zeros(self.P, **f32), torch.zeros(self.P, **f32)
@@ -142,7 +167,7 @@ class PPO:
     # ---- learning -----------------------------------------------------------------------------------------------
     def update(self, actor_obs, value_obs, log_this_iteration, update):
         last_values = self.critic.predict(value_obs)
-        self.storage.compute_returns(last_values, self.gamma, self.lam)
+        self.storage.compute_returns(last_values, self.gamma, self.lam, peer=self.peer)
         mean_value_loss, mean_surrogate_loss, infos = self._train_step()
         self.storage.clear()
         if log_this_iteration and len(self.ep_infos) > 0:
@@ -153,6 +178,20 @@ class PPO:
 
     def _minibatch(self, lo: int, hi: int, index=None):
         """One optimiser step on rows [lo, hi) of the flattened storage, or on the rows listed in `index`."""
+        M = self._local_grad(lo, hi, index)
+        if self.peer is not None:
+            rc = self.lib.ppo_loopz_grad_exchange_f32(ctypes.byref(self.peer.comm), ctypes.byref(self._store.net), _lib.ptr(self.grads),
+                                                      _lib.ptr(self.peer.seq), _lib.ptr(self.peer.err), _lib.stream())
+            _lib.check(rc, "ppo_loopz_grad_exchange_f32")
+        rc = self.lib.ppo_loopz_adam_step_f32(_lib.ptr(self.params), _lib.ptr(self.grads), _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq),
+                                              _lib.ptr(self.lr), _lib.ptr(self.adam_step), ctypes.c_int32(self._parity), _lib.ptr(self._accum),
+                                              ctypes.c_int64(self.P), ctypes.c_int64(M * self.world), ctypes.byref(self.loss_params),
+                                              ctypes.byref(self.adam_params), _lib.stream())
+        _lib.check(rc, "ppo_loopz_adam_step_f32")
+        self._parity ^= 1
+
+    def _local_grad(self, lo: int, hi: int, index=None) -> int:
+        """This rank's minibatch gradient and statistic sums into self.grads; returns the minibatch size."""
         st = self.storage
         ao, co, ac, va, ad, re, lp = st._flat()
         if index is None:
@@ -175,12 +214,7 @@ class PPO:
                                                        _lib.ptr(idx), ctypes.byref(self.loss_params), _lib.ptr(self.grads),
                                                        _lib.ptr(self.scratch), ctypes.c_int64(M), _lib.stream())
             _lib.check(rc, "ppo_loopz_minibatch_grad_f32")
-        rc = self.lib.ppo_loopz_adam_step_f32(_lib.ptr(self.params), _lib.ptr(self.grads), _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq),
-                                              _lib.ptr(self.lr), _lib.ptr(self.adam_step), ctypes.c_int32(self._parity), _lib.ptr(self._accum),
-                                              ctypes.c_int64(self.P), ctypes.c_int64(M), ctypes.byref(self.loss_params),
-                                              ctypes.byref(self.adam_params), _lib.stream())
-        _lib.check(rc, "ppo_loopz_adam_step_f32")
-        self._parity ^= 1
+        return M
 
     def _run_epochs(self):
         batch = self.num_envs * self.num_transitions_per_env
@@ -224,6 +258,12 @@ class PPO:
         self.last_stats = {"num_valid_updates": int(n_valid), "mean_value_loss": mean_value_loss,
                            "mean_surrogate_loss": mean_surrogate_loss}
         return mean_value_loss, mean_surrogate_loss, self.last_stats
+
+    def check_peers(self) -> None:
+        """Raises when an exchange with the peer ranks timed out on this rank (one host read; from the failing exchange on, Adam skips
+        every step, so ranks cannot silently diverge)."""
+        if self.peer is not None:
+            self.peer.check()
 
     def minibatch_statistics(self):
         """Statistics of the LAST minibatch step (means over the minibatch), one host read."""

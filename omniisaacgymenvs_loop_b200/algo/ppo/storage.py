@@ -58,12 +58,18 @@ class RolloutStorage:
     def clear(self):
         self.step = 0
 
-    def compute_returns(self, last_values, gamma, lam):
+    def compute_returns(self, last_values, gamma, lam, peer=None):
+        """`peer` (a rl.peer.PeerLoopzExchange of world > 1): this storage is one rank's shard, the advantages are standardised over
+        the batch of all ranks."""
         last_values = _dev(last_values, self.device).reshape(-1).contiguous()
-        rc = _lib.lib().ppo_loopz_returns_f32(
-            _lib.ptr(self.rewards), _lib.ptr(self.values), _lib.ptr(self.dones), _lib.ptr(last_values), ctypes.c_float(gamma),
-            ctypes.c_float(lam), _lib.ptr(self.returns), _lib.ptr(self.advantages), _lib.ptr(self._scratch),
-            ctypes.c_int32(self.num_transitions_per_env), ctypes.c_int64(self.num_envs), _lib.stream())
+        args = [_lib.ptr(self.rewards), _lib.ptr(self.values), _lib.ptr(self.dones), _lib.ptr(last_values), ctypes.c_float(gamma),
+                ctypes.c_float(lam), _lib.ptr(self.returns), _lib.ptr(self.advantages), _lib.ptr(self._scratch),
+                ctypes.c_int32(self.num_transitions_per_env), ctypes.c_int64(self.num_envs)]
+        if peer is not None:
+            rc = _lib.lib().ppo_loopz_returns_peer_f32(*args, ctypes.byref(peer.comm), _lib.ptr(peer.seq), _lib.ptr(peer.err), _lib.stream())
+            _lib.check(rc, "ppo_loopz_returns_peer_f32")
+            return
+        rc = _lib.lib().ppo_loopz_returns_f32(*args, _lib.stream())
         _lib.check(rc, "ppo_loopz_returns_f32")
 
     def _flat(self):

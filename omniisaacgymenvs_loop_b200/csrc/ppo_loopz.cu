@@ -824,7 +824,9 @@ __global__ void __launch_bounds__(256) returns_kernel(const float* __restrict__ 
     part[2 * blockIdx.x + 1] = b;
   }
 }
-__global__ void __launch_bounds__(256) adv_norm_kernel(float* __restrict__ adv, const double* __restrict__ part, int nparts, int64_t total) {
+// moments over `total` entries (all ranks' batches when the moments were exchanged), normalising the `count` local entries
+__global__ void __launch_bounds__(256) adv_norm_kernel(float* __restrict__ adv, const double* __restrict__ part, int nparts, int64_t total,
+                                                       int64_t count) {
   __shared__ double sh[2][8];
   __shared__ float s_mean, s_inv;
   double s1 = 0.0, s2 = 0.0;
@@ -845,8 +847,129 @@ __global__ void __launch_bounds__(256) adv_norm_kernel(float* __restrict__ adv, 
   }
   __syncthreads();
   const float mean = s_mean, den = s_inv;
-  for (int64_t q = (int64_t)blockIdx.x * 256 + threadIdx.x; q < total; q += (int64_t)gridDim.x * 256)
+  for (int64_t q = (int64_t)blockIdx.x * 256 + threadIdx.x; q < count; q += (int64_t)gridDim.x * 256)
     adv[q] = sanitize0((adv[q] - mean) / den);
+}
+
+// ---------------------------------------------------------------------------------------------
+// data-parallel training over `world` ranks (one process per GPU, CUDA-IPC windows of ppo_peer_window_alloc / _open).  Two exchanges
+// share one window set and one sequence counter, in the order every rank issues them: the advantage moments once per update, the
+// minibatch gradient once per minibatch.  Window of rank q: [2 parities][world][ecap] packets {fp32 payload, sequence} (usv::st_packet),
+// ecap = cap / (2 world).  A rank stores its packet for entry e straight into slot [seq & 1][its rank][e] of every peer's window and
+// polls its own window until every peer's packet of entry e carries this sequence number, then adds the values in rank order: every
+// rank gets the same bits.  Double buffering by parity: a peer can be at most one exchange ahead (it needs this rank's packets of
+// exchange s+1 to finish s+1), and its packets of s+1 land in the other parity.
+// seq_dev = device uint32[2] {sequence number of the last exchange, arrival counter}, zero at start and the same on every rank; the last
+// CTA to finish advances the sequence, i.e. after every CTA has read it.  A peer that does not arrive within usv::kPeerSpinNs sets the
+// sticky err_flag; from then on the exchanges stop waiting and the gradient exchange marks its statistics non-finite, so Adam skips the
+// step on un-reduced gradients (the host reads the flag: PPO.check_peers).
+constexpr int kXThreads = 256;
+
+__device__ inline bool wait_packet(const float* src, uint32_t seq, float& x, const uint32_t* err_flag) {
+  if (usv::ld_packet(src, seq, x)) return true;
+  const unsigned long long t0 = usv::global_ns();
+  uint32_t spins = 0;
+  while (!usv::ld_packet(src, seq, x))
+    if ((++spins & 255u) == 0 && (usv::global_ns() - t0 > usv::kPeerSpinNs || *reinterpret_cast<const volatile uint32_t*>(err_flag))) return false;
+  return true;
+}
+
+// grads[0, n) summed over ranks; the gradient entries [0, P) are means over each rank's minibatch, so their sum is scaled by 1/world
+// (the mean over all ranks' samples); the statistics behind them are sums and stay sums (Adam divides them by world x M).
+// CTA b handles entries b, b + grid, ... on every rank and only waits for CTA b of its peers, so each CTA needs its peers' CTAs to be
+// resident at some point, never its own rank's other CTAs.  The grid is at most one CTA per SM (one wave of a kernel without shared
+// memory), so all CTAs of a launch are resident together; there is no grid-wide barrier, hence no cooperative launch.
+__global__ void __launch_bounds__(kXThreads) grad_exchange_kernel(PpoPeerComm c, float* __restrict__ g, int n, int P, float inv_world,
+                                                                  uint32_t* __restrict__ seq_dev, uint32_t* __restrict__ err_flag) {
+  __shared__ uint32_t s_seq;
+  __shared__ int s_bad;
+  if (threadIdx.x == 0) { s_seq = seq_dev[0] + 1u; s_bad = *reinterpret_cast<volatile uint32_t*>(err_flag) != 0; }
+  __syncthreads();
+  const uint32_t seq = s_seq;
+  const int64_t ecap = c.cap / (2 * c.world);
+  const int64_t par = (int64_t)(seq & 1u) * c.world;
+  if (!s_bad) {
+    for (int e = blockIdx.x * kXThreads + threadIdx.x; e < n; e += gridDim.x * kXThreads) {
+      const float v = g[e];
+      for (int p = 0; p < c.world; ++p)
+        if (p != c.rank) usv::st_packet(c.windows[p] + ((par + c.rank) * ecap + e) * 2, v, seq);
+    }
+    bool bad = false;
+    const float* mine = c.windows[c.rank];
+    for (int e = blockIdx.x * kXThreads + threadIdx.x; e < n && !bad; e += gridDim.x * kXThreads) {
+      const float own = g[e];
+      float acc = 0.f;
+      for (int p = 0; p < c.world && !bad; ++p) {
+        float x = own;
+        if (p != c.rank) bad = !wait_packet(mine + ((par + p) * ecap + e) * 2, seq, x, err_flag);
+        acc = p == 0 ? x : acc + x;
+      }
+      if (!bad) g[e] = e < P ? acc * inv_world : acc;
+    }
+    if (bad) { atomicOr(err_flag, 1u); s_bad = 1; }
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(seq_dev + 1, 1u) == gridDim.x - 1) {   // the last CTA: every CTA has read the sequence number and written its entries
+      seq_dev[1] = 0u;
+      seq_dev[0] = seq;
+      if (*reinterpret_cast<volatile uint32_t*>(err_flag)) g[P + PPO_LOOPZ_STAT_SURROGATE] = CUDART_NAN_F;   // Adam skips the step
+    }
+  }
+}
+
+// the advantage moments: this rank's fp64 (sum a, sum a^2) reduced from the per-block partials of returns_kernel, exchanged as four
+// packets (low and high words of each), added in rank order into part[0], part[1].  One CTA.
+__global__ void __launch_bounds__(256) moment_exchange_kernel(PpoPeerComm c, double* __restrict__ part, int nparts,
+                                                              uint32_t* __restrict__ seq_dev, uint32_t* __restrict__ err_flag) {
+  __shared__ double sh[2][8];
+  __shared__ double s_mom[16][2];
+  __shared__ int s_bad;
+  double s1 = 0.0, s2 = 0.0;
+  for (int k = threadIdx.x; k < nparts; k += 256) { s1 += part[2 * k]; s2 += part[2 * k + 1]; }
+  for (int o = 16; o > 0; o >>= 1) { s1 += __shfl_xor_sync(0xffffffffu, s1, o); s2 += __shfl_xor_sync(0xffffffffu, s2, o); }
+  if ((threadIdx.x & 31) == 0) { sh[0][threadIdx.x >> 5] = s1; sh[1][threadIdx.x >> 5] = s2; }
+  if (threadIdx.x == 0) s_bad = *reinterpret_cast<volatile uint32_t*>(err_flag) != 0;
+  __syncthreads();
+  const uint32_t seq = seq_dev[0] + 1u;
+  const int64_t ecap = c.cap / (2 * c.world);
+  const int64_t par = (int64_t)(seq & 1u) * c.world;
+  double a = 0.0, b = 0.0;
+  for (int w = 0; w < 8; ++w) { a += sh[0][w]; b += sh[1][w]; }
+  const int p = threadIdx.x;                  // thread p trades packets with rank p
+  if (p < c.world) {
+    const uint64_t ua = (uint64_t)__double_as_longlong(a), ub = (uint64_t)__double_as_longlong(b);
+    const float words[4] = {__uint_as_float((uint32_t)ua), __uint_as_float((uint32_t)(ua >> 32)), __uint_as_float((uint32_t)ub),
+                            __uint_as_float((uint32_t)(ub >> 32))};
+    float got[4] = {words[0], words[1], words[2], words[3]};
+    if (p != c.rank && !s_bad) {
+      for (int k = 0; k < 4; ++k) usv::st_packet(c.windows[p] + ((par + c.rank) * ecap + k) * 2, words[k], seq);
+      bool ok = true;
+      for (int k = 0; k < 4 && ok; ++k) ok = wait_packet(c.windows[c.rank] + ((par + p) * ecap + k) * 2, seq, got[k], err_flag);
+      if (!ok) { atomicOr(err_flag, 1u); s_bad = 1; }
+    }
+    s_mom[p][0] = __longlong_as_double((long long)(((uint64_t)__float_as_uint(got[1]) << 32) | __float_as_uint(got[0])));
+    s_mom[p][1] = __longlong_as_double((long long)(((uint64_t)__float_as_uint(got[3]) << 32) | __float_as_uint(got[2])));
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double ta = s_mom[0][0], tb = s_mom[0][1];
+    for (int q = 1; q < c.world; ++q) { ta += s_mom[q][0]; tb += s_mom[q][1]; }
+    part[0] = s_bad ? CUDART_NAN : ta;          // a failed exchange leaves no moments: the advantages come out zero
+    part[1] = s_bad ? CUDART_NAN : tb;
+    seq_dev[0] = seq;
+  }
+}
+
+static int check_comm(const PpoPeerComm* c, int64_t entries, const uint32_t* seq_dev, const uint32_t* err_flag) {
+  if (!c || !seq_dev || !err_flag) return USV_E_NULL;
+  if (c->world < 1 || c->world > 16 || c->rank < 0 || c->rank >= c->world) return USV_E_PARAM;
+  if (c->cap < (int64_t)c->world * entries * 2) return USV_E_SIZE;
+  for (int r = 0; r < c->world; ++r)
+    if (!c->windows[r]) return USV_E_NULL;
+    else if ((uintptr_t)c->windows[r] & 7) return USV_E_ALIGN;
+  return USV_OK;
 }
 
 static int check_net(const PpoLoopzNet* net) {
@@ -905,8 +1028,31 @@ int ppo_loopz_returns_f32(const float* rewards, const float* values, const uint8
   const int64_t total = (int64_t)T * n;
   int64_t nb = (total + 255) / 256;
   if (nb > kRetBlocks) nb = kRetBlocks;
-  adv_norm_kernel<<<(int)nb, 256, 0, (cudaStream_t)stream>>>(advantages, (const double*)scratch, (int)blocks, total);
+  adv_norm_kernel<<<(int)nb, 256, 0, (cudaStream_t)stream>>>(advantages, (const double*)scratch, (int)blocks, total, total);
   return usv::finish_launch(2);
+}
+
+int64_t ppo_loopz_peer_entries(const PpoLoopzNet* net) {
+  return check_net(net) == USV_OK ? (int64_t)(Spans(*net).P + PPO_LOOPZ_STAT_COUNT + 63) / 64 * 64 : -1;
+}
+
+int ppo_loopz_returns_peer_f32(const float* rewards, const float* values, const uint8_t* dones, const float* last_values, float gamma,
+                               float lam, float* returns, float* advantages, void* scratch, int32_t T, int64_t n,
+                               const PpoPeerComm* comm, uint32_t* seq_dev, uint32_t* err_flag, void* stream) {
+  if (T <= 0 || n <= 0) return USV_E_SIZE;     // every rank takes part in every exchange: no empty shard
+  if (!rewards || !values || !dones || !last_values || !returns || !advantages || !scratch) return USV_E_NULL;
+  const int rc = check_comm(comm, 4, seq_dev, err_flag);
+  if (rc != USV_OK) return rc;
+  int64_t blocks = (n + 255) / 256;
+  if (blocks > kRetBlocks) blocks = kRetBlocks;
+  cudaStream_t st = (cudaStream_t)stream;
+  returns_kernel<<<(int)blocks, 256, 0, st>>>(rewards, values, dones, last_values, gamma, lam, returns, advantages, (double*)scratch, T, n);
+  moment_exchange_kernel<<<1, 256, 0, st>>>(*comm, (double*)scratch, (int)blocks, seq_dev, err_flag);
+  const int64_t count = (int64_t)T * n;
+  int64_t nb = (count + 255) / 256;
+  if (nb > kRetBlocks) nb = kRetBlocks;
+  adv_norm_kernel<<<(int)nb, 256, 0, st>>>(advantages, (const double*)scratch, 1, count * comm->world, count);
+  return usv::finish_launch(3);
 }
 
 int ppo_loopz_minibatch_grad_f32(const float* params, const PpoLoopzNet* net, const float* actor_obs, const float* critic_obs,
@@ -930,6 +1076,20 @@ int ppo_loopz_minibatch_grad_f32(const float* params, const PpoLoopzNet* net, co
   const int n = Spans(*net).P + PPO_LOOPZ_STAT_COUNT;
   reduce_kernel<<<(n + 63) / 64, 256, 0, (cudaStream_t)stream>>>(scratch, gx, *net, *lp, grads);
   return usv::finish_launch(2);
+}
+
+int ppo_loopz_grad_exchange_f32(const PpoPeerComm* comm, const PpoLoopzNet* net, float* grads, uint32_t* seq_dev, uint32_t* err_flag,
+                                void* stream) {
+  int rc = check_net(net);
+  if (rc != USV_OK) return rc;
+  if (!grads) return USV_E_NULL;
+  const int P = Spans(*net).P, n = P + PPO_LOOPZ_STAT_LOG_PROB + 1;   // the gradient and the three statistic sums
+  rc = check_comm(comm, ppo_loopz_peer_entries(net), seq_dev, err_flag);
+  if (rc != USV_OK) return rc;
+  int grid = (n + kXThreads - 1) / kXThreads;
+  if (grid > usv::num_sms()) grid = usv::num_sms();
+  grad_exchange_kernel<<<grid, kXThreads, 0, (cudaStream_t)stream>>>(*comm, grads, n, P, 1.0f / (float)comm->world, seq_dev, err_flag);
+  return usv::finish_launch();
 }
 
 int ppo_loopz_adam_step_f32(float* params, float* grads, float* exp_avg, float* exp_avg_sq, const float* lr, int32_t* step, int32_t parity,

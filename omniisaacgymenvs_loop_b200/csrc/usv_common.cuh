@@ -92,4 +92,23 @@ __device__ __forceinline__ int lut_index(float cmd, int n_lut) {
   return idx;
 }
 
+// Peer exchange packets: one 8-byte {fp32 payload, sequence number} store is both the value and its flag, so a receiver that sees this
+// step's sequence number in a packet also sees its payload (the store is one 64-bit access).  Used by the fused rl_games minibatch
+// tail (ppo_mlp_tc_impl.inc) and the loopz exchanges (ppo_loopz_peer.cu).  A peer that does not show up within kPeerSpinNs is an error.
+constexpr unsigned long long kPeerSpinNs = 10ull * 1000 * 1000 * 1000;
+__device__ __forceinline__ void st_packet(float* p, float v, uint32_t seq) {
+  asm volatile("st.volatile.global.v2.b32 [%0], {%1, %2};" ::"l"(p), "r"(__float_as_uint(v)), "r"(seq) : "memory");
+}
+__device__ __forceinline__ bool ld_packet(const float* p, uint32_t seq, float& v) {
+  uint32_t a, b;
+  asm volatile("ld.volatile.global.v2.b32 {%0, %1}, [%2];" : "=r"(a), "=r"(b) : "l"(p) : "memory");
+  v = __uint_as_float(a);
+  return b == seq;
+}
+__device__ __forceinline__ unsigned long long global_ns() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+
 }  // namespace usv

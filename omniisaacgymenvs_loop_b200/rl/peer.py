@@ -84,6 +84,20 @@ class PeerStepExchange(PeerAllReduce):
         super().__init__(int(world_size) * entries * 2, device, rank, world_size, group)
 
 
+class PeerLoopzExchange(PeerAllReduce):
+    """The windows of the loopz learner's two exchanges (ppo_loopz_returns_peer_f32: advantage moments once per update,
+    ppo_loopz_grad_exchange_f32: the gradient once per minibatch): per rank [2 parities][world][entries] packets of 8 bytes
+    {value, sequence}, one sequence counter {sequence, arrival counter} shared by both."""
+
+    def __init__(self, net, device, rank: int = 0, world_size: int = 1, group=None):
+        entries = int(_lib.lib().ppo_loopz_peer_entries(ctypes.byref(net)))
+        if entries <= 0:
+            raise ValueError("unsupported loopz network shape")
+        self.entries = entries
+        super().__init__(int(world_size) * entries * 2, device, rank, world_size, group)
+        self.seq = torch.zeros(2, dtype=torch.int32, device=self.device)
+
+
 class InProcessStepExchange:
     """`world` ranks of the fused exchange living in ONE process on ONE device (each rank drives its own stream): the windows are plain
     device allocations instead of IPC mappings, the kernel and its packet protocol are the same.  Used to exercise the multi-rank
@@ -93,7 +107,9 @@ class InProcessStepExchange:
         pass
 
     def __init__(self, obs_dim: int, device, world_size: int):
-        entries = int(_lib.lib().ppo_minibatch_step_peer_entries(ctypes.c_int32(int(obs_dim))))
+        self._build(int(_lib.lib().ppo_minibatch_step_peer_entries(ctypes.c_int32(int(obs_dim)))), device, world_size, 1)
+
+    def _build(self, entries: int, device, world_size: int, seq_words: int):
         cap = int(world_size) * entries * 2
         self.windows = [torch.zeros(2 * cap + 64, dtype=torch.float32, device=device) for _ in range(world_size)]
         self.ranks = []
@@ -104,6 +120,14 @@ class InProcessStepExchange:
             k.comm.cap, k.comm.world, k.comm.rank = cap, int(world_size), r
             for q in range(world_size):
                 k.comm.windows[q] = self.windows[q].data_ptr()
-            k.seq = torch.zeros(1, dtype=torch.int32, device=device)
+            k.seq = torch.zeros(seq_words, dtype=torch.int32, device=device)
             k.err = torch.zeros(1, dtype=torch.int32, device=device)
+            k.check = PeerAllReduce.check.__get__(k)
             self.ranks.append(k)
+
+
+class InProcessLoopzExchange(InProcessStepExchange):
+    """In-process ranks of PeerLoopzExchange (tests/test_gpu_loopz_peer.py): `ranks[r]` goes to PPO(..., peer=...)."""
+
+    def __init__(self, net, device, world_size: int):
+        self._build(int(_lib.lib().ppo_loopz_peer_entries(ctypes.byref(net))), device, world_size, 2)

@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """The loopz training loop on the GPU learner [ref: OIGE/scripts/rlgames_train_loopz.py:700-1440]: MLPEncode actor / critic with a
 squashed Gaussian, horizon-length rollouts, reward scale 0.01, 4 epochs x 4 in-order minibatches, lr 5e-4, std floor 0.05 after
-every update.  python scripts/train_loopz.py --num-envs 4096 --updates 200 [--classic]"""
+every update.  python scripts/train_loopz.py --num-envs 4096 --updates 200 [--classic]
+Data-parallel on one node: torchrun --nproc-per-node 8 scripts/train_loopz.py --num-envs 4096 (4096 envs per GPU; NCCL only at
+start-up and for the log lines, the gradient exchange runs over NVLink peer memory inside the update graph; rank 0 prints and saves)."""
 import argparse
 import os
 import sys
@@ -11,30 +13,33 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import ctypes
 
 import torch
+import torch.distributed as dist
 
 from omniisaacgymenvs_loop_b200 import _lib
 from omniisaacgymenvs_loop_b200.algo.ppo import PPO, module as ppo_module
 from omniisaacgymenvs_loop_b200.config import live_default_config, live_task_cfg, load_task_yaml
 from omniisaacgymenvs_loop_b200.envs.usv_raisim_vecenv import USVRaisimVecEnv
 from omniisaacgymenvs_loop_b200.envs.vec_env_rlgames import VecEnvRLGames
+from omniisaacgymenvs_loop_b200.rl.a2c import reduce_episode_stats
 from omniisaacgymenvs_loop_b200.tasks.USV_Virtual import SimConfig, USVVirtual
 
 
-def make_env(task_cfg: dict, device: str, seed: int):
+def make_env(task_cfg: dict, device: str, seed: int, env_id_offset: int = 0):
     env = VecEnvRLGames(headless=True)
-    sim = SimConfig({"sim_device": device, "rl_device": device, "seed": seed, "env_id_offset": 0, "task": task_cfg})
+    sim = SimConfig({"sim_device": device, "rl_device": device, "seed": seed, "env_id_offset": env_id_offset, "task": task_cfg})
     env.set_task(USVVirtual("USVVirtual", sim, env, collect_stats=False), backend="torch")
     return USVRaisimVecEnv(env)
 
 
-def build_learner(env, device, horizon, seed, mass_dim=8, sampling="in_order", use_cuda_graph=True):
+def build_learner(env, device, horizon, seed, mass_dim=8, sampling="in_order", use_cuda_graph=True, rank=0, world_size=1):
     """rlgames_train_loopz.py:784-842"""
     arch = dict(speed_dim=3, mass_dim=mass_dim, mass_latent_dim=8, mass_encoder_shape=[64, 16])
     actor = ppo_module.Actor(ppo_module.MLPEncode_wrap([128, 128], "LeakyReLU", env.num_obs, env.num_acts, "Tanh", False, **arch),
                              ppo_module.SquashedGaussianDiagonalCovariance(env.num_acts, 0.3, action_scale=1.0), device, seed=seed)
     critic = ppo_module.Critic(ppo_module.MLPEncode_wrap([128, 128], "LeakyReLU", env.num_obs, 1, **arch), device)
     return PPO(actor=actor, critic=critic, num_envs=env.num_envs, num_transitions_per_env=horizon, num_learning_epochs=4, gamma=0.997,
-               lam=0.95, num_mini_batches=4, device=device, mini_batch_sampling=sampling, learning_rate=5e-4, use_cuda_graph=use_cuda_graph)
+               lam=0.95, num_mini_batches=4, device=device, mini_batch_sampling=sampling, learning_rate=5e-4, use_cuda_graph=use_cuda_graph,
+               rank=rank, world_size=world_size)
 
 
 class LoopzRunner:
@@ -110,10 +115,11 @@ class LoopzRunner:
         self.cycles += 1
 
     def pop_episode_stats(self):
-        """(mean return, count) of the episodes that finished since the last call (one host read)."""
-        s, _, c = self.fin.tolist()
+        """(mean return, count) of the episodes that finished since the last call on any rank (one host read; one all-reduce on
+        `world` ranks)."""
+        mean_ret, _, c = reduce_episode_stats(self.fin, self.ppo.world)
         self.fin.zero_()
-        return (s / c if c > 0 else float("nan")), int(c)
+        return mean_ret, c
 
 
 def train(env, ppo, updates, horizon=16, reward_scale=0.01, log_every=10, quiet=False, use_cuda_graph=True, runner=None):
@@ -127,8 +133,9 @@ def train(env, ppo, updates, horizon=16, reward_scale=0.01, log_every=10, quiet=
             torch.cuda.synchronize(ppo.device)
             if run.engine is not None:
                 run.engine.check_finite()
+            ppo.check_peers()
             dt = time.time() - t0
-            fps = horizon * env.num_envs * (update + 1 - n0) / max(dt, 1e-9)
+            fps = horizon * env.num_envs * ppo.world * (update + 1 - n0) / max(dt, 1e-9)
             t0, n0 = time.time(), update + 1
             mean_ret, n_ep = run.pop_episode_stats()
             hist.append((update, mean_ret, fps))
@@ -148,17 +155,24 @@ def main():
     ap.add_argument("--save", default=None)
     ap.add_argument("--checkpoint", default=None)
     args = ap.parse_args()
-    device = "cuda:0"
+    world, rank, local = int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0))
+    device = f"cuda:{local}"
+    torch.cuda.set_device(device)
+    if world > 1:
+        dist.init_process_group("nccl", device_id=torch.device(device))
     task_cfg = load_task_yaml(args.task_yaml, num_envs=args.num_envs) if args.task_yaml else live_task_cfg(live_default_config(num_envs=args.num_envs))
-    env = make_env(task_cfg, device, args.seed)
-    ppo = build_learner(env, device, args.horizon, args.seed)
+    env = make_env(task_cfg, device, args.seed, env_id_offset=rank * args.num_envs)
+    ppo = build_learner(env, device, args.horizon, args.seed, rank=rank, world_size=world)
     start = 0
     if args.checkpoint:
         start = ppo.load_state_dict(torch.load(args.checkpoint, map_location=device, weights_only=False))
-        print(f"[loopz] resumed from {args.checkpoint} (start_update={start})")
-    train(env, ppo, args.updates, args.horizon)
-    if args.save:
+        if rank == 0:
+            print(f"[loopz] resumed from {args.checkpoint} (start_update={start})")
+    train(env, ppo, args.updates, args.horizon, quiet=rank != 0)
+    if args.save and rank == 0:
         torch.save(ppo.state_dict(start + args.updates - 1), args.save)
+    if world > 1:
+        dist.destroy_process_group()
 
 
 if __name__ == "__main__":
