@@ -20,9 +20,10 @@ inline int finish_launch(int n_launches = 1) {
 
 inline int grid_for(int64_t n, int block) { return (int)((n + block - 1) / block); }
 
-// SM count of the current device, queried once per device; 148 (a B200) when the query fails.  Concurrent first calls on one
+// Attribute A of the current device, queried once per device; `fallback` when the query fails.  Concurrent first calls on one
 // device store the same value.
-inline int num_sms() {
+template <cudaDeviceAttr A>
+inline int device_attr(int fallback) {
   constexpr int kMaxDevices = 64;
   static std::atomic<int> cached[kMaxDevices];
   int dev = 0;
@@ -30,11 +31,15 @@ inline int num_sms() {
   const bool keyed = dev >= 0 && dev < kMaxDevices;
   int n = keyed ? cached[dev].load(std::memory_order_relaxed) : 0;
   if (n == 0) {
-    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
+    if (cudaDeviceGetAttribute(&n, A, dev) != cudaSuccess || n <= 0) n = fallback;
     if (keyed) cached[dev].store(n, std::memory_order_relaxed);
   }
   return n;
 }
+
+// SM count and L2 size in bytes of the current device (a B200's when the query fails)
+inline int num_sms() { return device_attr<cudaDevAttrMultiProcessorCount>(148); }
+inline int l2_bytes() { return device_attr<cudaDevAttrL2CacheSize>(126 << 20); }
 
 // Lets `kernel` launch with `bytes` of dynamic shared memory on the current device.  The largest size set per (kernel, device) is
 // remembered and the attribute is set again only when a request exceeds it: some kernels' sizes depend on their arguments.

@@ -19,6 +19,9 @@
 namespace usv {
 
 constexpr int kBlock = 128, kMinB = 7;   // threads per CTA, CTAs per SM (see above)
+// The fused step streams its one-pass data when the bytes the next step reads again fit in this share of L2 (see step_fused_kernel;
+// measured on a B200: gains at 0.5 of L2, losses at 1.0)
+constexpr double kResidentL2Share = 0.75;
 
 // Variant A (classic CaptureXY) task part of a control step: observation (13), reward + penalties, kills / done
 // `what` (USV_TASK_* bits) selects which of the reference's four calls advance their cross-step state: compute_reward owns the goal
@@ -158,6 +161,7 @@ __device__ __forceinline__ void accumulate_stats(float* __restrict__ st0, int64_
 
 // Each WARP stages its own 32 x 13 observation tile in smem (stride 13 is odd -> conflict-free) and writes it
 // out as one contiguous 1664 B run of float4 lines: only a __syncwarp, no CTA barrier on the store path.
+template <Cache C = Cache::kNormal>
 __device__ __forceinline__ void write_obs_tile(float* s_obs, const StepOut& o, bool active, float* __restrict__ obs,
                                                int64_t block_start, int64_t n) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -176,14 +180,20 @@ __device__ __forceinline__ void write_obs_tile(float* s_obs, const StepOut& o, b
     const float4* s4 = reinterpret_cast<const float4*>(sw);
     float4* g4 = reinterpret_cast<float4*>(g);
 #pragma unroll
-    for (int q = lane; q < (32 * kObs) / 4; q += 32) g4[q] = s4[q];
+    for (int q = lane; q < (32 * kObs) / 4; q += 32) st<C>(g4 + q, s4[q]);
   } else {
-    for (int q = lane; q < total; q += 32) g[q] = sw[q];
+    for (int q = lane; q < total; q += 32) st<C>(g + q, sw[q]);
   }
   __syncwarp();
 }
 
-template <int kDisturb, bool kStats>
+// One control step per launch.  Between launches the env state (52 B), reset_buf (8 B) and, with kStats, the episode sums (60 B) are
+// the only bytes the next launch reads again: they always take plain accesses.  kOnePass is the L2 policy of the rest -- per-episode
+// constants, actions, obs and reward, read or written once per step.  Evict-first (kStream) keeps those lines from pushing the
+// re-read set out of L2, which pays while that set fits; once it does not, evict-first is slower than plain accesses (B200, r03:
+// +6 % / +9 % env-steps/s at 2^19 / 2^20 envs, -2 % at 2^21; with stats +27 % at 2^19, -3 % at 2^20), so the launch picks kStream only
+// when the re-read set fits in a fraction of L2 (kResidentL2Share).  The thruster LUTs keep the read-only path (L1).
+template <int kDisturb, bool kStats, Cache kOnePass>
 __global__ void __launch_bounds__(kBlock, kMinB) step_fused_kernel(UsvEnvBuffers b, const float2* __restrict__ actions,
                                                             float* __restrict__ obs, float* __restrict__ rew,
                                                             int64_t n, const __grid_constant__ UsvStepParams p) {
@@ -203,18 +213,18 @@ __global__ void __launch_bounds__(kBlock, kMinB) step_fused_kernel(UsvEnvBuffers
   float2 act = make_float2(0.f, 0.f);
   if (active) {
     load_state(b.state, i, e);
-    load_consts<kDisturb>(b.consts, i, k);
+    load_consts<kDisturb, kOnePass>(b.consts, i, k);
     do_reset = b.reset_buf[i] != 0;
-    act = actions[i];
+    act = ld<kOnePass>(actions + i);
   }
   StepOut o;
   if (active) {
     control_step<kDisturb, true>(e, k, p, do_reset, act, (uint64_t)(p.env_id_offset + i), i, p.step_counter + (b.step_offset ? *b.step_offset : 0ull),
                                  p.first_call != 0, s_lutL, s_lutR, o);
     store_state(b.state, i, e);
-    if (do_reset) store_consts<kDisturb>(b.consts, i, k);
+    if (do_reset) store_consts<kDisturb, kOnePass>(b.consts, i, k);
     if (kStats) accumulate_stats(b.stats, i, do_reset, o, p);
-    rew[i] = o.rew;
+    st<kOnePass>(rew + i, o.rew);
     b.reset_buf[i] = (int64_t)o.done;
     if (b.nonfinite_flag) {
       if (!o.finite) atomicOr(b.nonfinite_flag, 1u);
@@ -223,7 +233,7 @@ __global__ void __launch_bounds__(kBlock, kMinB) step_fused_kernel(UsvEnvBuffers
       if (!isfinite(act.x) || !isfinite(act.y)) atomicOr(b.nonfinite_flag, 2u);
     }
   }
-  write_obs_tile(s_obs, o, active, obs, block_start, n);
+  write_obs_tile<kOnePass>(s_obs, o, active, obs, block_start, n);
 }
 
 // T control steps per launch, state in registers between steps.
@@ -400,10 +410,14 @@ int usv_step_fused_f32(const UsvEnvBuffers* b, const float* actions, float* obs,
   const int grid = grid_for(n, kBlock);
   const bool dis = wants_disturb(p), st = b->stats != nullptr;
   cudaStream_t s = (cudaStream_t)stream;
-#define USV_LAUNCH_STEP(D, S)                                                                              \
-  do {                                                                                                     \
-    ensure_dynamic_smem(step_fused_kernel<D, S>, smem);                                                    \
-    step_fused_kernel<D, S><<<grid, kBlock, smem, s>>>(*b, (const float2*)actions, obs, rew, n, *p);       \
+  // bytes per env the next step reads again (state, reset_buf, episode sums): see step_fused_kernel
+  const double reread = (double)n * (USV_S_COUNT * 4 + 8 + (st ? USV_ST_COUNT * 4 : 0));
+  const bool one_pass_cs = reread <= kResidentL2Share * l2_bytes();
+#define USV_LAUNCH_STEP(D, S)                                                                                                       \
+  do {                                                                                                                              \
+    auto* kern = one_pass_cs ? step_fused_kernel<D, S, Cache::kStream> : step_fused_kernel<D, S, Cache::kNormal>;                       \
+    ensure_dynamic_smem(kern, smem);                                                                                                \
+    kern<<<grid, kBlock, smem, s>>>(*b, (const float2*)actions, obs, rew, n, *p);                                                   \
   } while (0)
   const bool all4 = p->use_const_force && p->use_sin_force && p->use_const_torque && p->use_sin_torque && !p->use_water_current;
   if (dis && all4 && !st) USV_LAUNCH_STEP(2, false);

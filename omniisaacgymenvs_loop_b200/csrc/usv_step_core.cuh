@@ -39,6 +39,21 @@ struct StepOut {
 constexpr int kTile = 32;
 __device__ __forceinline__ int64_t tile_base(int64_t i, int count) { return (i >> 5) * (int64_t)(count * kTile) + (i & 31); }
 
+// L2 policy of a global access.  kStream (ld/st.global.cs: evict-first in L2) marks data that one launch of the per-step kernel
+// touches once and the next launch does not read again, so that the L2 victimises those lines before the ones that it does re-read
+// (env state, reset flags).  kNormal is a plain access and leaves the code of every other caller unchanged.
+enum class Cache { kNormal, kStream };
+template <Cache C, class T>
+__device__ __forceinline__ T ld(const T* p) {
+  if constexpr (C == Cache::kStream) return __ldcs(p);
+  else return *p;
+}
+template <Cache C, class T>
+__device__ __forceinline__ void st(T* p, T v) {
+  if constexpr (C == Cache::kStream) __stcs(p, v);
+  else *p = v;
+}
+
 __device__ __forceinline__ void load_state(const float* __restrict__ s0, int64_t i0, EnvState& e) {
   const float* __restrict__ s = s0 + tile_base(i0, USV_S_COUNT);
   e.x = s[USV_S_X * kTile];
@@ -73,67 +88,67 @@ __device__ __forceinline__ void store_state(float* __restrict__ s0, int64_t i0, 
   s[USV_S_PROGRESS * kTile] = __int_as_float(e.progress);
 }
 
-template <int kDisturb>
+template <int kDisturb, Cache C = Cache::kNormal>
 __device__ __forceinline__ void load_consts(const float* __restrict__ c0, int64_t i0, EnvConst& k) {
   const float* __restrict__ c = c0 + tile_base(i0, USV_C_COUNT);
-  k.tx = c[USV_C_TX * kTile];
-  k.ty = c[USV_C_TY * kTile];
-  k.mass = c[USV_C_MASS * kTile];
-  k.linu = c[USV_C_LIN_U * kTile];
-  k.linv = c[USV_C_LIN_V * kTile];
-  k.linr = c[USV_C_LIN_R * kTile];
-  k.quadu = c[USV_C_QUAD_U * kTile];
-  k.quadv = c[USV_C_QUAD_V * kTile];
-  k.quadr = c[USV_C_QUAD_R * kTile];
-  k.kdrag = c[USV_C_KDRAG * kTile];
-  k.mL = c[USV_C_THR_ML * kTile];
-  k.mR = c[USV_C_THR_MR * kTile];
-  k.kiz = c[USV_C_KIZ * kTile];
+  k.tx = ld<C>(c + USV_C_TX * kTile);
+  k.ty = ld<C>(c + USV_C_TY * kTile);
+  k.mass = ld<C>(c + USV_C_MASS * kTile);
+  k.linu = ld<C>(c + USV_C_LIN_U * kTile);
+  k.linv = ld<C>(c + USV_C_LIN_V * kTile);
+  k.linr = ld<C>(c + USV_C_LIN_R * kTile);
+  k.quadu = ld<C>(c + USV_C_QUAD_U * kTile);
+  k.quadv = ld<C>(c + USV_C_QUAD_V * kTile);
+  k.quadr = ld<C>(c + USV_C_QUAD_R * kTile);
+  k.kdrag = ld<C>(c + USV_C_KDRAG * kTile);
+  k.mL = ld<C>(c + USV_C_THR_ML * kTile);
+  k.mR = ld<C>(c + USV_C_THR_MR * kTile);
+  k.kiz = ld<C>(c + USV_C_KIZ * kTile);
   if (kDisturb) {
-    k.fcx = c[USV_C_FCX * kTile];
-    k.fcy = c[USV_C_FCY * kTile];
-    k.fxf = c[USV_C_FXF * kTile];
-    k.fyf = c[USV_C_FYF * kTile];
-    k.fxs = c[USV_C_FXS * kTile];
-    k.fys = c[USV_C_FYS * kTile];
-    k.famp = c[USV_C_FAMP * kTile];
-    k.tc = c[USV_C_TC * kTile];
-    k.tf = c[USV_C_TF * kTile];
-    k.ts = c[USV_C_TS * kTile];
-    k.tamp = c[USV_C_TAMP * kTile];
+    k.fcx = ld<C>(c + USV_C_FCX * kTile);
+    k.fcy = ld<C>(c + USV_C_FCY * kTile);
+    k.fxf = ld<C>(c + USV_C_FXF * kTile);
+    k.fyf = ld<C>(c + USV_C_FYF * kTile);
+    k.fxs = ld<C>(c + USV_C_FXS * kTile);
+    k.fys = ld<C>(c + USV_C_FYS * kTile);
+    k.famp = ld<C>(c + USV_C_FAMP * kTile);
+    k.tc = ld<C>(c + USV_C_TC * kTile);
+    k.tf = ld<C>(c + USV_C_TF * kTile);
+    k.ts = ld<C>(c + USV_C_TS * kTile);
+    k.tamp = ld<C>(c + USV_C_TAMP * kTile);
   } else {
     k.fcx = k.fcy = k.fxf = k.fyf = k.fxs = k.fys = k.famp = k.tc = k.tf = k.ts = k.tamp = 0.0f;
   }
 }
 
-template <int kDisturb>
+template <int kDisturb, Cache C = Cache::kNormal>
 __device__ __forceinline__ void store_consts(float* __restrict__ c0, int64_t i0, const EnvConst& k) {
   float* __restrict__ c = c0 + tile_base(i0, USV_C_COUNT);
-  c[USV_C_TX * kTile] = k.tx;
-  c[USV_C_TY * kTile] = k.ty;
-  c[USV_C_MASS * kTile] = k.mass;
-  c[USV_C_LIN_U * kTile] = k.linu;
-  c[USV_C_LIN_V * kTile] = k.linv;
-  c[USV_C_LIN_R * kTile] = k.linr;
-  c[USV_C_QUAD_U * kTile] = k.quadu;
-  c[USV_C_QUAD_V * kTile] = k.quadv;
-  c[USV_C_QUAD_R * kTile] = k.quadr;
-  c[USV_C_KDRAG * kTile] = k.kdrag;
-  c[USV_C_THR_ML * kTile] = k.mL;
-  c[USV_C_THR_MR * kTile] = k.mR;
-  c[USV_C_KIZ * kTile] = k.kiz;
+  st<C>(c + USV_C_TX * kTile, k.tx);
+  st<C>(c + USV_C_TY * kTile, k.ty);
+  st<C>(c + USV_C_MASS * kTile, k.mass);
+  st<C>(c + USV_C_LIN_U * kTile, k.linu);
+  st<C>(c + USV_C_LIN_V * kTile, k.linv);
+  st<C>(c + USV_C_LIN_R * kTile, k.linr);
+  st<C>(c + USV_C_QUAD_U * kTile, k.quadu);
+  st<C>(c + USV_C_QUAD_V * kTile, k.quadv);
+  st<C>(c + USV_C_QUAD_R * kTile, k.quadr);
+  st<C>(c + USV_C_KDRAG * kTile, k.kdrag);
+  st<C>(c + USV_C_THR_ML * kTile, k.mL);
+  st<C>(c + USV_C_THR_MR * kTile, k.mR);
+  st<C>(c + USV_C_KIZ * kTile, k.kiz);
   if (kDisturb) {
-    c[USV_C_FCX * kTile] = k.fcx;
-    c[USV_C_FCY * kTile] = k.fcy;
-    c[USV_C_FXF * kTile] = k.fxf;
-    c[USV_C_FYF * kTile] = k.fyf;
-    c[USV_C_FXS * kTile] = k.fxs;
-    c[USV_C_FYS * kTile] = k.fys;
-    c[USV_C_FAMP * kTile] = k.famp;
-    c[USV_C_TC * kTile] = k.tc;
-    c[USV_C_TF * kTile] = k.tf;
-    c[USV_C_TS * kTile] = k.ts;
-    c[USV_C_TAMP * kTile] = k.tamp;
+    st<C>(c + USV_C_FCX * kTile, k.fcx);
+    st<C>(c + USV_C_FCY * kTile, k.fcy);
+    st<C>(c + USV_C_FXF * kTile, k.fxf);
+    st<C>(c + USV_C_FYF * kTile, k.fyf);
+    st<C>(c + USV_C_FXS * kTile, k.fxs);
+    st<C>(c + USV_C_FYS * kTile, k.fys);
+    st<C>(c + USV_C_FAMP * kTile, k.famp);
+    st<C>(c + USV_C_TC * kTile, k.tc);
+    st<C>(c + USV_C_TF * kTile, k.tf);
+    st<C>(c + USV_C_TS * kTile, k.ts);
+    st<C>(c + USV_C_TAMP * kTile, k.tamp);
   }
 }
 
