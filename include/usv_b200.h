@@ -718,6 +718,21 @@ int dagger_mlp_forward_f32(const float* params, int32_t n_layers, const int32_t*
                            const int32_t* w_offsets /*host [n_layers]*/, const int32_t* b_offsets /*host [n_layers]*/,
                            int32_t last_activation, const float* x /*[M, x_ld]*/, int64_t x_ld, float* y /*[M, dims[n_layers]]*/,
                            int64_t M, void* stream);
+/* The deployed student's control step in one launch (USVSysIDStudentPolicy): append obs[:, :obs_nonpriv_dim] (rows obs_ld floats   */
+/* apart) to each env's history ring, run the id_encoder on the window in chronological order and the frozen action head on           */
+/* [frame | z^].  mu_out[M, head_dims[head_layers]] and latent_out[M, latent_dim] (or NULL) are bit-identical to                     */
+/* dagger_mlp_forward_f32(head, [frame | dagger_history_encoder_forward_f32(history)]) on the unrolled history.                       */
+/* ring: device [M, tsteps, obs_nonpriv_dim]; slot: device int32[2] = {slot of the oldest frame, 0}, zeroed with the ring: the launch */
+/* overwrites that slot and advances the index on the device (graph-capturable).  The window follows USVSysIDVecEnv: init = 1 is    */
+/* its reset() (fill_mode 0 "zeros": zeros then the frame last; 1 "repeat": the frame in every slot), init = 0 a step; dones (int64  */
+/* [M] or NULL, the flags of the step that produced obs) refill a finished env's window with the frame in "repeat" mode only.        */
+/* head_*: as dagger_mlp_forward_f32; head_dims[0] must be obs_nonpriv_dim + latent_dim.  Every argument is checked before any CUDA    */
+/* call.   [ref: OIGE/envs/usv_raisim_vecenv.py:387-617, OIGE/algo/ppo/dagger.py:50-66]                                               */
+int dagger_student_act_f32(const float* encoder_params, const float* head_params, int32_t head_layers, const int32_t* head_dims /*host*/,
+                           const int32_t* head_w_offsets /*host*/, const int32_t* head_b_offsets /*host*/, int32_t head_last_activation,
+                           float* ring, int32_t* slot, const float* obs /*[M, obs_ld]*/, int64_t obs_ld, int32_t obs_nonpriv_dim,
+                           int32_t tsteps, int32_t latent_dim, const int64_t* dones, int32_t fill_mode, int32_t init, float* mu_out,
+                           float* latent_out, int64_t M, void* stream);
 
 #ifdef __cplusplus
 }

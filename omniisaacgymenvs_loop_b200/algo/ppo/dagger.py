@@ -6,6 +6,8 @@
   action           a  = frozen_action_head([obs_nonpriv, z^])  (frozen; `MLPEncode.action_mlp`)
   update           4 epochs x 4 in-order minibatches of  MSE(z^, z*) -> Adam(5e-4), StepLR(200, 0.1) once per update
                    (dagger_sysid_minibatch_step_f32: forward + backward + Adam in two launches per minibatch, no host sync inside an update)
+  deployment       USVSysIDStudentPolicy: history ring + z^ + action head in one launch per control step (dagger_student_act_f32),
+                   loaded from the file scripts/dagger_usv_sysid_loopz.py --save writes (student_checkpoint)
 
 Same class / method surface as the reference; numpy in -> numpy out where the reference does that, CUDA tensors stay on the device."""
 from __future__ import annotations
@@ -16,8 +18,12 @@ import numpy as np
 import torch
 
 from ... import _lib
-from .module import StateHistoryEncoder
+from .module import E1, E2, H, FlatMLP, MLPEncode, StateHistoryEncoder
 from .storage import ObsStorage
+
+FILL_MODES = ("zeros", "repeat")
+# what a student checkpoint records beside the trainer's state and the teacher's PPO state (scripts/dagger_usv_sysid_loopz.py --save)
+STUDENT_META = {"history_len": int, "priv_dim": int, "obs_nonpriv_dim": int, "latent_dim": int, "fill_history_on_reset": str, "seed": int}
 
 
 class USVSysIDAgent:
@@ -144,3 +150,117 @@ class USVSysIDTrainer:
             self.adam_step.fill_(int(sd.get("step", 0)))
         self.itr = int(sd.get("itr", 0))
         self.lr.fill_(self.base_lr * (0.1 ** (self.itr // 200)))
+
+
+# ---- deployment: save the distilled student, play it closed-loop ------------------------------------------------------------------------
+def student_meta(meta: dict) -> dict:
+    """The checkpoint's `meta` entry, checked against STUDENT_META (every key present, each of its type, a known fill mode)."""
+    missing = [k for k in STUDENT_META if k not in meta]
+    if missing:
+        raise KeyError(f"student checkpoint meta lacks {missing}")
+    out = {k: t(meta[k]) for k, t in STUDENT_META.items()}
+    if out["fill_history_on_reset"] not in FILL_MODES:
+        raise ValueError(f"fill_history_on_reset must be one of {FILL_MODES}, got {out['fill_history_on_reset']!r}")
+    return out
+
+
+def student_checkpoint(trainer_state: dict, teacher_state: dict, **meta) -> dict:
+    """One self-contained file: USVSysIDTrainer.state_dict() keys unchanged (load_state_dict reads it), `teacher` = the loopz
+    PPO.state_dict() the student was distilled from (frozen action head, action_scale), `meta` = STUDENT_META."""
+    return {**trainer_state, "teacher": teacher_state, "meta": student_meta(meta)}
+
+
+class USVSysIDStudentPolicy:
+    """The distilled student as a deployable policy: each control step is ONE launch of dagger_student_act_f32, which appends the
+    current non-privileged frame to a per-env history ring on the device, runs the id_encoder on the window and the frozen action head on
+    [frame | z^].  mu is bit-identical to USVSysIDAgent.get_student_action on USVSysIDVecEnv's history (same window semantics, quirks
+    included), without the wrapper's roll / cat passes.  The ring and its slot index live on the device, so act() can be captured in a
+    CUDA graph.  CUDA tensors only."""
+
+    def __init__(self, *, id_encoder: StateHistoryEncoder, frozen_action_head: FlatMLP, history_len: int, obs_nonpriv_dim: int,
+                 fill_history_on_reset: str = "zeros") -> None:
+        self.id_encoder, self.head = id_encoder, frozen_action_head
+        self.history_len, self.obs_nonpriv_dim = int(history_len), int(obs_nonpriv_dim)
+        if id_encoder.tsteps != self.history_len or id_encoder.input_size != self.obs_nonpriv_dim:
+            raise ValueError("id_encoder was built for another history shape")
+        if fill_history_on_reset not in FILL_MODES:
+            raise ValueError(f"fill_history_on_reset must be one of {FILL_MODES}")
+        if frozen_action_head.dims[0] != self.obs_nonpriv_dim + id_encoder.output_size:
+            raise ValueError(f"action head input {frozen_action_head.dims[0]} != obs_nonpriv_dim + latent_dim "
+                             f"({self.obs_nonpriv_dim} + {id_encoder.output_size})")
+        self.fill_history_on_reset = fill_history_on_reset
+        self.device = id_encoder.device
+        self.ring = None                                                      # (N, T, D), allocated by reset()
+        self.slot = torch.zeros(2, dtype=torch.int32, device=self.device)     # {slot of the oldest frame, CTA arrivals}
+        self.action_scale = None                                              # set by from_checkpoint (the teacher's)
+        self.meta = None
+
+    def _launch(self, obs: torch.Tensor, dones, init: bool, latent_out) -> torch.Tensor:
+        if not torch.is_tensor(obs) or not obs.is_cuda:
+            raise _lib.UsvLibraryError("USVSysIDStudentPolicy needs CUDA tensors (there is no CPU fallback)")
+        if obs.dtype != torch.float32 or obs.dim() != 2 or obs.stride(1) != 1 or obs.shape[1] < self.obs_nonpriv_dim:
+            raise ValueError(f"obs must be fp32 [N, >= {self.obs_nonpriv_dim}] with unit column stride, got {obs.dtype} {tuple(obs.shape)}")
+        n, T, D, lat = obs.shape[0], self.history_len, self.obs_nonpriv_dim, self.id_encoder.output_size
+        if init:
+            if self.ring is None or self.ring.shape[0] != n:
+                self.ring = torch.zeros((n, T, D), dtype=torch.float32, device=self.device)
+                self.slot.zero_()
+        elif self.ring is None or self.ring.shape[0] != n:
+            raise RuntimeError("reset(obs) initialises the history before the first act(obs)")
+        if dones is not None:
+            dones = dones.reshape(-1)
+            if dones.numel() != n:
+                raise ValueError(f"dones has {dones.numel()} entries for {n} envs")
+            dones = dones if dones.dtype == torch.int64 and dones.is_contiguous() else dones.to(torch.int64).contiguous()
+        if latent_out is not None and (latent_out.shape != (n, lat) or latent_out.dtype != torch.float32):
+            raise ValueError(f"latent_out must be fp32 [{n}, {lat}]")
+        flat = self.head._flat()
+        mu = torch.empty((n, self.head.dims[-1]), dtype=torch.float32, device=self.device)
+        nl, I32 = len(self.head.layers), ctypes.c_int32
+        rc = _lib.lib().dagger_student_act_f32(
+            _lib.ptr(self.id_encoder.flat), _lib.ptr(flat), I32(nl), (I32 * (nl + 1))(*self.head.dims),
+            (I32 * nl)(*[l[0] for l in self.head.layers]), (I32 * nl)(*[l[1] for l in self.head.layers]), I32(self.head.last_activation),
+            _lib.ptr(self.ring), _lib.ptr(self.slot), ctypes.c_void_p(obs.data_ptr()), ctypes.c_int64(obs.stride(0)), I32(D), I32(T), I32(lat),
+            _lib.ptr(dones), I32(FILL_MODES.index(self.fill_history_on_reset)), I32(int(init)), _lib.ptr(mu), _lib.ptr(latent_out),
+            ctypes.c_int64(n), _lib.stream())
+        _lib.check(rc, "dagger_student_act_f32")
+        return mu
+
+    def reset(self, obs: torch.Tensor, latent_out=None) -> torch.Tensor:
+        """USVSysIDVecEnv.reset(): fills every env's window from obs[:, :D] ("zeros" or "repeat"); -> mu of that window."""
+        return self._launch(obs, None, True, latent_out)
+
+    def act(self, obs: torch.Tensor, dones=None, latent_out=None) -> torch.Tensor:
+        """One control step: appends obs[:, :D] to the history (dones: the flags of the step that produced obs, used by "repeat");
+        -> the head's raw output mu (N, 2).  latent_out (N, latent_dim), if given, receives z^."""
+        return self._launch(obs, dones, False, latent_out)
+
+    def history(self) -> torch.Tensor:
+        """(N, T, D) copy of the window, oldest frame first (USVSysIDVecEnv._history_torch).  Not for the hot path."""
+        if self.ring is None:
+            raise RuntimeError("no history before reset(obs)")
+        idx = (torch.arange(self.history_len, device=self.device) + self.slot[0].long()) % self.history_len
+        return self.ring.index_select(1, idx)
+
+    @classmethod
+    def from_checkpoint(cls, path, device) -> "USVSysIDStudentPolicy":
+        """A student file written by scripts/dagger_usv_sysid_loopz.py --save: id_encoder from the trainer state, the frozen action head
+        and action_scale from the embedded teacher."""
+        sd = torch.load(path, map_location=device, weights_only=False)
+        meta = student_meta(sd["meta"])
+        T, D, lat, priv = meta["history_len"], meta["obs_nonpriv_dim"], meta["latent_dim"], meta["priv_dim"]
+        enc = StateHistoryEncoder("LeakyReLU", D, T, lat, device)
+        enc.load_state_dict(sd["id_encoder_state_dict"])
+        teacher = sd["teacher"]
+        arch_sd = teacher["actor_architecture_state_dict"]
+        n_act = int(arch_sd["architecture.action_mlp.4.weight"].shape[0])
+        with torch.random.fork_rng(devices=[]):                           # MLPEncode's init draws; the loaded weights replace them
+            arch = MLPEncode([H, H], "LeakyReLU", D + priv, n_act, "Tanh", speed_dim=3, mass_dim=priv, mass_latent_dim=lat,
+                             mass_encoder_shape=[E1, E2])
+        arch.load_state_dict(arch_sd, "architecture.")
+        arch.flat = arch.flat.to(enc.device)
+        pol = cls(id_encoder=enc, frozen_action_head=arch.action_mlp, history_len=T, obs_nonpriv_dim=D,
+                  fill_history_on_reset=meta["fill_history_on_reset"])
+        pol.action_scale = torch.as_tensor(teacher["actor_distribution_state_dict"]["action_scale"], dtype=torch.float32).to(enc.device)
+        pol.meta = meta
+        return pol

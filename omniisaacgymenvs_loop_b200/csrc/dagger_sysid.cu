@@ -497,6 +497,163 @@ __global__ void __launch_bounds__(256) mlp_forward_kernel(const float* __restric
   }
 }
 
+// ---- deployment: the student's control step = history ring update + encoder + frozen action head, one launch ----------------------------
+// ring[M][T][D] holds each env's last T frames; slot[0] is the slot of the oldest frame, which the launch overwrites with the current frame,
+// so the frames in chronological order are slots p+1, ..., p+T-1, p (mod T) afterwards.  slot[1] counts the CTAs that have read slot[0];
+// the last one advances slot[0] and clears the count, so the index lives on the device and a captured graph can replay the launch.
+// Head weights live in shared memory as [out][in + 1] (lane = output unit: row stride in + 1 is conflict-free, and the copy from the
+// nn.Linear [out][in] layout is coalesced) followed by the bias.  Where they do not fit beside the encoder's weights and the 8 activation
+// blocks (T = 50: 81 + 113 + 84 KB), the CTA works in two phases: the encoder, then the head weights copied over the dead activation
+// blocks (from L2, coalesced), then the head.
+__host__ __device__ inline int head_smem_floats(const MlpDesc& d, int* off) {
+  int p = 0;
+  for (int l = 0; l < d.nl; ++l) { off[l] = p; p += d.dim[l + 1] * (d.dim[l] + 1) + d.dim[l + 1]; }
+  return (p + 3) & ~3;
+}
+
+__device__ void load_head(float* sh, const float* __restrict__ prm, const MlpDesc& d, const int* off) {
+  for (int l = 0; l < d.nl; ++l) {
+    const int I = d.dim[l], O = d.dim[l + 1];
+    for (int q = threadIdx.x; q < I * O; q += blockDim.x) { const int o = q / I, i = q - o * I; sh[off[l] + o * (I + 1) + i] = prm[d.w[l] + q]; }
+    for (int q = threadIdx.x; q < O; q += blockDim.x) sh[off[l] + O * (I + 1) + q] = prm[d.b[l] + q];
+  }
+}
+
+// the frozen head on buf[0, dim[0]) for one sample by one warp, in mlp_forward_kernel's fmaf order (bit-identical); returns the output row
+__device__ __forceinline__ const float* head_forward(const float* sh, const MlpDesc& d, const int* off, float* buf, int lane) {
+  float* in = buf;
+  float* out = buf + 128;
+  for (int l = 0; l < d.nl; ++l) {
+    const int I = d.dim[l], O = d.dim[l + 1];
+    const float* w = sh + off[l];
+    for (int o = lane; o < O; o += 32) {
+      float acc = w[O * (I + 1) + o];
+      const float* wr = w + o * (I + 1);
+      for (int i = 0; i < I; ++i) acc = fmaf(wr[i], in[i], acc);
+      const bool last = l == d.nl - 1;
+      out[o] = (last && d.tanh_out == 1) ? tanhf(acc) : ((last && d.tanh_out == 2) ? acc : lrelu(acc));
+    }
+    __syncwarp();
+    float* t = in; in = out; out = t;
+  }
+  return in;
+}
+
+template <int T>
+__host__ __device__ inline size_t act_block_floats(int In, int Out) { return (size_t)kWarps * SmemA<T>(In, Out).total; }
+
+// Shared memory: encoder weights | 8 activation blocks | head weights (resident only) | 8 head ping-pong buffers | per warp, the head
+// inputs [frame | z^] of G samples.  Split CTAs run the encoder over G chunks of their grid-stride sequence, then copy the head over the
+// activation blocks once and run it over the same G chunks: one head copy per G chunks (G = 16 covers 16 384 envs at T = 50 in one copy).
+template <int T>
+__global__ void __launch_bounds__(kThreads, 1) student_act_kernel(const float* __restrict__ enc, const float* __restrict__ head, MlpDesc hd,
+                                                                  float* __restrict__ ring, int* __restrict__ slot, const float* __restrict__ obs,
+                                                                  int64_t obs_ld, int D, int Lat, const int64_t* __restrict__ dones, int repeat,
+                                                                  int init, int resident, int G, float* __restrict__ mu, float* __restrict__ latent,
+                                                                  int64_t M) {
+  extern __shared__ __align__(16) float smem[];
+  __shared__ int s_p;
+  const SmemW<T> s(D, Lat);
+  const SmemA<T> m(D, Lat);
+  int hoff[3];
+  const int hfl = head_smem_floats(hd, hoff);
+  const int afl = (int)act_block_floats<T>(D, Lat);
+  const int XS = D + Lat;
+  float* act = smem + s.total;
+  float* hw = resident ? act + afl : act;                                   // resident: beside the activations; else over them
+  float* bufs = resident ? hw + hfl : act + (afl > hfl ? afl : hfl);
+  if (threadIdx.x == 0) s_p = slot[0];
+  load_weights<T>(smem, enc, D, Lat);
+  if (resident) load_head(hw, head, hd, hoff);
+  __syncthreads();
+  const int p = s_p;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float* a = act + warp * m.total;
+  float* buf = bufs + warp * 256;
+  float* xs = bufs + kWarps * 256 + warp * G * XS;
+  const int Oh = hd.dim[hd.nl];
+  const int64_t nchunks = (M + kWarps - 1) / kWarps;
+  const int64_t stride = (int64_t)gridDim.x * G;
+  for (int64_t c0 = blockIdx.x; c0 < nchunks; c0 += stride) {
+    // ---- phase 1, per warp: the ring update and the chronological staging in one pass, then the encoder; G chunks ----
+    for (int g = 0; g < G; ++g) {
+      const int64_t r = (c0 + (int64_t)g * gridDim.x) * kWarps + warp;
+      if (r >= M) break;
+      const bool fill = repeat && (init || (dones != nullptr && dones[r] != 0));
+      if (lane < D) {
+        const float f = obs[r * obs_ld + lane];
+        float* rr = ring + r * (int64_t)T * D + lane;
+        xs[g * XS + lane] = f;
+        int sl = p + 1 == T ? 0 : p + 1;                                    // window element t lives in slot (p + 1 + t) mod T
+#pragma unroll 10
+        for (int t = 0; t < T; ++t) {
+          const bool newest = t == T - 1;
+          // "zeros" leaves a finished env's old frames in place (the reference zeroes an advanced-indexing copy); init zeroes the window
+          const float v = (fill || newest) ? f : (init ? 0.f : rr[sl * D]);
+          a[m.hist + t * D + lane] = v;
+          if (fill || newest || init) rr[sl * D] = v;
+          sl = sl + 1 == T ? 0 : sl + 1;
+        }
+      }
+      __syncwarp();
+      float z[8];
+      sample_forward<T>(smem, a, D, Lat, lane, z);
+      if (lane < Lat) {
+        float v = 0.f;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) if (j == lane) v = z[j];
+        xs[g * XS + D + lane] = v;
+        if (latent) latent[r * Lat + lane] = v;
+      }
+      __syncwarp();
+    }
+    if (!resident) {                       // every warp is past its encoder before the head overwrites the activation blocks
+      __syncthreads();
+      load_head(hw, head, hd, hoff);
+      __syncthreads();
+    }
+    // ---- phase 2, per warp: the frozen head over the same G chunks ----
+    for (int g = 0; g < G; ++g) {
+      const int64_t r = (c0 + (int64_t)g * gridDim.x) * kWarps + warp;
+      if (r >= M) break;
+      for (int q = lane; q < XS; q += 32) buf[q] = xs[g * XS + q];
+      __syncwarp();
+      const float* y = head_forward(hw, hd, hoff, buf, lane);
+      for (int q = lane; q < Oh; q += 32) mu[r * Oh + q] = y[q];
+      __syncwarp();
+    }
+    if (!resident) __syncthreads();        // the next chunks' staging overwrites the head weights
+  }
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(slot + 1, 1) == (int)gridDim.x - 1) {
+      slot[0] = p + 1 == T ? 0 : p + 1;
+      slot[1] = 0;
+    }
+  }
+}
+
+template <int T>
+static int launch_student_act(const float* enc, const float* head, const MlpDesc& hd, float* ring, int* slot, const float* obs, int64_t obs_ld,
+                              int D, int Lat, const int64_t* dones, int repeat, int init, float* mu, float* latent, int64_t M, cudaStream_t st) {
+  constexpr size_t kMax = 227 * 1024 / sizeof(float);
+  int hoff[3];
+  const size_t hfl = (size_t)head_smem_floats(hd, hoff), afl = act_block_floats<T>(D, Lat), wfl = (size_t)SmemW<T>(D, Lat).total;
+  const size_t bufs = (size_t)kWarps * 256, xs = (size_t)kWarps * (D + Lat);                       // xs: per sample of G
+  const int resident = wfl + afl + hfl + bufs + xs <= kMax;
+  const size_t fixed = resident ? wfl + afl + hfl + bufs : wfl + (afl > hfl ? afl : hfl) + bufs;
+  if (fixed + xs > kMax) return USV_E_SIZE;
+  const int G = resident ? 1 : (int)((kMax - fixed) / xs < 16 ? (kMax - fixed) / xs : 16);
+  const size_t smem = (fixed + G * xs) * sizeof(float);
+  usv::ensure_dynamic_smem(student_act_kernel<T>, smem);
+  const int64_t want = (M + kWarps - 1) / kWarps;
+  const int sms = usv::num_sms();
+  const int grid = (int)(want < sms ? want : sms);
+  student_act_kernel<T><<<grid, kThreads, smem, st>>>(enc, head, hd, ring, slot, obs, obs_ld, D, Lat, dones, repeat, init, resident, G, mu, latent,
+                                                      M);
+  return usv::finish_launch();
+}
+
 template <int T>
 static int launch_forward(const float* prm, const float* hist, int64_t ld, int In, int Out, float* out, int64_t M, cudaStream_t st) {
   const size_t smem = fwd_smem_bytes<T>(In, Out);
@@ -604,6 +761,34 @@ int dagger_mlp_forward_f32(const float* params, int32_t n_layers, const int32_t*
   const int grid = (int)(want < sms ? want : sms);
   mlp_forward_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(params, d, x, x_ld, y, M);
   return usv::finish_launch();
+}
+
+int dagger_student_act_f32(const float* encoder_params, const float* head_params, int32_t head_layers, const int32_t* head_dims,
+                           const int32_t* head_w_offsets, const int32_t* head_b_offsets, int32_t head_last_activation, float* ring,
+                           int32_t* slot, const float* obs, int64_t obs_ld, int32_t obs_nonpriv_dim, int32_t tsteps, int32_t latent_dim,
+                           const int64_t* dones, int32_t fill_mode, int32_t init, float* mu_out, float* latent_out, int64_t M, void* stream) {
+  if (!encoder_params || !head_params || !head_dims || !head_w_offsets || !head_b_offsets || !ring || !slot || !obs || !mu_out) return USV_E_NULL;
+  if (tsteps != 50 && tsteps != 20 && tsteps != 10) return USV_E_UNSUPPORTED;
+  if (M < 0 || obs_nonpriv_dim < 1 || obs_nonpriv_dim > 32 || latent_dim < 1 || latent_dim > 8 || obs_ld < obs_nonpriv_dim) return USV_E_SIZE;
+  if (head_layers < 1 || head_layers > 3) return USV_E_SIZE;
+  for (int l = 0; l <= head_layers; ++l)
+    if (head_dims[l] < 1 || head_dims[l] > 128) return USV_E_SIZE;
+  if (head_dims[0] != obs_nonpriv_dim + latent_dim) return USV_E_SIZE;
+  if (head_last_activation < 0 || head_last_activation > 2 || (fill_mode != 0 && fill_mode != 1) || (init != 0 && init != 1)) return USV_E_PARAM;
+  MlpDesc d{};
+  d.nl = head_layers;
+  d.tanh_out = head_last_activation;
+  for (int l = 0; l <= head_layers; ++l) d.dim[l] = head_dims[l];
+  for (int l = 0; l < head_layers; ++l) { d.w[l] = head_w_offsets[l]; d.b[l] = head_b_offsets[l]; }
+  if (M == 0) return USV_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  DAGGER_DISPATCH(tsteps,
+                  launch_student_act<50>(encoder_params, head_params, d, ring, slot, obs, obs_ld, obs_nonpriv_dim, latent_dim, dones, fill_mode, init,
+                                         mu_out, latent_out, M, st),
+                  launch_student_act<20>(encoder_params, head_params, d, ring, slot, obs, obs_ld, obs_nonpriv_dim, latent_dim, dones, fill_mode, init,
+                                         mu_out, latent_out, M, st),
+                  launch_student_act<10>(encoder_params, head_params, d, ring, slot, obs, obs_ld, obs_nonpriv_dim, latent_dim, dones, fill_mode, init,
+                                         mu_out, latent_out, M, st));
 }
 
 }  // extern "C"

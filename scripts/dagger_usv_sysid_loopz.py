@@ -4,7 +4,10 @@ labels every step with z* = mass_encoder(privileged tail), the student (StateHis
 drives the boat through the frozen action head and is regressed onto z* every `horizon` steps.  Everything stays on the device: fused live
 env step, history window, student inference, teacher labels, MSE / backward / Adam kernels; one host read per update (the metrics).
 
-    python scripts/dagger_usv_sysid_loopz.py --envs 4096 --updates 50 [--checkpoint teacher.pt]
+    python scripts/dagger_usv_sysid_loopz.py --envs 4096 --updates 50 [--checkpoint teacher.pt] [--save student.pt]
+
+--save writes one file with the trainer's state, the teacher it was distilled from and the shapes (algo/ppo/dagger.student_checkpoint);
+scripts/play_loopz.py --student plays it.
 """
 import argparse
 import os
@@ -14,14 +17,15 @@ import time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 
-from omniisaacgymenvs_loop_b200.algo.ppo.dagger import USVSysIDAgent, USVSysIDTrainer
+from omniisaacgymenvs_loop_b200.algo.ppo.dagger import USVSysIDAgent, USVSysIDTrainer, student_checkpoint
 from omniisaacgymenvs_loop_b200.algo.ppo.module import StateHistoryEncoder
 from omniisaacgymenvs_loop_b200.config import UsvLiveConfig, live_default_config, live_task_cfg
 from omniisaacgymenvs_loop_b200.envs.usv_raisim_vecenv import USVSysIDVecEnv
 from scripts.train_loopz import build_learner, make_env
 
 
-def build(envs: int, device: str, seed: int, history_len: int = 50, priv_dim: int = 8, horizon: int = 16, checkpoint=None):
+def build_with_teacher(envs: int, device: str, seed: int, history_len: int = 50, priv_dim: int = 8, horizon: int = 16, checkpoint=None):
+    """-> (env, trainer, teacher PPO)"""
     base = make_env(live_task_cfg(live_default_config(num_envs=envs), UsvLiveConfig(priv_dim=priv_dim)), device, seed=seed)
     env = USVSysIDVecEnv(base._env, history_len=history_len, priv_dim=priv_dim, device=device)
     ppo = build_learner(base, device, horizon, seed=seed, mass_dim=priv_dim)         # the teacher policy (random unless a checkpoint is given)
@@ -33,7 +37,21 @@ def build(envs: int, device: str, seed: int, history_len: int = 50, priv_dim: in
                           history_len=history_len, obs_nonpriv_dim=env.obs_nonpriv_dim, device=device)
     trainer = USVSysIDTrainer(actor=agent, num_envs=env.num_envs, num_transitions_per_env=horizon, history_dim=history_len * env.obs_nonpriv_dim,
                               latent_dim=8, num_learning_epochs=4, num_mini_batches=4, device=device, learning_rate=5e-4)
+    return env, trainer, ppo
+
+
+def build(envs: int, device: str, seed: int, history_len: int = 50, priv_dim: int = 8, horizon: int = 16, checkpoint=None):
+    env, trainer, _ = build_with_teacher(envs, device, seed, history_len, priv_dim, horizon, checkpoint)
     return env, trainer
+
+
+def save_student(path: str, env, trainer, ppo, seed: int) -> None:
+    """The student file: trainer state + the teacher's PPO state + meta (USVSysIDStudentPolicy.from_checkpoint reads it)."""
+    ckpt = student_checkpoint(trainer.state_dict(), ppo.state_dict(), history_len=env.history_len, priv_dim=env.priv_dim,
+                              obs_nonpriv_dim=env.obs_nonpriv_dim, latent_dim=trainer.latent_dim,
+                              fill_history_on_reset=env._fill_history_on_reset, seed=seed)
+    os.makedirs(os.path.dirname(os.path.abspath(path)), exist_ok=True)
+    torch.save(ckpt, path)
 
 
 def run(env, trainer, updates: int, horizon: int = 16, log_every: int = 10, quiet: bool = False):
@@ -61,11 +79,12 @@ if __name__ == "__main__":
     ap.add_argument("--priv-dim", type=int, default=8)
     ap.add_argument("--seed", type=int, default=1234)
     ap.add_argument("--checkpoint", default=None)
+    ap.add_argument("--save", default=None, help="write the distilled student (with its teacher) to this file")
     ap.add_argument("--device", default="cuda:0")
     a = ap.parse_args()
     torch.cuda.set_device(a.device)
     torch.manual_seed(a.seed)
-    env, trainer = build(a.envs, a.device, a.seed, a.history_len, a.priv_dim, a.horizon, a.checkpoint)
+    env, trainer, ppo = build_with_teacher(a.envs, a.device, a.seed, a.history_len, a.priv_dim, a.horizon, a.checkpoint)
     run(env, trainer, 2, a.horizon, quiet=True)                      # warm-up
     torch.cuda.synchronize()
     t0 = time.perf_counter()
@@ -74,3 +93,6 @@ if __name__ == "__main__":
     dt = time.perf_counter() - t0
     print(f"[sysid] {a.envs} envs x horizon {a.horizon}: {a.updates} updates in {dt:.2f} s = {a.updates * a.horizon * a.envs / dt:.3e} frames/s "
           f"({dt / a.updates * 1e3:.1f} ms per collect + update); final r2_total {ms[-1]['r2_total']:.4f}")
+    if a.save:
+        save_student(a.save, env, trainer, ppo, a.seed)
+        print(f"[sysid] wrote the student to {a.save}")
