@@ -733,6 +733,33 @@ int dagger_student_act_f32(const float* encoder_params, const float* head_params
                            float* ring, int32_t* slot, const float* obs /*[M, obs_ld]*/, int64_t obs_ld, int32_t obs_nonpriv_dim,
                            int32_t tsteps, int32_t latent_dim, const int64_t* dones, int32_t fill_mode, int32_t init, float* mu_out,
                            float* latent_out, int64_t M, void* stream);
+/* Distillation from a frame store (USVSysIDDistiller).  Over a rollout of H steps the store keeps each frame once:                   */
+/*   store  device [M, tsteps - 1 + H, obs_nonpriv_dim]: index t + tsteps - 1 is the frame of rollout step t; indices 0 .. tsteps - 1 */
+/*          hold the whole window of step 0;                                                                                         */
+/*   refill device int32 [H, M]: the store index of the last "repeat" refill at or before step t, 0 when there was none;              */
+/*   row t * M + e (time-major, as ObsStorage flattens its samples) is the window of step t for env e, whose element k (oldest       */
+/*   first) is store[e][max(t + k, refill[t][e])].                                                                                    */
+/* dagger_sysid_collect_f32: dagger_student_act_f32 on rollout step t in [0, H) (init = 1 only at t = 0), plus the window into the   */
+/* store, refill[t], and the label zstar[t] (device [H, M, latent_dim]) = the teacher's mass encoder (teacher_*: as                  */
+/* dagger_mlp_forward_f32, teacher_dims[teacher_layers] = latent_dim) on obs[:, obs_nonpriv_dim : obs_nonpriv_dim + teacher_dims[0]], */
+/* bit-identical to dagger_mlp_forward_f32 on that slice.  One launch.  Every argument is checked before any CUDA call.               */
+int dagger_sysid_collect_f32(const float* encoder_params, const float* head_params, int32_t head_layers, const int32_t* head_dims /*host*/,
+                             const int32_t* head_w_offsets /*host*/, const int32_t* head_b_offsets /*host*/, int32_t head_last_activation,
+                             const float* teacher_params, int32_t teacher_layers, const int32_t* teacher_dims /*host*/,
+                             const int32_t* teacher_w_offsets /*host*/, const int32_t* teacher_b_offsets /*host*/,
+                             int32_t teacher_last_activation, float* ring, int32_t* slot, const float* obs /*[M, obs_ld]*/, int64_t obs_ld,
+                             int32_t obs_nonpriv_dim, int32_t tsteps, int32_t latent_dim, const int64_t* dones, int32_t fill_mode, int32_t init,
+                             float* store, int32_t* refill, float* zstar, int32_t t, int32_t horizon, float* mu_out, int64_t M, void* stream);
+/* dagger_history_encoder_forward_f32 / dagger_sysid_minibatch_step_f32 on the store's rows [row0, row0 + M) of horizon * num_envs  */
+/* (input_size = obs_nonpriv_dim); zstar is the whole label buffer [horizon * num_envs, Out].  Same bits as the row versions on the */
+/* unrolled windows.                                                                                                                  */
+int dagger_history_encoder_forward_store_f32(const float* params, const float* store, const int32_t* refill, int64_t num_envs, int32_t horizon,
+                                             int64_t row0, int32_t input_size, int32_t tsteps, int32_t output_size, float* latent /*[M, Out]*/,
+                                             int64_t M, void* stream);
+int dagger_sysid_minibatch_step_store_f32(float* params, const float* store, const int32_t* refill, int64_t num_envs, int32_t horizon, int64_t row0,
+                                          const float* zstar, int32_t input_size, int32_t tsteps, int32_t output_size, float* grads, float* scratch,
+                                          float* exp_avg, float* exp_avg_sq, const float* lr, int32_t* step, int32_t parity, float* mse_accum,
+                                          int64_t M, void* stream);
 
 #ifdef __cplusplus
 }

@@ -19,6 +19,7 @@
 #include <cuda_runtime.h>
 #include <math_constants.h>
 #include <stdint.h>
+#include <type_traits>
 #include "usv_common.cuh"
 
 namespace dagger {
@@ -205,10 +206,35 @@ __device__ __forceinline__ void stage_hist(float* dst, const float* __restrict__
   for (int q = lane; q < n; q += 32) dst[q] = src[q];
 }
 
-// ---- inference: out[M, Out] = StateHistoryEncoder(hist[M, ld]) ------------------------------------------------------------------------
-template <int T>
-__global__ void __launch_bounds__(kThreads, 1) encoder_forward_kernel(const float* __restrict__ prm, const float* __restrict__ hist, int64_t ld,
-                                                                      int In, int Out, float* __restrict__ out, int64_t M) {
+// How a kernel finds sample r's window (T * In floats, oldest frame first).  RowWindows: row r of a [M][ld] matrix.
+struct RowWindows {
+  const float* __restrict__ hist;
+  int64_t ld;
+  __device__ __forceinline__ void operator()(float* dst, int64_t r, int n, int lane) const { stage_hist(dst, hist + r * ld, n, lane); }
+};
+
+// StoreWindows: the frame store of a rollout.  store[N][S][In] (S = T - 1 + H) holds each frame once: index t + T - 1 is the frame of
+// rollout step t, indices 0 .. T - 1 the window of step 0.  refill[H][N] is the store index of the last "repeat" refill at or before
+// step t (0: none).  Global row g = t * N + e (the time-major order of ObsStorage) is window(t) of env e, whose element k is
+// store[e][max(t + k, refill[t][e])]: a contiguous span when nothing was refilled, else the refill frame repeated below it.
+struct StoreWindows {
+  const float* __restrict__ store;
+  const int* __restrict__ refill;
+  int64_t row0, N;
+  int S, In;
+  __device__ __forceinline__ void operator()(float* dst, int64_t r, int n, int lane) const {
+    const int64_t g = row0 + r, t = g / N, e = g - t * N;
+    const float* src = store + (e * S + t) * In;
+    const int lo = (refill[g] - (int)t) * In;                          // elements below lo repeat the frame that starts at lo
+    if (lo <= 0) stage_hist(dst, src, n, lane);                        // the common case keeps the row copy's pipelined loads
+    else
+      for (int q = lane; q < n; q += 32) dst[q] = src[q < lo ? lo + q % In : q];
+  }
+};
+
+// ---- inference: out[M, Out] = StateHistoryEncoder(window of row r) ----------------------------------------------------------------------
+template <int T, class Win>
+__device__ __forceinline__ void encoder_forward(const float* __restrict__ prm, Win win, int In, int Out, float* __restrict__ out, int64_t M) {
   extern __shared__ __align__(16) float smem[];
   const SmemW<T> s(In, Out);
   const SmemA<T> m(In, Out);
@@ -217,7 +243,7 @@ __global__ void __launch_bounds__(kThreads, 1) encoder_forward_kernel(const floa
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* a = smem + s.total + warp * m.total;
   for (int64_t r = (int64_t)blockIdx.x * kWarps + warp; r < M; r += (int64_t)gridDim.x * kWarps) {
-    stage_hist(a + m.hist, hist + r * ld, T * In, lane);
+    win(a + m.hist, r, T * In, lane);
     __syncwarp();
     float o[8];
     sample_forward<T>(smem, a, In, Out, lane, o);
@@ -231,11 +257,24 @@ __global__ void __launch_bounds__(kThreads, 1) encoder_forward_kernel(const floa
   }
 }
 
-// ---- training: MSE(encoder(hist), zstar) forward + backward; one partial gradient per CTA -------------------------------------------------
-// partial layout: [P gradient | sum of squared errors | unused x3], stride P + 4
 template <int T>
-__global__ void __launch_bounds__(kThreads, 1) train_kernel(const float* __restrict__ prm, const float* __restrict__ hist, int64_t ld,
-                                                            const float* __restrict__ zstar, int In, int Out, float* __restrict__ partial, int64_t M) {
+__global__ void __launch_bounds__(kThreads, 1) encoder_forward_kernel(const float* __restrict__ prm, const float* __restrict__ hist, int64_t ld,
+                                                                      int In, int Out, float* __restrict__ out, int64_t M) {
+  encoder_forward<T>(prm, RowWindows{hist, ld}, In, Out, out, M);
+}
+
+template <int T>
+__global__ void __launch_bounds__(kThreads, 1) encoder_forward_store_kernel(const float* __restrict__ prm, StoreWindows win, int In, int Out,
+                                                                            float* __restrict__ out, int64_t M) {
+  encoder_forward<T>(prm, win, In, Out, out, M);
+}
+
+// ---- training: MSE(encoder(hist), zstar) forward + backward; one partial gradient per CTA -------------------------------------------------
+// partial layout: [P gradient | sum of squared errors | unused x3], stride P + 4.  tid: threadIdx.x read in the kernel, whose
+// __launch_bounds__ bound it there (the range does not reach reads inside an inlined body, and the owner maps below use it).
+template <int T, class Win>
+__device__ __forceinline__ void train(const float* __restrict__ prm, Win win, const float* __restrict__ zstar, int In, int Out,
+                                      float* __restrict__ partial, int64_t M, unsigned tid) {
   using SP = Spec<T>;
   extern __shared__ __align__(16) float smem[];
   const SmemW<T> s(In, Out);
@@ -243,7 +282,7 @@ __global__ void __launch_bounds__(kThreads, 1) train_kernel(const float* __restr
   const Offsets o = offsets<T>(In, Out);
   load_weights<T>(smem, prm, In, Out);
   __syncthreads();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int warp = tid >> 5, lane = tid & 31;
   float* abase = smem + s.total;
   float* a = abase + warp * m.total;
   constexpr int K0 = SP::K(0), K1 = SP::K(1), K2 = SP::K(2);
@@ -267,7 +306,7 @@ __global__ void __launch_bounds__(kThreads, 1) train_kernel(const float* __restr
     const bool valid = r < M;
     // ---- per warp: forward, output gradient ----
     if (valid) {
-      stage_hist(a + m.hist, hist + r * ld, T * In, lane);
+      win(a + m.hist, r, T * In, lane);
       __syncwarp();
       float out[8];
       sample_forward<T>(smem, a, In, Out, lane, out);
@@ -427,6 +466,18 @@ __global__ void __launch_bounds__(kThreads, 1) train_kernel(const float* __restr
   }
 }
 
+template <int T>
+__global__ void __launch_bounds__(kThreads, 1) train_kernel(const float* __restrict__ prm, const float* __restrict__ hist, int64_t ld,
+                                                            const float* __restrict__ zstar, int In, int Out, float* __restrict__ partial, int64_t M) {
+  train<T>(prm, RowWindows{hist, ld}, zstar, In, Out, partial, M, threadIdx.x);
+}
+
+template <int T>
+__global__ void __launch_bounds__(kThreads, 1) train_store_kernel(const float* __restrict__ prm, StoreWindows win, const float* __restrict__ zstar,
+                                                                  int In, int Out, float* __restrict__ partial, int64_t M) {
+  train<T>(prm, win, zstar, In, Out, partial, M, threadIdx.x);
+}
+
 // second stage + Adam (torch.optim.Adam defaults, no clipping) in one launch: grads[P + 1] = [gradient | mse]
 __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ prm, const float* __restrict__ partial, int nparts, int P, float* __restrict__ grads,
                                                    float* __restrict__ m, float* __restrict__ v, const float* __restrict__ lr, int* __restrict__ step,
@@ -545,26 +596,49 @@ __host__ __device__ inline size_t act_block_floats(int In, int Out) { return (si
 // Shared memory: encoder weights | 8 activation blocks | head weights (resident only) | 8 head ping-pong buffers | per warp, the head
 // inputs [frame | z^] of G samples.  Split CTAs run the encoder over G chunks of their grid-stride sequence, then copy the head over the
 // activation blocks once and run it over the same G chunks: one head copy per G chunks (G = 16 covers 16 384 envs at T = 50 in one copy).
-template <int T>
-__global__ void __launch_bounds__(kThreads, 1) student_act_kernel(const float* __restrict__ enc, const float* __restrict__ head, MlpDesc hd,
-                                                                  float* __restrict__ ring, int* __restrict__ slot, const float* __restrict__ obs,
-                                                                  int64_t obs_ld, int D, int Lat, const int64_t* __restrict__ dones, int repeat,
-                                                                  int init, int resident, int G, float* __restrict__ mu, float* __restrict__ latent,
-                                                                  int64_t M) {
+//
+// The distillation's collect step (Collect = Distill) is the same step on rollout step t of H, plus: it writes window(t) into the frame
+// store (StoreWindows: all T frames at t = 0, the new frame after that) and the refill index, and labels the sample with the frozen
+// teacher's z* = mass_encoder(obs[:, D : D + priv]), in mlp_forward_kernel's fmaf order.  The teacher's weights sit behind the head's
+// ([out][in + 1] as well), resident or over the dead activation blocks.  Deployment (Collect = NoDistill) compiles none of it.
+struct NoDistill {
+  static constexpr bool kOn = false;
+};
+struct Distill {
+  static constexpr bool kOn = true;
+  const float* __restrict__ teacher;   // flat parameters of the teacher's mass encoder
+  MlpDesc td;                          // its layers: priv -> ... -> latent
+  float* __restrict__ store;           // [M][S][D], S = T - 1 + H
+  int* __restrict__ refill;            // [H][M]
+  float* __restrict__ zstar;           // [H][M][latent]
+  int t, S;
+};
+
+template <int T, class Collect>
+__device__ __forceinline__ void student_step(const float* __restrict__ enc, const float* __restrict__ head, MlpDesc hd, float* __restrict__ ring,
+                                             int* __restrict__ slot, const float* __restrict__ obs, int64_t obs_ld, int D, int Lat,
+                                             const int64_t* __restrict__ dones, int repeat, int init, int resident, int G, float* __restrict__ mu,
+                                             float* __restrict__ latent, int64_t M, Collect col) {
   extern __shared__ __align__(16) float smem[];
   __shared__ int s_p;
   const SmemW<T> s(D, Lat);
   const SmemA<T> m(D, Lat);
-  int hoff[3];
+  int hoff[3], toff[3];
   const int hfl = head_smem_floats(hd, hoff);
+  int tfl = 0;
+  if constexpr (Collect::kOn) tfl = head_smem_floats(col.td, toff);
   const int afl = (int)act_block_floats<T>(D, Lat);
   const int XS = D + Lat;
   float* act = smem + s.total;
   float* hw = resident ? act + afl : act;                                   // resident: beside the activations; else over them
-  float* bufs = resident ? hw + hfl : act + (afl > hfl ? afl : hfl);
+  float* tw = hw + hfl;                                                     // the teacher's weights (collect only)
+  float* bufs = resident ? hw + hfl + tfl : act + (afl > hfl + tfl ? afl : hfl + tfl);
   if (threadIdx.x == 0) s_p = slot[0];
   load_weights<T>(smem, enc, D, Lat);
-  if (resident) load_head(hw, head, hd, hoff);
+  if (resident) {
+    load_head(hw, head, hd, hoff);
+    if constexpr (Collect::kOn) load_head(tw, col.teacher, col.td, toff);
+  }
   __syncthreads();
   const int p = s_p;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -594,8 +668,16 @@ __global__ void __launch_bounds__(kThreads, 1) student_act_kernel(const float* _
           if (fill || newest || init) rr[sl * D] = v;
           sl = sl + 1 == T ? 0 : sl + 1;
         }
+        if constexpr (Collect::kOn)
+          if (col.t > 0) col.store[(r * col.S + col.t + T - 1) * D + lane] = f;
       }
       __syncwarp();
+      if constexpr (Collect::kOn) {
+        if (col.t == 0)
+          for (int q = lane; q < T * D; q += 32) col.store[r * col.S * D + q] = a[m.hist + q];
+        if (lane == 0)
+          col.refill[col.t * M + r] = fill ? col.t + T - 1 : (col.t == 0 ? 0 : col.refill[(col.t - 1) * M + r]);
+      }
       float z[8];
       sample_forward<T>(smem, a, D, Lat, lane, z);
       if (lane < Lat) {
@@ -610,12 +692,20 @@ __global__ void __launch_bounds__(kThreads, 1) student_act_kernel(const float* _
     if (!resident) {                       // every warp is past its encoder before the head overwrites the activation blocks
       __syncthreads();
       load_head(hw, head, hd, hoff);
+      if constexpr (Collect::kOn) load_head(tw, col.teacher, col.td, toff);
       __syncthreads();
     }
     // ---- phase 2, per warp: the frozen head over the same G chunks ----
     for (int g = 0; g < G; ++g) {
       const int64_t r = (c0 + (int64_t)g * gridDim.x) * kWarps + warp;
       if (r >= M) break;
+      if constexpr (Collect::kOn) {        // the label z* = teacher(priv tail)
+        for (int q = lane; q < col.td.dim[0]; q += 32) buf[q] = obs[r * obs_ld + D + q];
+        __syncwarp();
+        const float* y = head_forward(tw, col.td, toff, buf, lane);
+        for (int q = lane; q < Lat; q += 32) col.zstar[(col.t * M + r) * Lat + q] = y[q];
+        __syncwarp();
+      }
       for (int q = lane; q < XS; q += 32) buf[q] = xs[g * XS + q];
       __syncwarp();
       const float* y = head_forward(hw, hd, hoff, buf, lane);
@@ -634,49 +724,102 @@ __global__ void __launch_bounds__(kThreads, 1) student_act_kernel(const float* _
 }
 
 template <int T>
+__global__ void __launch_bounds__(kThreads, 1) student_act_kernel(const float* __restrict__ enc, const float* __restrict__ head, MlpDesc hd,
+                                                                  float* __restrict__ ring, int* __restrict__ slot, const float* __restrict__ obs,
+                                                                  int64_t obs_ld, int D, int Lat, const int64_t* __restrict__ dones, int repeat,
+                                                                  int init, int resident, int G, float* __restrict__ mu, float* __restrict__ latent,
+                                                                  int64_t M) {
+  student_step<T>(enc, head, hd, ring, slot, obs, obs_ld, D, Lat, dones, repeat, init, resident, G, mu, latent, M, NoDistill{});
+}
+
+template <int T>
+__global__ void __launch_bounds__(kThreads, 1) sysid_collect_kernel(const float* __restrict__ enc, const float* __restrict__ head, MlpDesc hd,
+                                                                    float* __restrict__ ring, int* __restrict__ slot, const float* __restrict__ obs,
+                                                                    int64_t obs_ld, int D, int Lat, const int64_t* __restrict__ dones, int repeat,
+                                                                    int init, int resident, int G, float* __restrict__ mu, int64_t M, Distill col) {
+  student_step<T>(enc, head, hd, ring, slot, obs, obs_ld, D, Lat, dones, repeat, init, resident, G, mu, nullptr, M, col);
+}
+
+// col: the collect step's extra outputs, or nullptr for the deployment step
+template <int T>
 static int launch_student_act(const float* enc, const float* head, const MlpDesc& hd, float* ring, int* slot, const float* obs, int64_t obs_ld,
-                              int D, int Lat, const int64_t* dones, int repeat, int init, float* mu, float* latent, int64_t M, cudaStream_t st) {
+                              int D, int Lat, const int64_t* dones, int repeat, int init, float* mu, float* latent, int64_t M, const Distill* col,
+                              cudaStream_t st) {
   constexpr size_t kMax = 227 * 1024 / sizeof(float);
   int hoff[3];
-  const size_t hfl = (size_t)head_smem_floats(hd, hoff), afl = act_block_floats<T>(D, Lat), wfl = (size_t)SmemW<T>(D, Lat).total;
+  const size_t hfl = (size_t)head_smem_floats(hd, hoff) + (col ? (size_t)head_smem_floats(col->td, hoff) : 0);   // + the teacher's
+  const size_t afl = act_block_floats<T>(D, Lat), wfl = (size_t)SmemW<T>(D, Lat).total;
   const size_t bufs = (size_t)kWarps * 256, xs = (size_t)kWarps * (D + Lat);                       // xs: per sample of G
   const int resident = wfl + afl + hfl + bufs + xs <= kMax;
   const size_t fixed = resident ? wfl + afl + hfl + bufs : wfl + (afl > hfl ? afl : hfl) + bufs;
   if (fixed + xs > kMax) return USV_E_SIZE;
   const int G = resident ? 1 : (int)((kMax - fixed) / xs < 16 ? (kMax - fixed) / xs : 16);
   const size_t smem = (fixed + G * xs) * sizeof(float);
-  usv::ensure_dynamic_smem(student_act_kernel<T>, smem);
   const int64_t want = (M + kWarps - 1) / kWarps;
   const int sms = usv::num_sms();
   const int grid = (int)(want < sms ? want : sms);
-  student_act_kernel<T><<<grid, kThreads, smem, st>>>(enc, head, hd, ring, slot, obs, obs_ld, D, Lat, dones, repeat, init, resident, G, mu, latent,
-                                                      M);
+  if (col) {
+    usv::ensure_dynamic_smem(sysid_collect_kernel<T>, smem);
+    sysid_collect_kernel<T><<<grid, kThreads, smem, st>>>(enc, head, hd, ring, slot, obs, obs_ld, D, Lat, dones, repeat, init, resident, G, mu, M,
+                                                          *col);
+  } else {
+    usv::ensure_dynamic_smem(student_act_kernel<T>, smem);
+    student_act_kernel<T><<<grid, kThreads, smem, st>>>(enc, head, hd, ring, slot, obs, obs_ld, D, Lat, dones, repeat, init, resident, G, mu,
+                                                        latent, M);
+  }
   return usv::finish_launch();
 }
 
-template <int T>
-static int launch_forward(const float* prm, const float* hist, int64_t ld, int In, int Out, float* out, int64_t M, cudaStream_t st) {
+template <int T, class Win>
+static int launch_forward(const float* prm, const Win& win, int In, int Out, float* out, int64_t M, cudaStream_t st) {
   const size_t smem = fwd_smem_bytes<T>(In, Out);
   if (smem > 227 * 1024) return USV_E_SIZE;
-  usv::ensure_dynamic_smem(encoder_forward_kernel<T>, smem);
   const int64_t want = (M + kWarps - 1) / kWarps;
   const int sms = usv::num_sms();
   const int grid = (int)(want < sms ? want : sms);
-  encoder_forward_kernel<T><<<grid, kThreads, smem, st>>>(prm, hist, ld, In, Out, out, M);
+  if constexpr (std::is_same<Win, RowWindows>::value) {
+    usv::ensure_dynamic_smem(encoder_forward_kernel<T>, smem);
+    encoder_forward_kernel<T><<<grid, kThreads, smem, st>>>(prm, win.hist, win.ld, In, Out, out, M);
+  } else {
+    usv::ensure_dynamic_smem(encoder_forward_store_kernel<T>, smem);
+    encoder_forward_store_kernel<T><<<grid, kThreads, smem, st>>>(prm, win, In, Out, out, M);
+  }
   return usv::finish_launch();
 }
 
-template <int T>
-static int launch_train(const float* prm, const float* hist, int64_t ld, const float* zstar, int In, int Out, float* partial, int64_t M, int* nparts,
+template <int T, class Win>
+static int launch_train(const float* prm, const Win& win, const float* zstar, int In, int Out, float* partial, int64_t M, int* nparts,
                         cudaStream_t st) {
   const size_t smem = fwd_smem_bytes<T>(In, Out);
   if (smem > 227 * 1024) return USV_E_SIZE;
-  usv::ensure_dynamic_smem(train_kernel<T>, smem);
   const int64_t want = (M + kWarps - 1) / kWarps;
   const int sms = usv::num_sms();
   const int grid = (int)(want < sms ? want : sms);
   *nparts = grid;
-  train_kernel<T><<<grid, kThreads, smem, st>>>(prm, hist, ld, zstar, In, Out, partial, M);
+  if constexpr (std::is_same<Win, RowWindows>::value) {
+    usv::ensure_dynamic_smem(train_kernel<T>, smem);
+    train_kernel<T><<<grid, kThreads, smem, st>>>(prm, win.hist, win.ld, zstar, In, Out, partial, M);
+  } else {
+    usv::ensure_dynamic_smem(train_store_kernel<T>, smem);
+    train_store_kernel<T><<<grid, kThreads, smem, st>>>(prm, win, zstar, In, Out, partial, M);
+  }
+  return usv::finish_launch();
+}
+
+// one minibatch: the training kernel over the windows `win` names, then Adam
+template <class Win>
+static int minibatch_step(float* params, const Win& win, const float* zstar, int32_t input_size, int32_t tsteps, int32_t output_size, float* grads,
+                          float* scratch, float* exp_avg, float* exp_avg_sq, const float* lr, int32_t* step, int32_t parity, float* mse_accum,
+                          int64_t M, cudaStream_t st) {
+  const int64_t P = dagger_history_encoder_param_count(input_size, tsteps, output_size);
+  if (P < 0) return USV_E_UNSUPPORTED;
+  int nparts = 0, rc;
+  if (tsteps == 50) rc = launch_train<50>(params, win, zstar, input_size, output_size, scratch, M, &nparts, st);
+  else if (tsteps == 20) rc = launch_train<20>(params, win, zstar, input_size, output_size, scratch, M, &nparts, st);
+  else rc = launch_train<10>(params, win, zstar, input_size, output_size, scratch, M, &nparts, st);
+  if (rc) return rc;
+  adam_kernel<<<(int)((P + 1 + 255) / 256), 256, 0, st>>>(params, scratch, nparts, (int)P, grads, exp_avg, exp_avg_sq, lr, step, parity,
+                                                         1.0f / ((float)M * (float)output_size), mse_accum);
   return usv::finish_launch();
 }
 
@@ -713,9 +856,10 @@ int dagger_history_encoder_forward_f32(const float* params, const float* hist, i
   if (M == 0) return USV_OK;
   if (!params || !hist || !latent) return USV_E_NULL;
   cudaStream_t st = (cudaStream_t)stream;
-  DAGGER_DISPATCH(tsteps, launch_forward<50>(params, hist, hist_ld, input_size, output_size, latent, M, st),
-                  launch_forward<20>(params, hist, hist_ld, input_size, output_size, latent, M, st),
-                  launch_forward<10>(params, hist, hist_ld, input_size, output_size, latent, M, st));
+  const RowWindows win{hist, hist_ld};
+  DAGGER_DISPATCH(tsteps, launch_forward<50>(params, win, input_size, output_size, latent, M, st),
+                  launch_forward<20>(params, win, input_size, output_size, latent, M, st),
+                  launch_forward<10>(params, win, input_size, output_size, latent, M, st));
 }
 
 int dagger_sysid_minibatch_step_f32(float* params, const float* hist, int64_t hist_ld, const float* zstar, int32_t input_size, int32_t tsteps,
@@ -724,17 +868,43 @@ int dagger_sysid_minibatch_step_f32(float* params, const float* hist, int64_t hi
   if (M <= 0 || input_size < 1 || input_size > 32 || output_size < 1 || output_size > 8 || hist_ld < (int64_t)input_size * tsteps) return USV_E_SIZE;
   if (!params || !hist || !zstar || !grads || !scratch || !exp_avg || !exp_avg_sq || !lr || !step) return USV_E_NULL;
   if (parity != 0 && parity != 1) return USV_E_PARAM;
-  const int64_t P = dagger_history_encoder_param_count(input_size, tsteps, output_size);
-  if (P < 0) return USV_E_UNSUPPORTED;
+  return minibatch_step(params, RowWindows{hist, hist_ld}, zstar, input_size, tsteps, output_size, grads, scratch, exp_avg, exp_avg_sq, lr, step,
+                        parity, mse_accum, M, (cudaStream_t)stream);
+}
+
+// the frame store's shape and the rows [row0, row0 + M) of its H * N windows
+static int check_store(int32_t input_size, int32_t output_size, int64_t num_envs, int32_t horizon, int64_t row0, int64_t M) {
+  if (M < 0 || input_size < 1 || input_size > 32 || output_size < 1 || output_size > 8 || num_envs < 1 || horizon < 1 || row0 < 0) return USV_E_SIZE;
+  if (num_envs > INT32_MAX || row0 + M > (int64_t)horizon * num_envs) return USV_E_SIZE;
+  return USV_OK;
+}
+
+int dagger_history_encoder_forward_store_f32(const float* params, const float* store, const int32_t* refill, int64_t num_envs, int32_t horizon,
+                                             int64_t row0, int32_t input_size, int32_t tsteps, int32_t output_size, float* latent, int64_t M,
+                                             void* stream) {
+  if (!params || !store || !refill || !latent) return USV_E_NULL;
+  if (tsteps != 50 && tsteps != 20 && tsteps != 10) return USV_E_UNSUPPORTED;
+  if (const int rc = check_store(input_size, output_size, num_envs, horizon, row0, M)) return rc;
+  if (M == 0) return USV_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  int nparts = 0, rc;
-  if (tsteps == 50) rc = launch_train<50>(params, hist, hist_ld, zstar, input_size, output_size, scratch, M, &nparts, st);
-  else if (tsteps == 20) rc = launch_train<20>(params, hist, hist_ld, zstar, input_size, output_size, scratch, M, &nparts, st);
-  else rc = launch_train<10>(params, hist, hist_ld, zstar, input_size, output_size, scratch, M, &nparts, st);
-  if (rc) return rc;
-  adam_kernel<<<(int)((P + 1 + 255) / 256), 256, 0, st>>>(params, scratch, nparts, (int)P, grads, exp_avg, exp_avg_sq, lr, step, parity,
-                                                         1.0f / ((float)M * (float)output_size), mse_accum);
-  return usv::finish_launch();
+  const StoreWindows win{store, refill, row0, num_envs, tsteps - 1 + horizon, input_size};
+  DAGGER_DISPATCH(tsteps, launch_forward<50>(params, win, input_size, output_size, latent, M, st),
+                  launch_forward<20>(params, win, input_size, output_size, latent, M, st),
+                  launch_forward<10>(params, win, input_size, output_size, latent, M, st));
+}
+
+int dagger_sysid_minibatch_step_store_f32(float* params, const float* store, const int32_t* refill, int64_t num_envs, int32_t horizon, int64_t row0,
+                                          const float* zstar, int32_t input_size, int32_t tsteps, int32_t output_size, float* grads, float* scratch,
+                                          float* exp_avg, float* exp_avg_sq, const float* lr, int32_t* step, int32_t parity, float* mse_accum,
+                                          int64_t M, void* stream) {
+  if (!params || !store || !refill || !zstar || !grads || !scratch || !exp_avg || !exp_avg_sq || !lr || !step) return USV_E_NULL;
+  if (tsteps != 50 && tsteps != 20 && tsteps != 10) return USV_E_UNSUPPORTED;
+  if (M <= 0) return USV_E_SIZE;
+  if (const int rc = check_store(input_size, output_size, num_envs, horizon, row0, M)) return rc;
+  if (parity != 0 && parity != 1) return USV_E_PARAM;
+  const StoreWindows win{store, refill, row0, num_envs, tsteps - 1 + horizon, input_size};
+  return minibatch_step(params, win, zstar + row0 * output_size, input_size, tsteps, output_size, grads, scratch, exp_avg, exp_avg_sq, lr, step,
+                        parity, mse_accum, M, (cudaStream_t)stream);
 }
 
 int dagger_mlp_forward_f32(const float* params, int32_t n_layers, const int32_t* dims, const int32_t* w_offsets, const int32_t* b_offsets,
@@ -763,10 +933,25 @@ int dagger_mlp_forward_f32(const float* params, int32_t n_layers, const int32_t*
   return usv::finish_launch();
 }
 
-int dagger_student_act_f32(const float* encoder_params, const float* head_params, int32_t head_layers, const int32_t* head_dims,
-                           const int32_t* head_w_offsets, const int32_t* head_b_offsets, int32_t head_last_activation, float* ring,
-                           int32_t* slot, const float* obs, int64_t obs_ld, int32_t obs_nonpriv_dim, int32_t tsteps, int32_t latent_dim,
-                           const int64_t* dones, int32_t fill_mode, int32_t init, float* mu_out, float* latent_out, int64_t M, void* stream) {
+// a small MLP's layers from host arrays: USV_E_SIZE for a bad shape, USV_E_PARAM for a bad last activation
+static int mlp_desc(int32_t n_layers, const int32_t* dims, const int32_t* w_offsets, const int32_t* b_offsets, int32_t last_activation, MlpDesc* d) {
+  if (n_layers < 1 || n_layers > 3) return USV_E_SIZE;
+  for (int l = 0; l <= n_layers; ++l)
+    if (dims[l] < 1 || dims[l] > 128) return USV_E_SIZE;
+  if (last_activation < 0 || last_activation > 2) return USV_E_PARAM;
+  *d = MlpDesc{};
+  d->nl = n_layers;
+  d->tanh_out = last_activation;
+  for (int l = 0; l <= n_layers; ++l) d->dim[l] = dims[l];
+  for (int l = 0; l < n_layers; ++l) { d->w[l] = w_offsets[l]; d->b[l] = b_offsets[l]; }
+  return USV_OK;
+}
+
+// dagger_student_act_f32 and, with col, dagger_sysid_collect_f32 past the collect step's own checks
+static int student_act(const float* encoder_params, const float* head_params, int32_t head_layers, const int32_t* head_dims,
+                       const int32_t* head_w_offsets, const int32_t* head_b_offsets, int32_t head_last_activation, float* ring, int32_t* slot,
+                       const float* obs, int64_t obs_ld, int32_t obs_nonpriv_dim, int32_t tsteps, int32_t latent_dim, const int64_t* dones,
+                       int32_t fill_mode, int32_t init, float* mu_out, float* latent_out, int64_t M, const Distill* col, void* stream) {
   if (!encoder_params || !head_params || !head_dims || !head_w_offsets || !head_b_offsets || !ring || !slot || !obs || !mu_out) return USV_E_NULL;
   if (tsteps != 50 && tsteps != 20 && tsteps != 10) return USV_E_UNSUPPORTED;
   if (M < 0 || obs_nonpriv_dim < 1 || obs_nonpriv_dim > 32 || latent_dim < 1 || latent_dim > 8 || obs_ld < obs_nonpriv_dim) return USV_E_SIZE;
@@ -784,11 +969,41 @@ int dagger_student_act_f32(const float* encoder_params, const float* head_params
   cudaStream_t st = (cudaStream_t)stream;
   DAGGER_DISPATCH(tsteps,
                   launch_student_act<50>(encoder_params, head_params, d, ring, slot, obs, obs_ld, obs_nonpriv_dim, latent_dim, dones, fill_mode, init,
-                                         mu_out, latent_out, M, st),
+                                         mu_out, latent_out, M, col, st),
                   launch_student_act<20>(encoder_params, head_params, d, ring, slot, obs, obs_ld, obs_nonpriv_dim, latent_dim, dones, fill_mode, init,
-                                         mu_out, latent_out, M, st),
+                                         mu_out, latent_out, M, col, st),
                   launch_student_act<10>(encoder_params, head_params, d, ring, slot, obs, obs_ld, obs_nonpriv_dim, latent_dim, dones, fill_mode, init,
-                                         mu_out, latent_out, M, st));
+                                         mu_out, latent_out, M, col, st));
+}
+
+int dagger_student_act_f32(const float* encoder_params, const float* head_params, int32_t head_layers, const int32_t* head_dims,
+                           const int32_t* head_w_offsets, const int32_t* head_b_offsets, int32_t head_last_activation, float* ring,
+                           int32_t* slot, const float* obs, int64_t obs_ld, int32_t obs_nonpriv_dim, int32_t tsteps, int32_t latent_dim,
+                           const int64_t* dones, int32_t fill_mode, int32_t init, float* mu_out, float* latent_out, int64_t M, void* stream) {
+  return student_act(encoder_params, head_params, head_layers, head_dims, head_w_offsets, head_b_offsets, head_last_activation, ring, slot, obs,
+                     obs_ld, obs_nonpriv_dim, tsteps, latent_dim, dones, fill_mode, init, mu_out, latent_out, M, nullptr, stream);
+}
+
+int dagger_sysid_collect_f32(const float* encoder_params, const float* head_params, int32_t head_layers, const int32_t* head_dims,
+                             const int32_t* head_w_offsets, const int32_t* head_b_offsets, int32_t head_last_activation, const float* teacher_params,
+                             int32_t teacher_layers, const int32_t* teacher_dims, const int32_t* teacher_w_offsets, const int32_t* teacher_b_offsets,
+                             int32_t teacher_last_activation, float* ring, int32_t* slot, const float* obs, int64_t obs_ld, int32_t obs_nonpriv_dim,
+                             int32_t tsteps, int32_t latent_dim, const int64_t* dones, int32_t fill_mode, int32_t init, float* store, int32_t* refill,
+                             float* zstar, int32_t t, int32_t horizon, float* mu_out, int64_t M, void* stream) {
+  if (!teacher_params || !teacher_dims || !teacher_w_offsets || !teacher_b_offsets || !store || !refill || !zstar) return USV_E_NULL;
+  Distill col{};
+  if (const int rc = mlp_desc(teacher_layers, teacher_dims, teacher_w_offsets, teacher_b_offsets, teacher_last_activation, &col.td)) return rc;
+  if (teacher_dims[teacher_layers] != latent_dim || obs_ld < (int64_t)obs_nonpriv_dim + teacher_dims[0]) return USV_E_SIZE;
+  if (horizon < 1 || t < 0 || t >= horizon) return USV_E_SIZE;
+  if (init && t != 0) return USV_E_PARAM;                 // the store keeps one window per rollout: it starts at step 0
+  col.teacher = teacher_params;
+  col.store = store;
+  col.refill = refill;
+  col.zstar = zstar;
+  col.t = t;
+  col.S = tsteps - 1 + horizon;
+  return student_act(encoder_params, head_params, head_layers, head_dims, head_w_offsets, head_b_offsets, head_last_activation, ring, slot, obs,
+                     obs_ld, obs_nonpriv_dim, tsteps, latent_dim, dones, fill_mode, init, mu_out, nullptr, M, &col, stream);
 }
 
 }  // extern "C"
