@@ -57,6 +57,24 @@ inline void ensure_dynamic_smem(void (*kernel)(Args...), size_t bytes) {
   ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), bytes);
 }
 
+// Programmatic dependent launch: a kernel launched with launch_pdl may start while its predecessor in the stream still runs.
+// pdl_wait() returns once that predecessor has completed and its writes are visible (a no-op for a plain launch); the kernel must not
+// touch global memory the predecessor may read or write before it.  pdl_trigger() lets the NEXT kernel of the stream start early.
+// After a copy or an event wait the attribute has no effect; under stream capture it becomes a programmatic graph edge.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+
 // rotation-matrix rows needed for R^T v with R = quaternion_to_matrix(q), q = (r,i,j,k) real-first,
 // two_s = 2/|q|^2  (public PyTorch3D formula; see oracle/ref_shim.py for the restatement we pin)
 struct Rot3 {

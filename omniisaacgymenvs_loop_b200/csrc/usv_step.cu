@@ -193,10 +193,18 @@ __device__ __forceinline__ void write_obs_tile(float* s_obs, const StepOut& o, b
 // re-read set out of L2, which pays while that set fits; once it does not, evict-first is slower than plain accesses (B200, r03:
 // +6 % / +9 % env-steps/s at 2^19 / 2^20 envs, -2 % at 2^21; with stats +27 % at 2^19, -3 % at 2^20), so the launch picks kStream only
 // when the re-read set fits in a fraction of L2 (kResidentL2Share).  The thruster LUTs keep the read-only path (L1).
+//
+// Programmatic dependent launch (launch_pdl): the launch may start while the previous kernel of the stream still runs, so NO
+// global-memory read or write may come before pdl_wait() -- that kernel may be the previous step (state, reset_buf), a policy
+// forward still reading obs, or a torch op still writing the actions or the state.  Only parameters and index arithmetic come first.
+// Each CTA lets the next step launch at entry: its CTAs can then only start once this launch's last wave is resident, so they never
+// take slots from this launch's own CTAs; they wait for its completion in place, which hides the launch and CTA ramp-up between steps.
 template <int kDisturb, bool kStats, Cache kOnePass>
 __global__ void __launch_bounds__(kBlock, kMinB) step_fused_kernel(UsvEnvBuffers b, const float2* __restrict__ actions,
                                                             float* __restrict__ obs, float* __restrict__ rew,
                                                             int64_t n, const __grid_constant__ UsvStepParams p) {
+  pdl_trigger();
+  pdl_wait();
   extern __shared__ __align__(16) float smem[];
   float* s_obs = smem;                       // [kBlock*13]
   // The two 4 KB thruster LUTs are gathered at 2 random indices per env-step.  Staging them per CTA cost 16 LDG+STS
@@ -417,7 +425,7 @@ int usv_step_fused_f32(const UsvEnvBuffers* b, const float* actions, float* obs,
   do {                                                                                                                              \
     auto* kern = one_pass_cs ? step_fused_kernel<D, S, Cache::kStream> : step_fused_kernel<D, S, Cache::kNormal>;                       \
     ensure_dynamic_smem(kern, smem);                                                                                                \
-    kern<<<grid, kBlock, smem, s>>>(*b, (const float2*)actions, obs, rew, n, *p);                                                   \
+    launch_pdl(kern, dim3(grid), dim3(kBlock), smem, s, *b, (const float2*)actions, obs, rew, n, *p);                               \
   } while (0)
   const bool all4 = p->use_const_force && p->use_sin_force && p->use_const_torque && p->use_sin_torque && !p->use_water_current;
   if (dis && all4 && !st) USV_LAUNCH_STEP(2, false);
