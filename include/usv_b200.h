@@ -267,6 +267,11 @@ typedef struct {
 int usv_step_fused_f32(const UsvEnvBuffers* b, const float* actions /*[n,2]*/,
                        float* obs /*[n,13]*/, float* rew /*[n]*/,
                        int64_t n, const UsvStepParams* p, void* stream);
+/* which kernel usv_step_fused_f32 launches for these parameters, with (stats != 0) or without episode statistics: one specialised
+ * on the full-DR configuration (UsvEnvConfig().full_dr(): discrete parameters fixed at compile time, same arithmetic) or the
+ * generic one.  <0: argument error. */
+enum { USV_STEP_PLAN_GENERIC = 0, USV_STEP_PLAN_FULL_DR = 1 };
+int usv_step_fused_plan(const UsvStepParams* p, int32_t stats);
 
 /* A7 stand-alone: the planar rigid body behind the simulator surface USVVirtual expects (HeronView.get_world_poses / get_velocities /
  * set_*, <body>.apply_forces_and_torques_at_pos, world.step())  [ref: OIGE/tasks/USV_Virtual.py:772-774,1119-1133,1567-1572].

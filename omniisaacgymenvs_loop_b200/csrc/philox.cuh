@@ -35,6 +35,32 @@ __host__ __device__ __forceinline__ Philox4 philox4x32_10(uint32_t c0, uint32_t 
   return Philox4{c0, c1, c2, c3};
 }
 
+// The 10 round keys (k0 + r*W0, k1 + r*W1) of one Philox key.  A kernel whose draws all use one seed takes them as a parameter and
+// reads them as constant-bank operands, instead of deriving them with 20 integer adds per draw.
+struct PhiloxKeys { uint32_t k0[10], k1[10]; };
+inline PhiloxKeys philox_round_keys(uint64_t seed) {
+  PhiloxKeys K;
+  uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+  for (int r = 0; r < 10; ++r) {
+    K.k0[r] = k0; K.k1[r] = k1;
+    k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+  }
+  return K;
+}
+__device__ __forceinline__ Philox4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, const PhiloxKeys& K) {
+  const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u;
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    uint32_t hi0, lo0, hi1, lo1;
+    philox_mulhilo(M0, c0, hi0, lo0);
+    philox_mulhilo(M1, c2, hi1, lo1);
+    uint32_t n0 = hi1 ^ c1 ^ K.k0[r];
+    uint32_t n2 = hi0 ^ c3 ^ K.k1[r];
+    c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
+  }
+  return Philox4{c0, c1, c2, c3};
+}
+
 // 24-bit uniform in [0,1), the same range contract as torch.rand (never returns 1.0)
 __host__ __device__ __forceinline__ float u01(uint32_t x) { return (float)(x >> 8) * (1.0f / 16777216.0f); }
 
@@ -51,10 +77,7 @@ __host__ __device__ __forceinline__ Uniform4 philox_uniform4(uint64_t seed, uint
 // 8 x 16-bit uniforms in [0,1) from ONE Philox call (per-step observation / action noise: amplitudes are
 // <= 0.05, so 2^-16 resolution is ~1e-6 of the signal; halves the RNG cost of the step)
 struct Uniform8 { float v[8]; };
-__host__ __device__ __forceinline__ Uniform8 philox_uniform8x16(uint64_t seed, uint64_t env_id, uint64_t step,
-                                                                uint32_t stream) {
-  Philox4 r = philox4x32_10((uint32_t)env_id, (uint32_t)step, (uint32_t)(step >> 32),
-                            stream ^ ((uint32_t)(env_id >> 32) << 8), (uint32_t)seed, (uint32_t)(seed >> 32));
+__host__ __device__ __forceinline__ Uniform8 uniform8x16(const Philox4& r) {
   const uint32_t w[4] = {r.x, r.y, r.z, r.w};
   Uniform8 u;
 #pragma unroll
@@ -63,6 +86,16 @@ __host__ __device__ __forceinline__ Uniform8 philox_uniform8x16(uint64_t seed, u
     u.v[2 * i + 1] = (float)(w[i] >> 16) * (1.0f / 65536.0f);
   }
   return u;
+}
+__host__ __device__ __forceinline__ Uniform8 philox_uniform8x16(uint64_t seed, uint64_t env_id, uint64_t step,
+                                                                uint32_t stream) {
+  return uniform8x16(philox4x32_10((uint32_t)env_id, (uint32_t)step, (uint32_t)(step >> 32),
+                                   stream ^ ((uint32_t)(env_id >> 32) << 8), (uint32_t)seed, (uint32_t)(seed >> 32)));
+}
+// the same draw from the round keys of `seed` (philox_round_keys)
+__device__ __forceinline__ Uniform8 philox_uniform8x16(const PhiloxKeys& K, uint64_t env_id, uint64_t step, uint32_t stream) {
+  return uniform8x16(philox4x32_10((uint32_t)env_id, (uint32_t)step, (uint32_t)(step >> 32),
+                                   stream ^ ((uint32_t)(env_id >> 32) << 8), K));
 }
 
 // Philox stream ids used by the fused env step (DESIGN.md "RNG streams")

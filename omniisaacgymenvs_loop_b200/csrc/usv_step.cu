@@ -14,6 +14,9 @@
 // issue-bound and ends in a partial wave: with 256 x 3 (24 warps per SM, 78 registers) 2^20 envs are 9.23 waves and the last 0.23 runs one
 // CTA per SM for a whole thread's latency; 28 warps per SM make it 7.9 waves.  Same-box A/B at 2^20 envs, 2000 steps (r02): 256 x 3 1.940e10
 // env-steps/s, 160 x 5 1.977, 224 x 4 2.014, 64 x 14 2.016, 128 x 7 2.02-2.05, 32 x 28 2.03; 64 registers (128 x 8, 96 x 10) 1.96-1.97.
+// The configuration training and the bench run (full DR, stats off) launches an instance specialised on it (PlanFullDr, usv_step_core.cuh):
+// discrete parameters fixed at compile time, five unrolled sub-steps, Philox round keys from the host; same arithmetic, 72 registers, no
+// spill.  B200 (1000 W), 2^20 envs: 46.7-46.9 -> 43.2-43.4 us per step; 2^19 -10 %, 2^21 -6 % (profiles/r05_step_plan.md).
 #include "usv_step_core.cuh"
 
 namespace usv {
@@ -26,6 +29,7 @@ constexpr double kResidentL2Share = 0.75;
 // Variant A (classic CaptureXY) task part of a control step: observation (13), reward + penalties, kills / done
 // `what` (USV_TASK_* bits) selects which of the reference's four calls advance their cross-step state: compute_reward owns the goal
 // counter and prev_position_dist, compute_penalty owns prev_state / prev_actions; the fused step passes the literal "all" (folded away)
+template <class Plan = PlanGeneric>
 __device__ __forceinline__ void post_classic(EnvState& e, const EnvConst& k, const UsvStepParams& p, bool do_reset,
                                              bool first_call, const DynOut& s, StepOut& o, const int what = USV_CXY_ALL) {
   const float pxn = s.pxn, pyn = s.pyn, vxn = s.vxn, vyn = s.vyn, wn = s.wn, yawn = s.yawn, hs = s.hs, hc = s.hc;
@@ -63,13 +67,13 @@ __device__ __forceinline__ void post_classic(EnvState& e, const EnvConst& k, con
   const float speed = sqrtf(vxn * vxn + vyn * vyn);
   const int goal = (d < p.position_tolerance) && (speed < p.goal_speed_gate);
   if (what & USV_CXY_REWARD) e.goal_cnt = e.goal_cnt * goal + goal;
-  float dist_rew;
-  if (p.reward_mode == USV_REWARD_LINEAR) {
-    dist_rew = p.position_scale * (e.prev_d - d);
-  } else if (p.reward_mode == USV_REWARD_SQUARE) {
-    dist_rew = p.position_scale * (e.prev_d * e.prev_d - d * d);
+  float dist_rew;   // products rounded on their own as in penalty_scalar
+  if (plan_or<Plan::reward_mode>(p.reward_mode) == USV_REWARD_LINEAR) {
+    dist_rew = __fmul_rn(p.position_scale, e.prev_d - d);
+  } else if (plan_or<Plan::reward_mode>(p.reward_mode) == USV_REWARD_SQUARE) {
+    dist_rew = __fmul_rn(p.position_scale, e.prev_d * e.prev_d - d * d);
   } else {
-    dist_rew = p.position_scale * (expf(-d / p.exponential_reward_coeff) - expf(-e.prev_d / p.exponential_reward_coeff));
+    dist_rew = __fmul_rn(p.position_scale, expf(-d / p.exponential_reward_coeff) - expf(-e.prev_d / p.exponential_reward_coeff));
   }
   const float h2 = herr * herr;
   const float align = p.align_la1 * (__expf(p.align_la2 * (h2 * h2)) + __expf(p.align_la3 * h2));
@@ -96,12 +100,16 @@ __device__ __forceinline__ void post_classic(EnvState& e, const EnvConst& k, con
   const float dw = first_call ? 0.0f : (wn - e.prev_w);
   const float dasum = first_call ? 0.0f : (asum - e.prev_asum);
   float pen_lin = 0.0f, pen_ang = 0.0f, pen_angvar = 0.0f, pen_energy = 0.0f, pen_actvar = 0.0f;
-  if (p.pen_linear_vel.form != USV_PEN_OFF) pen_lin = penalty_scalar(p.pen_linear_vel, speed);
-  if (p.pen_angular_vel.form != USV_PEN_OFF) pen_ang = penalty_scalar(p.pen_angular_vel, wn);
-  if (p.pen_angular_vel_variation.form != USV_PEN_OFF) pen_angvar = penalty_scalar(p.pen_angular_vel_variation, dw);
-  if (p.pen_energy.form == USV_PEN_NEG_SUM) pen_energy = -(pa0 + pa1) * p.pen_energy.c1 + p.pen_energy.c2;
-  else if (p.pen_energy.form == USV_PEN_EXP_NEG_SUMSQ) pen_energy = (__expf(-(pa0 * pa0 + pa1 * pa1)) - 1.0f) * p.pen_energy.c1;
-  if (p.pen_action_variation.form != USV_PEN_OFF) pen_actvar = penalty_scalar(p.pen_action_variation, dasum);
+  if (plan_or<Plan::pen_linear_vel>(p.pen_linear_vel.form) != USV_PEN_OFF)
+    pen_lin = penalty_scalar<Plan::pen_linear_vel>(p.pen_linear_vel, speed);
+  if (plan_or<Plan::pen_angular_vel>(p.pen_angular_vel.form) != USV_PEN_OFF)
+    pen_ang = penalty_scalar<Plan::pen_angular_vel>(p.pen_angular_vel, wn);
+  if (plan_or<Plan::pen_angular_vel_variation>(p.pen_angular_vel_variation.form) != USV_PEN_OFF)
+    pen_angvar = penalty_scalar<Plan::pen_angular_vel_variation>(p.pen_angular_vel_variation, dw);
+  if (plan_or<Plan::pen_energy>(p.pen_energy.form) == USV_PEN_NEG_SUM) pen_energy = -(pa0 + pa1) * p.pen_energy.c1 + p.pen_energy.c2;
+  else if (plan_or<Plan::pen_energy>(p.pen_energy.form) == USV_PEN_EXP_NEG_SUMSQ) pen_energy = __fmul_rn(__expf(-(pa0 * pa0 + pa1 * pa1)) - 1.0f, p.pen_energy.c1);
+  if (plan_or<Plan::pen_action_variation>(p.pen_action_variation.form) != USV_PEN_OFF)
+    pen_actvar = penalty_scalar<Plan::pen_action_variation>(p.pen_action_variation, dasum);
   const float penalties = pen_lin + pen_ang + pen_angvar + pen_energy + pen_actvar;
   if (what & USV_CXY_PENALTY) {
     e.prev_w = wn;
@@ -133,14 +141,14 @@ __device__ __forceinline__ void post_classic(EnvState& e, const EnvConst& k, con
 }
 
 // one full control step for one env, state in registers
-template <int kDisturb, bool kLutGlobal>
+template <int kDisturb, bool kLutGlobal, class Plan = PlanGeneric>
 __device__ __forceinline__ void control_step(EnvState& e, EnvConst& k, const UsvStepParams& p, bool do_reset,
                                              float2 act, uint64_t gid, int64_t lid, uint64_t step, bool first_call,
                                              const float* __restrict__ s_lutL, const float* __restrict__ s_lutR,
-                                             StepOut& o) {
+                                             StepOut& o, const PhiloxKeys* keys = nullptr) {
   DynOut s;
-  step_dynamics<kDisturb, kLutGlobal>(e, k, p, do_reset, act, gid, lid, step, s_lutL, s_lutR, s);
-  post_classic(e, k, p, do_reset, first_call, s, o);
+  step_dynamics<kDisturb, kLutGlobal, Plan>(e, k, p, do_reset, act, gid, lid, step, s_lutL, s_lutR, s, keys);
+  post_classic<Plan>(e, k, p, do_reset, first_call, s, o);
 }
 
 __device__ __forceinline__ void accumulate_stats(float* __restrict__ st0, int64_t i0, bool was_reset,
@@ -199,10 +207,14 @@ __device__ __forceinline__ void write_obs_tile(float* s_obs, const StepOut& o, b
 // forward still reading obs, or a torch op still writing the actions or the state.  Only parameters and index arithmetic come first.
 // Each CTA lets the next step launch at entry: its CTAs can then only start once this launch's last wave is resident, so they never
 // take slots from this launch's own CTAs; they wait for its completion in place, which hides the launch and CTA ramp-up between steps.
-template <int kDisturb, bool kStats, Cache kOnePass>
+//
+// Plan (usv_step_core.cuh) fixes the discrete parameters at compile time; `keys` are the Philox round keys of p.seed, read only by a
+// fixed plan.
+template <int kDisturb, bool kStats, Cache kOnePass, class Plan = PlanGeneric>
 __global__ void __launch_bounds__(kBlock, kMinB) step_fused_kernel(UsvEnvBuffers b, const float2* __restrict__ actions,
                                                             float* __restrict__ obs, float* __restrict__ rew,
-                                                            int64_t n, const __grid_constant__ UsvStepParams p) {
+                                                            int64_t n, const __grid_constant__ UsvStepParams p,
+                                                            const __grid_constant__ PhiloxKeys keys) {
   pdl_trigger();
   pdl_wait();
   extern __shared__ __align__(16) float smem[];
@@ -227,8 +239,9 @@ __global__ void __launch_bounds__(kBlock, kMinB) step_fused_kernel(UsvEnvBuffers
   }
   StepOut o;
   if (active) {
-    control_step<kDisturb, true>(e, k, p, do_reset, act, (uint64_t)(p.env_id_offset + i), i, p.step_counter + (b.step_offset ? *b.step_offset : 0ull),
-                                 p.first_call != 0, s_lutL, s_lutR, o);
+    control_step<kDisturb, true, Plan>(e, k, p, do_reset, act, (uint64_t)(p.env_id_offset + i), i,
+                                       p.step_counter + (b.step_offset ? *b.step_offset : 0ull), p.first_call != 0, s_lutL, s_lutR, o,
+                                       &keys);
     store_state(b.state, i, e);
     if (do_reset) store_consts<kDisturb, kOnePass>(b.consts, i, k);
     if (kStats) accumulate_stats(b.stats, i, do_reset, o, p);
@@ -407,6 +420,11 @@ int usv_capturexy_obs_reward_done_f32(const UsvCaptureXYIO* io, int64_t n, const
   return finish_launch();
 }
 
+int usv_step_fused_plan(const UsvStepParams* p, int32_t stats) {
+  if (!p) return USV_E_NULL;
+  return !stats && plan_matches<PlanFullDr>(*p) ? USV_STEP_PLAN_FULL_DR : USV_STEP_PLAN_GENERIC;
+}
+
 int usv_step_fused_f32(const UsvEnvBuffers* b, const float* actions, float* obs, float* rew, int64_t n,
                        const UsvStepParams* p, void* stream) {
   int rc = check_common(b, n, p);
@@ -421,18 +439,20 @@ int usv_step_fused_f32(const UsvEnvBuffers* b, const float* actions, float* obs,
   // bytes per env the next step reads again (state, reset_buf, episode sums): see step_fused_kernel
   const double reread = (double)n * (USV_S_COUNT * 4 + 8 + (st ? USV_ST_COUNT * 4 : 0));
   const bool one_pass_cs = reread <= kResidentL2Share * l2_bytes();
-#define USV_LAUNCH_STEP(D, S)                                                                                                       \
+  const PhiloxKeys keys = philox_round_keys(p->seed);
+#define USV_LAUNCH_STEP(D, S, P)                                                                                                    \
   do {                                                                                                                              \
-    auto* kern = one_pass_cs ? step_fused_kernel<D, S, Cache::kStream> : step_fused_kernel<D, S, Cache::kNormal>;                       \
+    auto* kern = one_pass_cs ? step_fused_kernel<D, S, Cache::kStream, P> : step_fused_kernel<D, S, Cache::kNormal, P>;             \
     ensure_dynamic_smem(kern, smem);                                                                                                \
-    launch_pdl(kern, dim3(grid), dim3(kBlock), smem, s, *b, (const float2*)actions, obs, rew, n, *p);                               \
+    launch_pdl(kern, dim3(grid), dim3(kBlock), smem, s, *b, (const float2*)actions, obs, rew, n, *p, keys);                         \
   } while (0)
   const bool all4 = p->use_const_force && p->use_sin_force && p->use_const_torque && p->use_sin_torque && !p->use_water_current;
-  if (dis && all4 && !st) USV_LAUNCH_STEP(2, false);
-  else if (dis && st) USV_LAUNCH_STEP(1, true);
-  else if (dis) USV_LAUNCH_STEP(1, false);
-  else if (st) USV_LAUNCH_STEP(0, true);
-  else USV_LAUNCH_STEP(0, false);
+  if (usv_step_fused_plan(p, st) == USV_STEP_PLAN_FULL_DR) USV_LAUNCH_STEP(2, false, PlanFullDr);
+  else if (dis && all4 && !st) USV_LAUNCH_STEP(2, false, PlanGeneric);
+  else if (dis && st) USV_LAUNCH_STEP(1, true, PlanGeneric);
+  else if (dis) USV_LAUNCH_STEP(1, false, PlanGeneric);
+  else if (st) USV_LAUNCH_STEP(0, true, PlanGeneric);
+  else USV_LAUNCH_STEP(0, false, PlanGeneric);
 #undef USV_LAUNCH_STEP
   return finish_launch();
 }

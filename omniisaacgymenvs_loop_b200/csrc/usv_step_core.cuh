@@ -235,11 +235,61 @@ __device__ __forceinline__ float wrap_pi(float a) {
   return a;
 }
 
+// Step plans: the discrete parameters of one step configuration, fixed at compile time so that the kernel neither tests them per
+// thread nor loops over a run-time sub-step count.  A field equal to kFromParams is read from UsvStepParams at run time; PlanGeneric
+// reads every field so.  Continuous parameters (dt, lag, bounds, scales, noise ranges, penalty coefficients) always come from
+// UsvStepParams, so a plan instance runs the same arithmetic as the generic one.
+constexpr int kFromParams = -1;
+template <int kPlan>
+__host__ __device__ __forceinline__ int plan_or(int from_params) { return kPlan == kFromParams ? from_params : kPlan; }
+
+// X(plan field, UsvStepParams member): every discrete field a plan may fix
+#define USV_PLAN_FIELDS(X)                                                                                                        \
+  X(n_substeps, n_substeps) X(action_affine, action_affine) X(action_noise, action_noise) X(noise_pos, noise_pos)                 \
+  X(noise_vel, noise_vel) X(noise_heading, noise_heading) X(envs_per_row, envs_per_row) X(use_drag_scale, use_drag_scale)          \
+  X(reward_mode, reward_mode) X(pen_linear_vel, pen_linear_vel.form) X(pen_angular_vel, pen_angular_vel.form)                     \
+  X(pen_angular_vel_variation, pen_angular_vel_variation.form) X(pen_energy, pen_energy.form)                                     \
+  X(pen_action_variation, pen_action_variation.form) X(use_const_force, use_const_force) X(use_sin_force, use_sin_force)          \
+  X(use_const_torque, use_const_torque) X(use_sin_torque, use_sin_torque) X(use_water_current, use_water_current)
+
+struct PlanGeneric {
+  static constexpr bool kFixed = false;
+#define USV_PLAN_ANY(f, m) static constexpr int f = kFromParams;
+  USV_PLAN_FIELDS(USV_PLAN_ANY)
+#undef USV_PLAN_ANY
+};
+
+// UsvEnvConfig().full_dr(), the configuration training and the benchmark run: classic action path, action / position / velocity /
+// heading noise, linear distance reward, the angular-velocity-variation and energy penalties, all four disturbance kinds without a
+// water current (the kDisturb == 2 kernel), no env grid.  Fields the plan leaves to UsvStepParams (penalties_use_u) are read only
+// behind a switch the plan turns off.  The reset switches (reset_env) stay run-time tests: a reset is rare, and folding them too made
+// the step slower on a B200 (47.3 against 43.1 us per step at 2^20 envs, profiles/r05_step_plan.md).
+struct PlanFullDr {
+  static constexpr bool kFixed = true;
+  static constexpr int n_substeps = 5, action_affine = 0, action_noise = 1, noise_pos = 1, noise_vel = 1, noise_heading = 1;
+  static constexpr int envs_per_row = 0, use_drag_scale = 0, reward_mode = USV_REWARD_LINEAR;
+  static constexpr int pen_linear_vel = USV_PEN_OFF, pen_angular_vel = USV_PEN_OFF, pen_angular_vel_variation = USV_PEN_EXP_NEG_ABS,
+                       pen_energy = USV_PEN_EXP_NEG_SUMSQ, pen_action_variation = USV_PEN_OFF;
+  static constexpr int use_const_force = 1, use_sin_force = 1, use_const_torque = 1, use_sin_torque = 1, use_water_current = 0;
+};
+
+// does `p` have the discrete parameters Plan fixes?
+template <class Plan>
+inline bool plan_matches(const UsvStepParams& p) {
+#define USV_PLAN_EQ(f, m) if (Plan::f != kFromParams && Plan::f != p.m) return false;
+  USV_PLAN_FIELDS(USV_PLAN_EQ)
+#undef USV_PLAN_EQ
+  return true;
+}
+
+// The products that end a term are rounded on their own (__fmul_rn): with the form fixed, the compiler could otherwise fuse one into
+// the sum of the terms, which the generic kernel (the term behind a run-time switch) never does.
+template <int kForm = kFromParams>
 __device__ __forceinline__ float penalty_scalar(const UsvPenaltyTerm& t, float x) {
-  switch (t.form) {
+  switch (plan_or<kForm>(t.form)) {
     case USV_PEN_NEG_ABS: return -fabsf(x) * t.c1 + t.c2;
-    case USV_PEN_NEG_DEADZONE: return -fmaxf(fabsf(x) - t.k, 0.0f) * t.c1;
-    case USV_PEN_EXP_NEG_ABS: return (__expf(-t.k * fabsf(x)) - 1.0f) * t.c1;
+    case USV_PEN_NEG_DEADZONE: return __fmul_rn(-fmaxf(fabsf(x) - t.k, 0.0f), t.c1);
+    case USV_PEN_EXP_NEG_ABS: return __fmul_rn(__expf(-t.k * fabsf(x)) - 1.0f, t.c1);
     default: return 0.0f;
   }
 }
@@ -379,8 +429,9 @@ __device__ __forceinline__ void reset_env(EnvState& e, EnvConst& k, const UsvSte
 // is affine in |v| with per-episode coefficients: D = a + b|v|.  a and b are formed once per control step (scaling and k_drag folded
 // in: 1e-7 relative against the reference's op order), the sub-step loop spends one FMA per axis.
 struct Damp { float au, bu, av, bv, ar, br; };
+template <class Plan = PlanGeneric>
 __device__ __forceinline__ Damp make_damp(const EnvConst& k, const UsvStepParams& p) {
-  const float sc = p.use_drag_scale ? p.scaling_damping * k.kdrag : p.scaling_damping;
+  const float sc = plan_or<Plan::use_drag_scale>(p.use_drag_scale) ? p.scaling_damping * k.kdrag : p.scaling_damping;
   const float off_fwd = p.offset_lin_forward_damping_speed;
   Damp d;
   d.au = ((k.linu + p.offset_linear_damping) - (p.lin_fwd[0] + off_fwd)) * sc;
@@ -435,6 +486,38 @@ __device__ __forceinline__ void planar_wrench(const EnvState& e, const EnvConst&
   rdot = Tz * inv_iz;
 }
 
+// one physics sub-step: thruster lag, wrench, semi-implicit Euler, heading advance.  (hsn, hcs) = (sin, cos) psi: one full evaluation per
+// control step, then advanced by the small per-sub-step yaw increment with a rotation by (cos d, sin d) from short Taylor polynomials
+// (|d| = dt*|r| <= 1/16; a full sincos beyond)
+template <int kDisturb>
+__device__ __forceinline__ void physics_substep(EnvState& e, const EnvConst& k, const UsvStepParams& p, const Damp& dm, float ox, float oy,
+                                                float inv_m, float inv_iz, float oma, float tgtL, float tgtR, float& hsn, float& hcs) {
+  // apply_forces(): update_forces() advances the lag BEFORE the wrench is applied
+  // [ref ThrusterDynamics.py:129-141; SNAP/USV_Virtual.py:640]
+  e.thrL = __fadd_rn(__fmul_rn(e.thrL, p.lag_alpha), __fmul_rn(oma, tgtL));
+  e.thrR = __fadd_rn(__fmul_rn(e.thrR, p.lag_alpha), __fmul_rn(oma, tgtR));
+  float du, dv, dr, Fx, Fy, Tz, ax, ay, rdot;
+  planar_wrench<kDisturb>(e, k, p, dm, ox, oy, inv_m, inv_iz, hsn, hcs, du, dv, dr, Fx, Fy, Tz, ax, ay, rdot);
+  // world.step(): semi-implicit Euler (velocities first, then positions)
+  e.vx += p.dt * ax;
+  e.vy += p.dt * ay;
+  e.r += p.dt * rdot;
+  e.x += p.dt * e.vx;
+  e.y += p.dt * e.vy;
+  const float dpsi = p.dt * e.r;
+  e.psi += dpsi;
+  if (fabsf(dpsi) <= 0.0625f) {   // |r| <= 3.1 rad/s at dt = 0.02: sin to d^5 (error d^7/5040 < 8e-13), cos to d^4 (d^6/720 < 9e-11)
+    const float d2 = dpsi * dpsi;
+    const float sd = dpsi * fmaf(d2, fmaf(d2, 1.0f / 120.0f, -1.0f / 6.0f), 1.0f);
+    const float cd = fmaf(d2, fmaf(d2, 1.0f / 24.0f, -0.5f), 1.0f);
+    const float nc = hcs * cd - hsn * sd;
+    hsn = hsn * cd + hcs * sd;
+    hcs = nc;
+  } else {
+    fsincos(e.psi, &hsn, &hcs);
+  }
+}
+
 // Sensed state + action bookkeeping handed from the shared dynamics part of a control step to the task-specific part.
 struct DynOut {
   float raw0, raw1;              // policy action after the VecEnv clamp (live: prev_thrust_cmds)
@@ -444,15 +527,22 @@ struct DynOut {
   float pxn, pyn, vxn, vyn, wn, yawn, hs, hc;  // noisy state the task observes; (hc, hs) = heading
 };
 
+// per-step noise draw; a fixed Plan draws it from `keys`, the round keys of p.seed
+template <class Plan>
+__device__ __forceinline__ Uniform8 step_noise(const UsvStepParams& p, const PhiloxKeys* keys, uint64_t gid, uint64_t step) {
+  if constexpr (Plan::kFixed) return philox_uniform8x16(*keys, gid, step, RS_STEP_A);
+  else return philox_uniform8x16(p.seed, gid, step, RS_STEP_A);
+}
+
 // pre_physics_step + the physics sub-steps + update_state of one control step for one env, state in registers
-template <int kDisturb, bool kLutGlobal>
+template <int kDisturb, bool kLutGlobal, class Plan = PlanGeneric>
 __device__ __forceinline__ void step_dynamics(EnvState& e, EnvConst& k, const UsvStepParams& p, bool do_reset,
                                              float2 act, uint64_t gid, int64_t lid, uint64_t step,
                                              const float* __restrict__ s_lutL, const float* __restrict__ s_lutR,
-                                             DynOut& s) {
+                                             DynOut& s, const PhiloxKeys* keys = nullptr) {
   // ---- pre_physics_step ------------------------------------------------------------------
   if (do_reset) reset_env<kDisturb>(e, k, p, gid, step);
-  const Uniform8 nz = philox_uniform8x16(p.seed, gid, step, RS_STEP_A);
+  const Uniform8 nz = step_noise<Plan>(p, keys, gid, step);
   const float u_a0 = nz.v[0], u_a1 = nz.v[1], u_vx = nz.v[2], u_vy = nz.v[3], u_w = nz.v[4], u_h = nz.v[5],
               u_px = nz.v[6], u_py = nz.v[7];
   // VecEnvRLGames.step clamps to +-clipActions  [ref vec_env_rlgames.py:136-140]
@@ -461,10 +551,10 @@ __device__ __forceinline__ void step_dynamics(EnvState& e, EnvConst& k, const Us
   float pa0, pa1;  // what Penalties sees as `actions`
   float c0, c1;    // command that indexes the LUT
   s.raw0 = a0; s.raw1 = a1;
-  if (!p.action_affine) {
+  if (!plan_or<Plan::action_affine>(p.action_affine)) {
     // classic [ref SNAP/USV_Virtual.py:589-615]: AN.add_noise_on_act works IN PLACE on the tensor that
     // self.actions aliases -> penalties see the noisy, unclamped action; resets zero only the thrust.
-    if (p.action_noise) {
+    if (plan_or<Plan::action_noise>(p.action_noise)) {
       a0 += urange(u_a0, p.action_noise_min, p.action_noise_max);
       a1 += urange(u_a1, p.action_noise_min, p.action_noise_max);
     }
@@ -475,7 +565,7 @@ __device__ __forceinline__ void step_dynamics(EnvState& e, EnvConst& k, const Us
   } else {
     // live [ref OIGE/tasks/USV_Virtual.py:1064-1097]
     float t0 = a0 + p.action_bias, t1 = a1 + p.action_bias;
-    if (p.action_noise) {
+    if (plan_or<Plan::action_noise>(p.action_noise)) {
       t0 += urange(u_a0, p.action_noise_min, p.action_noise_max);
       t1 += urange(u_a1, p.action_noise_min, p.action_noise_max);
     }
@@ -496,7 +586,7 @@ __device__ __forceinline__ void step_dynamics(EnvState& e, EnvConst& k, const Us
 
   // ---- physics sub-steps -----------------------------------------------------------------
   float ox = 0.0f, oy = 0.0f;
-  if (kDisturb && p.envs_per_row > 0) {
+  if (kDisturb && plan_or<Plan::envs_per_row>(p.envs_per_row) > 0) {
     const int row = (int)(lid / p.envs_per_row), col = (int)(lid % p.envs_per_row);
     ox = p.grid_row_offset - (float)row * p.env_spacing;
     oy = (float)col * p.env_spacing - p.grid_col_offset;
@@ -504,36 +594,14 @@ __device__ __forceinline__ void step_dynamics(EnvState& e, EnvConst& k, const Us
   const float oma = 1.0f - p.lag_alpha;
   // 2-ulp reciprocals (MUFU.RCP): the accelerations they scale are compared at 1e-5
   const float inv_m = __fdividef(1.0f, k.mass), inv_iz = __fdividef(1.0f, p.izz * k.kiz);
-  // heading (cos psi, sin psi): one full evaluation per control step, then advanced by the small per-sub-step yaw
-  // increment with a rotation by (cos d, sin d) from short Taylor polynomials (|d| = dt*|r| <= 1/16; a full sincos beyond)
   float hsn, hcs;
   fsincos(e.psi, &hsn, &hcs);
-  const Damp dm = make_damp(k, p);
-  for (int ss = 0; ss < p.n_substeps; ++ss) {
-    // apply_forces(): update_forces() advances the lag BEFORE the wrench is applied
-    // [ref ThrusterDynamics.py:129-141; SNAP/USV_Virtual.py:640]
-    e.thrL = __fadd_rn(__fmul_rn(e.thrL, p.lag_alpha), __fmul_rn(oma, tgtL));
-    e.thrR = __fadd_rn(__fmul_rn(e.thrR, p.lag_alpha), __fmul_rn(oma, tgtR));
-    float du, dv, dr, Fx, Fy, Tz, ax, ay, rdot;
-    planar_wrench<kDisturb>(e, k, p, dm, ox, oy, inv_m, inv_iz, hsn, hcs, du, dv, dr, Fx, Fy, Tz, ax, ay, rdot);
-    // world.step(): semi-implicit Euler (velocities first, then positions)
-    e.vx += p.dt * ax;
-    e.vy += p.dt * ay;
-    e.r += p.dt * rdot;
-    e.x += p.dt * e.vx;
-    e.y += p.dt * e.vy;
-    const float dpsi = p.dt * e.r;
-    e.psi += dpsi;
-    if (fabsf(dpsi) <= 0.0625f) {   // |r| <= 3.1 rad/s at dt = 0.02: sin to d^5 (error d^7/5040 < 8e-13), cos to d^4 (d^6/720 < 9e-11)
-      const float d2 = dpsi * dpsi;
-      const float sd = dpsi * fmaf(d2, fmaf(d2, 1.0f / 120.0f, -1.0f / 6.0f), 1.0f);
-      const float cd = fmaf(d2, fmaf(d2, 1.0f / 24.0f, -0.5f), 1.0f);
-      const float nc = hcs * cd - hsn * sd;
-      hsn = hsn * cd + hcs * sd;
-      hcs = nc;
-    } else {
-      fsincos(e.psi, &hsn, &hcs);
-    }
+  const Damp dm = make_damp<Plan>(k, p);
+  if constexpr (Plan::n_substeps != kFromParams) {
+#pragma unroll
+    for (int ss = 0; ss < Plan::n_substeps; ++ss) physics_substep<kDisturb>(e, k, p, dm, ox, oy, inv_m, inv_iz, oma, tgtL, tgtR, hsn, hcs);
+  } else {
+    for (int ss = 0; ss < p.n_substeps; ++ss) physics_substep<kDisturb>(e, k, p, dm, ox, oy, inv_m, inv_iz, oma, tgtL, tgtR, hsn, hcs);
   }
   e.psi = wrap_pi(e.psi);
 
@@ -541,8 +609,8 @@ __device__ __forceinline__ void step_dynamics(EnvState& e, EnvConst& k, const Us
   e.progress += 1;  // [ref rl_task.py:294]
   // update_state: observation noise  [ref SNAP/USV_Virtual.py:476-530 ; USV_disturbances.py:552-601]
   float pxn = e.x, pyn = e.y, vxn = e.vx, vyn = e.vy, wn = e.r, yawn = e.psi;
-  if (p.noise_pos) { pxn += urange(u_px, p.pos_noise_min, p.pos_noise_max); pyn += urange(u_py, p.pos_noise_min, p.pos_noise_max); }
-  if (p.noise_vel) {
+  if (plan_or<Plan::noise_pos>(p.noise_pos)) { pxn += urange(u_px, p.pos_noise_min, p.pos_noise_max); pyn += urange(u_py, p.pos_noise_min, p.pos_noise_max); }
+  if (plan_or<Plan::noise_vel>(p.noise_vel)) {
     vxn += urange(u_vx, p.vel_noise_min, p.vel_noise_max);
     vyn += urange(u_vy, p.vel_noise_min, p.vel_noise_max);
     wn += urange(u_w, p.vel_noise_min, p.vel_noise_max);
@@ -550,7 +618,7 @@ __device__ __forceinline__ void step_dynamics(EnvState& e, EnvConst& k, const Us
   // heading the task observes = (cos, sin)(psi + noise): the loop already tracks (cos psi, sin psi); rotate it by the small noise
   // angle (|dh| <= 0.5: same 5e-9 polynomial error as the per-sub-step update) instead of a third full sincos per control step
   float hs = hsn, hc = hcs;
-  if (p.noise_heading) {
+  if (plan_or<Plan::noise_heading>(p.noise_heading)) {
     const float dh = urange(u_h, p.heading_noise_min, p.heading_noise_max);
     yawn += dh;
     if (fabsf(dh) <= 0.5f) {
